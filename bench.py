@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--backend nvrtc|interp]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's CPU algorithm (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR    # also write the headline frame of the last timed step as .npy
 
 A "step" renders one whole frame of the workload.  One process per GPU: rank r renders its row band
 on its own GPU through the C ABI (maray_cuda_render_band); at N > 1 the band kernels store straight into
@@ -34,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from
 
 DEFAULT_WORKLOAD = "chess_4k"
 METRIC = "render_throughput"
@@ -62,8 +64,8 @@ def committed_dram_traffic(workload: str, backend: str):
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=_int_at_least(1), default=10)
+    ap.add_argument("--warmup", type=_int_at_least(0), default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=os.environ.get("MARAY_BENCH_WORKLOAD", DEFAULT_WORKLOAD),
                     choices=["chess_1k", "sdf", "chess_4k", "textured", "deep"])
@@ -79,7 +81,35 @@ def parse_args():
     ap.add_argument("--configs", default="all",
                     help="sub-records for the other BASELINE configs: all | none | comma list (chess_1k,sdf,textured,deep)")
     ap.add_argument("--no-first-frame", action="store_true", help="skip the cold time-to-first-frame measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline workload's frame of the last step as DIR/frame.npy "
+                         "(float32, rows x width x RGB; a fixed sample of rows when the frame exceeds 64 MB, their "
+                         "indices in DIR/frame_rows.npy) so that two builds can be compared output for output")
     return ap.parse_args()
+
+
+def _int_at_least(lo):
+    def parse(s):
+        v = int(s)
+        if v < lo:
+            raise argparse.ArgumentTypeError(f"must be at least {lo}")
+        return v
+    return parse
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_frame(out_dir, frame):
+    """Writes the frame (uint8, h x w x 3) as float32: whole when it fits in DUMP_BYTES, otherwise the rows of a fixed,
+    seeded sample (the same rows for the same frame size), sorted.  The row indices go beside it as float64."""
+    import numpy as np
+    h, w = frame.shape[:2]
+    n = min(h, (DUMP_BYTES - 8 * h - 1024) // (4 * 3 * w))
+    rows = np.arange(h) if n == h else np.sort(np.random.default_rng(0).choice(h, size=n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame.npy"), frame[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_rows.npy"), rows.astype(np.float64))
 
 
 # ---- CPU arm: the reference's algorithm (oracle port) on the host cores ---------------------------
@@ -454,6 +484,8 @@ def measure(name, args, steps, warmup, rank, local_rank, world, dev, full):
         else:
             frame_host = np.empty((h, w, 3), dtype=np.uint8)
             r.copy_to_host(frame_ptr, frame_host)
+        if full and args.dump_outputs:
+            dump_frame(args.dump_outputs, frame_host)
 
     # ---- e2e: host image buffer, device->host inside the timed region -----------------------------
     e2e_steps, e2e_warm = steps, min(warmup, 3)
@@ -723,6 +755,8 @@ def main():
     RESULT_OUT = _claim_stdout()
     args = parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes the GPU frame; --impl reference renders only a sample of rows")
         run_reference(args)
     else:
         run_ours(args)

@@ -1,8 +1,9 @@
 """The exact mode of the device libm (csrc/device_libm_glibc.cuh, MARAY_LIBM_GLIBC): sin/exp/ln with the bits of the
 host libm the reference calls (reference src/lib.rs:648-650, src/wasm.rs:11-13).
 
-CPU: the header's host rendition against this host's glibc, bit for bit (tools/glibc_libm_check.c); the committed
-tables against the host library; the exact mode compiles through NVRTC without a GPU.
+CPU: the header's host rendition against this host's glibc, bit for bit (tools/glibc_libm_check.c), and on any host
+against glibc 2.39's results stored under tests/golden; the committed tables against the host library; the exact mode
+compiles through NVRTC without a GPU.
 GPU (`-m gpu`): f64 channel values of sin/exp/ln scenes and of the deep scene are BIT-IDENTICAL to the oracle's in
 exact mode, with both back ends -- the class of scenes that is only "within 1 LSB" with the default libm."""
 import os
@@ -44,6 +45,59 @@ def test_exact_mode_returns_the_host_libms_bits(tmp_path):
         out = subprocess.run([str(exe), "2000000"], capture_output=True, text=True)
         assert "total differing: 0" in out.stdout and out.returncode == 0, out.stdout[-3000:]
         assert out.stdout.count(" 0 differ") >= 25          # every (function, range) line
+
+
+LIBM_DRIVER = r"""
+#define MR_LIBM_HOST 1
+#ifndef FAST_MODE
+#define MR_LIBM_GLIBC 1
+#endif
+#include "device_libm.cuh"
+#include <stdio.h>
+#include <stdlib.h>
+#include <string.h>
+/* argv: function (sin, exp, log, sgn), n, input file of n doubles, output file */
+int main(int argc, char** argv) {
+    if (argc != 5) return 2;
+    const long n = atol(argv[2]);
+    double* x = malloc(n * sizeof *x);
+    FILE* f = fopen(argv[3], "rb");
+    if (!f || fread(x, sizeof *x, n, f) != (size_t)n) return 3;
+    fclose(f);
+    for (long i = 0; i < n; i++) {
+        if (!strcmp(argv[1], "sin")) x[i] = mr_sin_g(x[i]);
+        else if (!strcmp(argv[1], "exp")) x[i] = mr_exp(x[i]);        /* the names the kernels call, in the mode compiled */
+        else if (!strcmp(argv[1], "log")) x[i] = mr_log(x[i]);
+        else x[i] = mr_sin_ge0(x[i]);
+    }
+    f = fopen(argv[4], "wb");
+    return !f || fwrite(x, sizeof *x, n, f) != (size_t)n || fclose(f);
+}
+"""
+
+
+def test_exact_mode_returns_the_stored_glibc_bits(tmp_path):
+    """The host rendition of the exact mode against results of glibc 2.39 kept under tests/golden (make_libm_golden.py):
+    the check of test_exact_mode_returns_the_host_libms_bits on a sample of its arguments, on any host.  Default mode
+    (-DFAST_MODE): exp and log are the same routines, and the sign of the sine is glibc's too."""
+    golden = os.path.join(ROOT, "tests", "golden")
+    (tmp_path / "driver.c").write_text(LIBM_DRIVER)
+    for flags in ([], ["-DFAST_MODE"]):
+        exe = tmp_path / ("driver" + "_fast" * bool(flags))
+        subprocess.check_call(["gcc", "-O2", "-std=gnu11", "-ffp-contract=off", "-fno-builtin", *flags,
+                               "-I", os.path.join(ROOT, "maray_b200", "csrc"), "-o", str(exe), str(tmp_path / "driver.c"), "-lm"])
+        for name in ("sin", "exp", "log"):
+            pairs = np.load(os.path.join(golden, f"glibc_239_{name}.npy"))
+            x, want = pairs[:, 0].view(np.float64), pairs[:, 1].view(np.float64)
+            checks = [("sgn", (want >= 0.0).astype(np.float64))] if name == "sin" else []
+            if not (flags and name == "sin"):
+                checks.append((name, want))
+            for fn, expect in checks:
+                np.ascontiguousarray(x).tofile(tmp_path / "x.bin")
+                subprocess.check_call([str(exe), fn, str(x.size), str(tmp_path / "x.bin"), str(tmp_path / "y.bin")])
+                got = np.fromfile(tmp_path / "y.bin", dtype=np.float64)
+                same = bits_equal(got, expect)
+                assert same.all(), (flags, fn, int((~same).sum()), x[~same][:4], got[~same][:4], expect[~same][:4])
 
 
 @needs_glibc_239

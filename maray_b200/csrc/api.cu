@@ -63,11 +63,8 @@ struct Gpu {
     // back ends
     std::vector<cudaLibrary_t> libs;                   // one per translation unit (chain form: one per segment)
     std::vector<cudaKernel_t> jit_kernels;             // the kernel of each unit, in launch order
-    cudaKernel_t jit_pre_x = nullptr, jit_pre_y = nullptr;
     double* d_frame = nullptr; size_t frame_cap = 0;   // chain form: values crossing segment cuts, F[slot * FS + pixel]
-    double* d_colv = nullptr; size_t colv_cap = 0;     // hoisting tables (doubles)
-    double* d_rowv = nullptr; size_t rowv_cap = 0;
-    cudaEvent_t hoist_done = nullptr;                  // last launch that read the tables (they are per GPU, not per stream)
+    cudaEvent_t frame_done = nullptr;                  // last chain launch that used d_frame (one per GPU, not per stream)
     uint64_t* d_code = nullptr;
     double* d_consts = nullptr;
     double* d_sink = nullptr;
@@ -120,13 +117,11 @@ struct maray_cuda {
     std::vector<uint64_t> bc_device;                   // bc.code with operand fields scaled for the launch shape
     unsigned interp_block = 128, interp_ppt = 2;       // launch shape: threads per block, pixels per thread
     int libm = MARAY_LIBM_FAST;                        // maray_cuda_set_libm / MARAY_LIBM
-    int interp_dispatch = 0;                           // MARAY_INTERP_DISPATCH=tree (kernels.hpp launch_interp), A/B
     unsigned jit_block = 256;
     unsigned jit_dyn_smem = 0;                         // dynamic shared memory of the generated kernel
     unsigned jit_maxreg = 0;
     bool jit_chain = false;                            // one kernel per segment, launched in order over a global frame
     unsigned jit_frame_slots = 0;
-    unsigned jit_ncol = 0, jit_nrow = 0;               // hoisted values per column / per row
     maray_cuda_stats stats{};
     int report_kind = MARAY_REPORT_NONE;
     uint32_t report_every = 0;
@@ -171,10 +166,8 @@ void release_backend(maray_cuda* h, bool cancel_job = true) {
     for (Gpu& g : h->gpus) {
         cudaSetDevice(g.device);
         for (cudaLibrary_t l : g.libs) cudaLibraryUnload(l);
-        g.libs.clear(); g.jit_kernels.clear(); g.jit_pre_x = g.jit_pre_y = nullptr;
+        g.libs.clear(); g.jit_kernels.clear();
         if (g.d_frame) { cudaFree(g.d_frame); g.d_frame = nullptr; g.frame_cap = 0; }
-        if (g.d_colv) { cudaFree(g.d_colv); g.d_colv = nullptr; g.colv_cap = 0; }
-        if (g.d_rowv) { cudaFree(g.d_rowv); g.d_rowv = nullptr; g.rowv_cap = 0; }
         if (g.d_code) { cudaFree(g.d_code); g.d_code = nullptr; }
         if (g.d_consts) { cudaFree(g.d_consts); g.d_consts = nullptr; }
     }
@@ -217,11 +210,6 @@ int upload_textures(maray_cuda* h) {
 // as the frame (the importers have it mapped already), behind the pixels.
 constexpr uint32_t kBandCounters = 64;
 constexpr uint32_t kBandCounterStride = 32;    // 32-bit words between two counters: one 128-byte line each
-// bit 0: signal by atomic exchange instead of a release store; bits 1-2: poll by atomic add of 0 (1) / volatile load (2)
-// instead of an acquire load.  Default 3, both atomic -- performed at the counter's home L2.  Measured at N = 2 (GPU call
-// 51): polled with LOADS (acquire.sys or volatile; LDG.E.STRONG.SYS + CCTL.IVALL in the SASS) the exporting GPU sees a
-// peer's store 1-50 ms late, with the atomic poll in 6-8 us.
-inline int band_signal_mode() { const char* e = std::getenv("MARAY_BAND_SIGNAL_MODE"); return e ? int(std::strtol(e, nullptr, 10)) : 3; }
 inline size_t band_counters_offset(uint32_t w, uint32_t hgt) { return (size_t(w) * hgt * 3 + 255) & ~size_t(255); }
 inline unsigned int* band_timeout_word(Gpu& g) { return reinterpret_cast<unsigned int*>(reinterpret_cast<uint8_t*>(g.d_sink) + 128); }
 
@@ -383,13 +371,8 @@ int nvrtc_compile(JitBuild* jb, const std::atomic<bool>* cancel, bool cached_onl
     if (const char* e = std::getenv("MARAY_JIT_LINEINFO")) lineinfo = std::strtoul(e, nullptr, 10) != 0;
     if (lineinfo) options.push_back("-lineinfo");
     if (jb->maxreg) options.push_back("--maxrregcount=" + std::to_string(jb->maxreg));
-    if (std::getenv("MARAY_JIT_NOSLOW")) options.push_back("-DMR_NO_SLOW=1");   // experiment only (wrong for huge/NaN arguments)
     if (jb->libm == MARAY_LIBM_CUDA) options.push_back("-DMR_LIBM_PLAIN=1");    // A/B: libdevice's sin/exp/log
     if (jb->libm == MARAY_LIBM_GLIBC) options.push_back("-DMR_LIBM_GLIBC=1");   // exact mode (device_libm_glibc.cuh)
-    if (const char* e = std::getenv("MARAY_LIBM_SIN"))                          // A/B: round 1's quadrant-parity sine
-        if (std::string(e) == "parity") options.push_back("-DMR_SIN_PARITY=1");
-    if (const char* e = std::getenv("MARAY_LIBM_EXPLOG"))                       // A/B: round 1's polynomial exp and log
-        if (std::string(e) == "poly") options.push_back("-DMR_EXPLOG_POLY=1");
 
     jb->registers = 0;
     jb->compile_threads = 0;
@@ -523,24 +506,16 @@ int jit_build(const Program& prog, JitBuild* jb, bool cached_only, const std::at
     copt.sm_count_hint = jb->sms ? jb->sms : 148;
     if (const char* e = std::getenv("MARAY_JIT_SEGMENT_VALUES")) copt.segment_values = uint32_t(std::strtoul(e, nullptr, 10));
     if (const char* e = std::getenv("MARAY_JIT_INLINE_TRANS_BELOW")) copt.inline_transcendentals_below = uint32_t(std::strtoul(e, nullptr, 10));
-    if (const char* e = std::getenv("MARAY_JIT_SYNC_EVERY")) copt.sync_every = uint32_t(std::strtoul(e, nullptr, 10));
     if (const char* e = std::getenv("MARAY_JIT_CONST_BANK")) copt.constants_in_bank = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_PERSISTENT")) copt.persistent = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_CONST_ORDER")) copt.constants_in_use_order = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_HOIST")) copt.hoist = std::strtoul(e, nullptr, 10) != 0;
     if (const char* e = std::getenv("MARAY_JIT_BOOLEAN")) copt.boolean_logic = std::strtoul(e, nullptr, 10) != 0;
     if (const char* e = std::getenv("MARAY_JIT_SIGN_OF_SINE")) copt.sign_of_sine = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_SCRATCH")) copt.scratch_batches = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_SCRATCH_TABLES")) copt.scratch_tables = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_PRIVATE_HELPERS")) copt.private_batch_helpers = std::strtoul(e, nullptr, 10) != 0;
-    if (const char* e = std::getenv("MARAY_JIT_BATCH_WIDTH")) copt.batch_width = uint32_t(std::strtoul(e, nullptr, 10));
     if (const char* e = std::getenv("MARAY_JIT_BLOCK")) { copt.block = uint32_t(std::strtoul(e, nullptr, 10)); copt.auto_shape = false; }
     if (const char* e = std::getenv("MARAY_JIT_MIN_BLOCKS")) { copt.min_blocks_per_sm = uint32_t(std::strtoul(e, nullptr, 10)); copt.auto_shape = false; }
     jb->maxreg = 0;
     if (const char* e = std::getenv("MARAY_JIT_MAXREG")) jb->maxreg = unsigned(std::strtoul(e, nullptr, 10));
     // Programs above the segment size compile as a CHAIN of kernels, one translation unit each (codegen.hpp):
     // the units compile concurrently on all host cores and nothing is linked.  MARAY_JIT_CHAIN=0 gives round
-    // 1's form (segment functions in one unit) for A/B.  sin/exp/ln stay out of line above the threshold:
+    // 1's form (segment functions in one unit).  sin/exp/ln stay out of line above the threshold:
     // inlined, the code of a transcendental-heavy program is several MB of instructions no warp ever re-uses
     // and the kernel becomes instruction-fetch bound (measured: 33.8 ms inlined vs 18.7 ms out of line on the
     // 20 000-value deep scene, no_instruction stalls 9.1 per issued instruction; profiles/).
@@ -586,8 +561,6 @@ int jit_install(maray_cuda* h, JitBuild&& jb) {
     h->jit = std::move(jb);
     h->jit_block = h->jit.info.block;
     h->jit_dyn_smem = h->jit.info.dynamic_smem_bytes;
-    h->jit_ncol = h->jit.info.n_col;
-    h->jit_nrow = h->jit.info.n_row;
     h->jit_chain = h->jit.info.chain;
     h->jit_frame_slots = h->jit.info.frame_slots;
     fill_jit_stats(h);
@@ -626,10 +599,6 @@ int jit_install(maray_cuda* h, JitBuild&& jb) {
                     cudaGetLastError();
             } else cudaGetLastError();
         }
-        if (h->jit_ncol || h->jit_nrow) {
-            CU_TRY(h, cudaLibraryGetKernel(&g.jit_pre_x, g.libs[0], kJitPreXName));
-            CU_TRY(h, cudaLibraryGetKernel(&g.jit_pre_y, g.libs[0], kJitPreYName));
-        }
     }
     if (!h->gpus.empty()) cudaSetDevice(h->gpus[0].device);
     h->stats.load_ms += now_ms() - t3;
@@ -648,8 +617,6 @@ int interp_build_and_install(maray_cuda* h) {
     if (!compile_bytecode(h->prog, &h->bc, &err, uniform)) return fail(h, MARAY_E_COMPILE, err);
     if (uniform && h->bc.n_uniform > 4096 && !compile_bytecode(h->prog, &h->bc, &err, false)) return fail(h, MARAY_E_COMPILE, err);
     choose_interp_shape(h);
-    h->interp_dispatch = 0;
-    if (const char* e = std::getenv("MARAY_INTERP_DISPATCH")) h->interp_dispatch = std::string(e) == "tree" ? 1 : 0;
     if (!h->interp_block)
         return fail(h, MARAY_E_UNSUPPORTED, "program needs " + std::to_string(h->bc.n_wide) +
                                                 " live values per pixel, more than the interpreter's shared-memory slot file holds");
@@ -686,54 +653,16 @@ int adopt_finished_job(maray_cuda* h) {
 
 int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint8_t* d_out, double* d_f64,
                 size_t f64_plane, cudaStream_t stream) {
-    MrParams p;
+    MrParams p{};
     p.out = d_out; p.f64_out = d_f64; p.f64_plane = f64_plane; p.tex = g.d_textab;
     p.p0 = p0; p.n = n; p.W = w;
     p.out_aligned = (reinterpret_cast<uintptr_t>(d_out) % 16 == 0) ? 1u : 0u;
-    p.colv = nullptr; p.rowv = nullptr; p.row_base = 0; p.rows = 0;
     if (n == 0) return MARAY_OK;
     if (h->use_jit) {
-        if (h->jit_ncol || h->jit_nrow) {
-            // Prologue: x-only values once per column, y-only values once per row of this launch.
-            const uint32_t y_first = p0 / w, y_last = (p0 + n - 1) / w, rows = y_last - y_first + 1;
-            const size_t need_c = std::max<size_t>(size_t(h->jit_ncol) * w, 1), need_r = std::max<size_t>(size_t(h->jit_nrow) * rows, 1);
-            if (g.colv_cap < need_c) {
-                if (g.d_colv) cudaFree(g.d_colv);
-                g.d_colv = nullptr; g.colv_cap = 0;
-                CU_TRY(h, cudaMalloc(&g.d_colv, need_c * sizeof(double)));
-                g.colv_cap = need_c;
-            }
-            if (g.rowv_cap < need_r) {
-                if (g.d_rowv) cudaFree(g.d_rowv);
-                g.d_rowv = nullptr; g.rowv_cap = 0;
-                CU_TRY(h, cudaMalloc(&g.d_rowv, need_r * sizeof(double)));
-                g.rowv_cap = need_r;
-            }
-            // The tables are one per GPU: a band issued on another stream must not overwrite them while
-            // the previous band's kernel still reads them (maray_cuda_render_band takes any stream).
-            if (!g.hoist_done) CU_TRY(h, cudaEventCreateWithFlags(&g.hoist_done, cudaEventDisableTiming));
-            else CU_TRY(h, cudaStreamWaitEvent(stream, g.hoist_done, 0));
-            const MrTexture* tex = g.d_textab;
-            uint32_t base = 0;
-            if (h->jit_ncol) {
-                uint32_t cnt = w;
-                void* a[] = {&g.d_colv, &cnt, &base, &tex};
-                CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(g.jit_pre_x), dim3((cnt + 127) / 128), dim3(128), a, 0, stream));
-            }
-            if (h->jit_nrow) {
-                uint32_t cnt = rows, ybase = y_first;
-                void* a[] = {&g.d_rowv, &cnt, &ybase, &tex};
-                CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(g.jit_pre_y), dim3((cnt + 127) / 128), dim3(128), a, 0, stream));
-            }
-            p.colv = g.d_colv; p.rowv = g.d_rowv; p.row_base = y_first; p.rows = rows;
-        }
         if (!h->jit_chain) {
             void* args[] = {&p};
-            unsigned grid = (n + h->jit_block - 1) / h->jit_block;
-            if (h->jit.info.persistent_blocks_per_sm)     // the kernel walks the band's blocks itself
-                grid = std::min(grid, unsigned(g.sms) * h->jit.info.persistent_blocks_per_sm);
+            const unsigned grid = (n + h->jit_block - 1) / h->jit_block;
             CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(g.jit_kernels[0]), dim3(grid), dim3(h->jit_block), args, h->jit_dyn_smem, stream));
-            if (g.hoist_done && (h->jit_ncol || h->jit_nrow)) CU_TRY(h, cudaEventRecord(g.hoist_done, stream));
         } else {
             // Chain form: the segment kernels run in order over a chunk of pixels whose frame (values that cross
             // a cut, F[slot * FS + pixel]) fits the budget; chunks follow each other on the stream.
@@ -742,9 +671,10 @@ int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
             const size_t per_px = std::max<size_t>(h->jit_frame_slots, 1) * sizeof(double);
             size_t chunk = std::max<size_t>(budget / per_px, h->jit_block);
             chunk = std::min<size_t>(chunk / h->jit_block * h->jit_block, (size_t(n) + h->jit_block - 1) / h->jit_block * h->jit_block);
-            // One frame per GPU: launches of a handle that use it are serialised across streams (like the hoisting tables).
-            if (!g.hoist_done) CU_TRY(h, cudaEventCreateWithFlags(&g.hoist_done, cudaEventDisableTiming));
-            else CU_TRY(h, cudaStreamWaitEvent(stream, g.hoist_done, 0));
+            // One frame per GPU: a band issued on another stream must not overwrite it while the previous band's
+            // kernels still use it (maray_cuda_render_band takes any stream), so launches that use it are serialised.
+            if (!g.frame_done) CU_TRY(h, cudaEventCreateWithFlags(&g.frame_done, cudaEventDisableTiming));
+            else CU_TRY(h, cudaStreamWaitEvent(stream, g.frame_done, 0));
             if (g.frame_cap < chunk * per_px) {
                 if (g.d_frame) cudaFree(g.d_frame);
                 g.d_frame = nullptr; g.frame_cap = 0;
@@ -766,7 +696,7 @@ int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
                 for (cudaKernel_t k : g.jit_kernels)
                     CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(k), dim3(grid), dim3(h->jit_block), args, h->jit_dyn_smem, stream));
             }
-            CU_TRY(h, cudaEventRecord(g.hoist_done, stream));
+            CU_TRY(h, cudaEventRecord(g.frame_done, stream));
         }
     } else {
         // The interpreter renders windows [x0,x1) x rows with every block inside one row: a linear pixel range
@@ -787,8 +717,7 @@ int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
             t.out_aligned = (reinterpret_cast<uintptr_t>(t.out) % 16 == 0) ? 1u : 0u;
             t.libm_exact = h->libm == MARAY_LIBM_GLIBC ? 1u : 0u;
             CU_TRY(h, launch_interp(t, g.d_code, unsigned(h->bc_device.size()), g.d_consts, unsigned(h->bc.consts.size()),
-                                    h->bc.n_uniform, h->bc.n_wide, !h->bc.row_uniform, h->interp_block, h->interp_ppt, stream,
-                                    h->interp_dispatch));
+                                    h->bc.n_uniform, h->bc.n_wide, !h->bc.row_uniform, h->interp_block, h->interp_ppt, stream));
             const uint32_t count = cols * rows;
             done += count; pix += count; left -= count;
         }
@@ -1100,7 +1029,7 @@ void maray_cuda_destroy(maray_cuda_t* h) {
         if (g.d_out) cudaFree(g.d_out);
         if (g.d_f64) cudaFree(g.d_f64);
         if (g.d_sink) cudaFree(g.d_sink);
-        if (g.hoist_done) cudaEventDestroy(g.hoist_done);
+        if (g.frame_done) cudaEventDestroy(g.frame_done);
         if (g.ev0) cudaEventDestroy(g.ev0);
         if (g.ev1) cudaEventDestroy(g.ev1);
         if (g.stream) cudaStreamDestroy(g.stream);
@@ -1293,7 +1222,7 @@ int maray_cuda_band_signal(maray_cuda_t* h, void* d_frame, uint32_t w, uint32_t 
     if (h->gpus.empty()) return fail(h, MARAY_E_CUDA, "host-only handle");
     CU_TRY(h, cudaSetDevice(h->gpus[0].device));
     auto* counters = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(d_frame) + band_counters_offset(w, hgt));
-    CU_TRY(h, launch_band_signal(counters + size_t(rank) * kBandCounterStride, value, static_cast<cudaStream_t>(stream), band_signal_mode()));
+    CU_TRY(h, launch_band_signal(counters + size_t(rank) * kBandCounterStride, value, static_cast<cudaStream_t>(stream)));
     return MARAY_OK;
 }
 
@@ -1306,7 +1235,7 @@ int maray_cuda_band_wait(maray_cuda_t* h, void* d_frame, uint32_t w, uint32_t hg
     int khz = 0;
     if (cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, g.device) != cudaSuccess || khz <= 0) { khz = 2000000; cudaGetLastError(); }
     CU_TRY(h, launch_band_wait(counters, kBandCounterStride, n_ranks, value, band_timeout_word(g), 2000ll * khz,
-                               static_cast<cudaStream_t>(stream), band_signal_mode()));   // ~2 s
+                               static_cast<cudaStream_t>(stream)));   // ~2 s
     return MARAY_OK;
 }
 

@@ -39,13 +39,6 @@ struct Emitter {
     const Program& P;
     bool inline_trans;
     const std::vector<int32_t>* bank_index;   // value id -> index in the __constant__ table, or -1
-    // Use-ordered table (CodegenOptions::constants_in_use_order): every constant OPERAND gets the next entry, so
-    // the constants of neighbouring statements are neighbours in the bank.
-    std::vector<uint64_t>* use_bank = nullptr;
-    // In the per-pixel kernel a hoisted value is a load from its table: 1 = column table, 2 = row table.
-    const std::vector<uint8_t>* load_kind = nullptr;
-    const std::vector<uint32_t>* table_index = nullptr;
-    bool scratch_batches = false;
     std::string helper_suffix;      // which instance of the batch helpers this function calls ("" or "_sK")
     // Values that are exactly +0.0 or 1.0 at every pixel (see find_booleans): kind 1 = boolean,
     // kind 2 = the NOT pattern `1 + -(b)`.  Emitted as `bool` logic plus a double shadow.
@@ -62,7 +55,7 @@ struct Emitter {
         std::snprintf(buf, sizeof buf, "b%u", id);
         s += buf;
     }
-    // `const bool bN = vN != 0.0;` after a boolean value arrived as a double (frame import, table load)
+    // `const bool bN = vN != 0.0;` after a boolean value arrived as a double (frame import)
     void bool_from_double(std::string& s, uint32_t id) const {
         if (!is_bool(id)) return;
         char buf[64];
@@ -73,14 +66,7 @@ struct Emitter {
     void operand(std::string& s, uint32_t id) const {
         const Node& n = P.nodes[id];
         if (n.op == OP_CONST) {
-            if (bank_index && (*bank_index)[id] >= 0 && use_bank && use_bank->size() < 8000) {
-                char kb[24];
-                uint64_t bits;
-                std::memcpy(&bits, &n.k, 8);
-                std::snprintf(kb, sizeof kb, "MRK(%zu)", use_bank->size());
-                use_bank->push_back(bits);
-                s += kb;
-            } else if (bank_index && (*bank_index)[id] >= 0 && !use_bank) {
+            if (bank_index && (*bank_index)[id] >= 0) {
                 char kb[24];
                 std::snprintf(kb, sizeof kb, "MRK(%d)", (*bank_index)[id]);
                 s += kb;
@@ -94,43 +80,25 @@ struct Emitter {
         s += buf;
     }
 
-    // Emits order[i..j) -- one batch of same-kind transcendentals -- as x4 / x2 / single out-of-line
-    // calls.  The four (two) bodies inside a call are independent, which is where the FP64 pipe gets
-    // its instruction-level parallelism in transcendental-heavy programs.
+    // Emits order[i..j) -- one batch of same-kind transcendentals -- as out-of-line batch calls: arguments
+    // -> this thread's scratch rows, one leaf call for the whole batch, results back (rows: kScratchRows;
+    // lower.cpp's kBatchMax never exceeds it).  The evaluations inside a call are independent, which is where
+    // the FP64 pipe gets its instruction-level parallelism in transcendental-heavy programs.
     void batch_calls(std::string& s, const std::vector<uint32_t>& order, size_t i, size_t j) const {
         const char* fn = P.nodes[order[i]].op == OP_SIN ? "sin" : (P.nodes[order[i]].op == OP_EXP ? "exp" : "log");
         char buf[96];
-        if (scratch_batches) {
-            // arguments -> this thread's scratch rows, one leaf call for the whole batch, results back
-            // (rows: kScratchRows; lower.cpp's kBatchMax never exceeds it)
-            while (i < j) {
-                const size_t k = std::min<size_t>(j - i, kScratchRows);
-                if (k == 1) { statement(s, order[i]); i++; continue; }
-                for (size_t m = 0; m < k; m++) {
-                    std::snprintf(buf, sizeof buf, "  MR_S(%zu) = ", m);
-                    s += buf; operand(s, P.nodes[order[i + m]].a); s += ";\n";
-                }
-                std::snprintf(buf, sizeof buf, "  if (mr_%s_batch%s(%zuu)) mr_%s_fix%s(%zuu);\n", fn, helper_suffix.c_str(), k, fn,
-                              helper_suffix.c_str(), k);
-                s += buf;
-                for (size_t m = 0; m < k; m++) {
-                    std::snprintf(buf, sizeof buf, "  const double v%u = MR_R(%zu);\n", order[i + m], m);
-                    s += buf;
-                }
-                i += k;
-            }
-            return;
-        }
         while (i < j) {
-            size_t k = (j - i >= 4) ? 4 : ((j - i >= 2) ? 2 : 1);
+            const size_t k = std::min<size_t>(j - i, kScratchRows);
             if (k == 1) { statement(s, order[i]); i++; continue; }
-            std::snprintf(buf, sizeof buf, "  const MrD%zu b%u = mr_%s_x%zu(", k, order[i], fn, k);
-            s += buf;
-            for (size_t m = 0; m < k; m++) { if (m) s += ", "; operand(s, P.nodes[order[i + m]].a); }
-            s += ");\n";
-            static const char* fld[4] = {"a", "b", "c", "d"};
             for (size_t m = 0; m < k; m++) {
-                std::snprintf(buf, sizeof buf, "  const double v%u = b%u.%s;\n", order[i + m], order[i], fld[m]);
+                std::snprintf(buf, sizeof buf, "  MR_S(%zu) = ", m);
+                s += buf; operand(s, P.nodes[order[i + m]].a); s += ";\n";
+            }
+            std::snprintf(buf, sizeof buf, "  if (mr_%s_batch%s(%zuu)) mr_%s_fix%s(%zuu);\n", fn, helper_suffix.c_str(), k, fn,
+                          helper_suffix.c_str(), k);
+            s += buf;
+            for (size_t m = 0; m < k; m++) {
+                std::snprintf(buf, sizeof buf, "  const double v%u = MR_R(%zu);\n", order[i + m], m);
                 s += buf;
             }
             i += k;
@@ -142,13 +110,6 @@ struct Emitter {
         if (n.op == OP_X || n.op == OP_Y) return;   // kernel arguments
         if (is_sign_only(id)) return;               // its one consumer, a step, evaluates mr_sin_ge0 of the argument
         char buf[160];
-        if (load_kind && (*load_kind)[id]) {
-            if ((*load_kind)[id] == 1) std::snprintf(buf, sizeof buf, "  const double v%u = __ldg(CV + %uu * CW);\n", id, (*table_index)[id]);
-            else std::snprintf(buf, sizeof buf, "  const double v%u = __ldg(RV + %uu * RW);\n", id, (*table_index)[id]);
-            s += buf;
-            bool_from_double(s, id);
-            return;
-        }
         if (is_bool(id)) {
             // 0/1-valued: compares and bit logic instead of FP64 multiplies, min/max and selects.  The
             // double shadow is what every non-boolean consumer reads; unused shadows are dead code.
@@ -278,45 +239,16 @@ std::vector<uint8_t> find_sign_only_sines(const Program& prog, const std::vector
 //     accesses are coalesced).  The units share nothing, so NVRTC compiles them concurrently and nothing is
 //     linked, no segment pays a call ABI, and every kernel has the whole register file;
 //   * larger programs, !opt.chain: __noinline__ segment functions inside ONE unit with a per-thread frame in
-//     local memory (round 1's form; kept for A/B).
+//     local memory (round 1's form; what generate_cuda_source returns).
 std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt, CodegenInfo* info) {
-    // The per-pixel kernel evaluates the values that depend on both x and y; x-only / y-only frontier
-    // values are loaded from the column / row tables (each at its first use), the x-only / y-only
-    // values behind them are evaluated by the two prologue kernels only.
-    const bool hoist = opt.hoist && (!prog.col_values.empty() || !prog.row_values.empty());
-    std::vector<uint8_t> load_kind(prog.nodes.size(), 0);
-    std::vector<uint32_t> table_index(prog.nodes.size(), 0);
-    std::vector<uint32_t> order, order_batch;
-    if (hoist) {
-        for (size_t k = 0; k < prog.col_values.size(); k++) { load_kind[prog.col_values[k]] = 1; table_index[prog.col_values[k]] = uint32_t(k); }
-        for (size_t k = 0; k < prog.row_values.size(); k++) { load_kind[prog.row_values[k]] = 2; table_index[prog.row_values[k]] = uint32_t(k); }
-        std::vector<uint8_t> loaded(prog.nodes.size(), 0);
-        for (size_t i = 0; i < prog.order.size(); i++) {
-            uint32_t id = prog.order[i];
-            const Node& n = prog.nodes[id];
-            if (n.op == OP_X || n.op == OP_Y) continue;
-            if (n.dep == DEP_X || n.dep == DEP_Y) continue;          // prologue work
-            auto need = [&](uint32_t v) {
-                if (load_kind[v] && !loaded[v]) { loaded[v] = 1; order.push_back(v); order_batch.push_back(0); }
-            };
-            if (op_is_unary(n.op) || op_is_binary(n.op)) need(n.a);
-            if (op_is_binary(n.op)) need(n.b);
-            order.push_back(id);
-            order_batch.push_back(prog.batch.size() == prog.order.size() ? prog.batch[i] : 0);
-        }
-        for (int c = 0; c < 3; c++) {
-            uint32_t r = prog.root[c];
-            if (load_kind[r] && !loaded[r]) { loaded[r] = 1; order.push_back(r); order_batch.push_back(0); }
-        }
-    } else {
-        order = prog.order;
-        order_batch = prog.batch.size() == prog.order.size() ? prog.batch : std::vector<uint32_t>(prog.order.size(), 0);
-    }
+    const std::vector<uint32_t>& order = prog.order;
+    const std::vector<uint32_t> order_batch =
+        prog.batch.size() == prog.order.size() ? prog.batch : std::vector<uint32_t>(prog.order.size(), 0);
     uint64_t n_trans = prog.stats.op_count[OP_SIN] + prog.stats.op_count[OP_EXP] + prog.stats.op_count[OP_LN];
 
     const uint32_t cut_off = opt.segment_values ? opt.segment_values : 4096;
     bool segmented = order.size() > cut_off;
-    bool chain = segmented && opt.chain && !hoist;
+    bool chain = segmented && opt.chain;
     const uint32_t seg_len = chain ? std::max(256u, std::min(cut_off, opt.chain_segment_values)) : cut_off;
     if (chain && order.size() <= seg_len) segmented = chain = false;      // a chain of one kernel is a plain kernel
     // chain: cut into equal parts (the last kernel is not a stub)
@@ -368,7 +300,6 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         return t;
     };
     const Bank whole_bank = make_bank(0, 0, true);
-    const bool use_order = opt.constants_in_bank && opt.constants_in_use_order;
 
     Emitter em{prog, n_trans < opt.inline_transcendentals_below, opt.constants_in_bank ? &whole_bank.index : nullptr};
     const std::vector<uint8_t> booleans = opt.boolean_logic ? find_booleans(prog) : std::vector<uint8_t>();
@@ -381,20 +312,18 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         const uint32_t neg = prog.nodes[n.a].op == OP_NEG ? n.a : n.b;
         return prog.nodes[neg].a;
     };
-    // sign-only sines: unsegmented, unhoisted programs whose sines are not batched (the straight-line form)
+    // sign-only sines: unsegmented programs whose sines are not batched (the straight-line form)
     std::vector<uint8_t> sign_only;
-    if (opt.boolean_logic && opt.sign_of_sine && !segmented && !hoist) {
+    if (opt.boolean_logic && opt.sign_of_sine && !segmented) {
         sign_only = find_sign_only_sines(prog, booleans);
         for (size_t i = 0; i < order.size(); i++)
             if (order_batch[i] && sign_only[order[i]]) sign_only[order[i]] = 0;
         em.sign_only = &sign_only;
     }
-    Emitter em_pre = em;                       // prologue kernels compute hoisted values, never load them
-    if (hoist) { em.load_kind = &load_kind; em.table_index = &table_index; }
 
     uint32_t block = opt.block ? ((opt.block + 31) / 32) * 32 : 256;
     uint32_t min_blocks_per_sm = opt.min_blocks_per_sm;
-    if (opt.auto_shape && em.inline_trans && !segmented && !hoist && order.size() >= kOneBlockPerSmValues) {
+    if (opt.auto_shape && em.inline_trans && !segmented && order.size() >= kOneBlockPerSmValues) {
         block = 640;
         min_blocks_per_sm = 1;
         if (opt.frame_pixels_hint) {
@@ -407,18 +336,13 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             }
         }
     }
-    const bool persistent = opt.persistent && !segmented && !hoist && min_blocks_per_sm > 0;
     const bool use_batches = !em.inline_trans;
-    const bool scratch = use_batches && opt.scratch_batches;
-    em.scratch_batches = scratch;
     std::string prelude = "// generated by maray_b200 (NVRTC back end); compiled with --fmad=false\n";
     // one private instance of the batch helpers per segment function of a single-unit program
-    const bool private_helpers = scratch && segmented && !chain && opt.private_batch_helpers;
-    if (scratch) {
+    const bool private_helpers = use_batches && segmented && !chain;
+    if (use_batches) {
         if (private_helpers) prelude += "#define MR_NO_DEFAULT_BATCH_HELPERS 1\n";
         prelude += "#define MR_SCR_STRIDE " + std::to_string(block) + "\n";
-        prelude += "#define MR_BATCH_WIDTH " + std::to_string(opt.batch_width == 4 ? 4 : 2) + "\n";
-        if (opt.scratch_tables) prelude += "#define MR_SCR_TABLES 1\n";
     }
     prelude += kDeviceSemText;
     prelude += "\n";
@@ -433,10 +357,6 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
                           block, kJitKernelName, extra_args);
         out += buf;
         out += "  __shared__ unsigned int stage[3 * " + std::to_string(block) + " / 4];\n  (void)stage;\n";
-        if (persistent) {   // one resident block walks the band: blocks blockIdx.x, blockIdx.x + gridDim.x, ...
-            out += "  for (unsigned int blk = blockIdx.x; blk * blockDim.x < p.n; blk += gridDim.x) {\n";
-            out += "  const unsigned int j = blk * blockDim.x + threadIdx.x;\n";
-        } else
         out += "  const unsigned int j = blockIdx.x * blockDim.x + threadIdx.x;\n";
         out += "  const bool active = j < p.n;\n";
         out += "  const unsigned int pix = p.p0 + (active ? j : 0u);\n";   // idle lanes redo pixel p0
@@ -444,18 +364,18 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         out += "  const unsigned int xi = pix - yi * p.W;\n";
         out += "  const double X = (double)xi;\n  const double Y = (double)yi;\n";   // `x as f64`
         out += "  const MrTexture* __restrict__ T = p.tex;\n  (void)T;\n";
-        if (scratch) out += "  mr_scratch_tables_init();\n";
+        if (use_batches) out += "  mr_scratch_tables_init();\n";
     };
     auto store_call = [&](std::string& out, const std::vector<int32_t>& slot, const std::function<std::string(int32_t)>& frame_ref,
                           const Emitter& e, const std::vector<uint8_t>* in_scope) {
-        out += persistent ? "  mr_store_block_at(p, stage, " : "  mr_store_block(p, stage, ";
+        out += "  mr_store_block(p, stage, ";
         for (int c = 0; c < 3; c++) {
             uint32_t r = prog.root[c];
             if (slot[r] >= 0 && !(in_scope && (*in_scope)[r])) out += frame_ref(slot[r]);
             else e.operand(out, r);
             out += ", ";
         }
-        out += persistent ? "active, j, blk * blockDim.x);\n  __syncthreads();\n  }\n}\n" : "active, j);\n}\n";
+        out += "active, j);\n}\n";
     };
 
     std::vector<std::string> modules;
@@ -534,7 +454,6 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             else e.statement(out, order[i]);
             for (size_t m = i; m < j; m++) {
                 uint32_t id = order[m];
-                if (opt.sync_every && (m - lo) % opt.sync_every == opt.sync_every - 1) out += "  __syncthreads();\n";
                 if (segmented && slot[id] >= 0) {
                     std::snprintf(buf, sizeof buf, "  %s%s = v%u;\n", store_guard, frame_ref(slot[id]).c_str(), id);
                     out += buf;
@@ -555,9 +474,7 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             std::string unit;
             unit.reserve((seg_hi(s) - seg_lo(s)) * 56 + prelude.size() + 4096);
             unit += prelude;
-            Bank used;                                   // the use-ordered table is known once the body is written
-            const size_t bank_pos = unit.size();
-            if (use_order) e.use_bank = &used.bits; else unit += bank_text(bk);
+            unit += bank_text(bk);
             std::snprintf(buf, sizeof buf, "// segment %u of %u\n", s, n_seg);
             unit += buf;
             kernel_head(unit, ", double* __restrict__ F, const unsigned long long FS");
@@ -574,7 +491,6 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             emit_range(unit, e, seg_lo(s), seg_hi(s), gref, "if (active) ");
             if (last) store_call(unit, slot, gref, e, &in_scope);
             else unit += "}\n";
-            if (use_order) unit.insert(bank_pos, bank_text(used));
             modules.push_back(std::move(unit));
         }
     } else {
@@ -582,16 +498,12 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         std::string src;
         src.reserve(order.size() * 40 + 8192);
         src += prelude;
-        Bank used;
-        const size_t bank_pos = src.size();
-        const bool use_order_here = use_order && !segmented && !hoist;
-        if (use_order_here) em.use_bank = &used.bits; else src += bank_text(whole_bank);
+        src += bank_text(whole_bank);
         auto lref = [](int32_t f) { return "F[" + std::to_string(f) + "]"; };
         if (segmented) {
             for (uint32_t s = 0; s < n_seg; s++) {
                 static const char* const kSegArgs =
-                    "(double* __restrict__ F, const double X, const double Y, const MrTexture* __restrict__ T, "
-                    "const double* __restrict__ CV, const unsigned int CW, const double* __restrict__ RV, const unsigned int RW)";
+                    "(double* __restrict__ F, const double X, const double Y, const MrTexture* __restrict__ T)";
                 if (private_helpers) {
                     std::snprintf(buf, sizeof buf, "MR_BATCH_HELPERS(_s%u)\n", s);
                     src += buf;
@@ -610,47 +522,17 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             }
         }
         kernel_head(src, "");
-        src += "  const double* __restrict__ CV = p.colv + xi;\n  const unsigned int CW = p.W;\n";
-        src += "  const double* __restrict__ RV = p.rowv + (yi - p.row_base);\n  const unsigned int RW = p.rows;\n";
-        src += "  (void)CV; (void)CW; (void)RV; (void)RW;\n";
         if (segmented) {
             std::snprintf(buf, sizeof buf, "  double F[%u];\n", frame_slots ? frame_slots : 1);
             src += buf;
             for (uint32_t s = 0; s < n_seg; s++) {
-                std::snprintf(buf, sizeof buf, "  mr_seg%u(F, X, Y, T, CV, CW, RV, RW);\n", s);
+                std::snprintf(buf, sizeof buf, "  mr_seg%u(F, X, Y, T);\n", s);
                 src += buf;
             }
         } else {
             emit_range(src, em, 0, order.size(), lref, "");
         }
         store_call(src, slot, lref, em, nullptr);
-        if (use_order_here) { src.insert(bank_pos, bank_text(used)); em.use_bank = nullptr; }
-
-        // Prologue kernels: one thread per column / per row evaluates the x-only / y-only sub-program and
-        // stores its frontier values (k-major, so the per-pixel kernel's column loads are coalesced and
-        // its row loads are a broadcast).
-        if (hoist) {
-            for (int which = 1; which <= 2; which++) {
-                const bool colk = which == 1;
-                src += colk ? "extern \"C\" __global__ void maray_pre_x(double* __restrict__ tab, const unsigned int n, const unsigned int base, const MrTexture* __restrict__ T) {\n"
-                            : "extern \"C\" __global__ void maray_pre_y(double* __restrict__ tab, const unsigned int n, const unsigned int base, const MrTexture* __restrict__ T) {\n";
-                src += "  const unsigned int t = blockIdx.x * blockDim.x + threadIdx.x;\n  if (t >= n) return;\n  (void)T;\n";
-                src += colk ? "  const double X = (double)(base + t);\n" : "  const double Y = (double)(base + t);\n";
-                // Values that depend on neither coordinate but are not literals either (a texture fetch at
-                // constant coordinates and what is computed from it) may feed the x-only / y-only cone: both
-                // prologues evaluate them too (there are at most a handful).
-                for (uint32_t id : prog.order) {
-                    const Node& n = prog.nodes[id];
-                    if (n.op == OP_X || n.op == OP_Y || (n.dep != (colk ? DEP_X : DEP_Y) && n.dep != DEP_CONST)) continue;
-                    em_pre.statement(src, id);
-                    if (load_kind[id] == which) {
-                        std::snprintf(buf, sizeof buf, "  tab[%uu * n + t] = v%u;\n", table_index[id], id);
-                        src += buf;
-                    }
-                }
-                src += "}\n";
-            }
-        }
         modules.push_back(std::move(src));
     }
 
@@ -660,11 +542,8 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         info->frame_slots = segmented ? frame_slots : 0;
         info->transcendentals_inlined = em.inline_trans;
         info->block = block;
-        info->persistent_blocks_per_sm = persistent ? min_blocks_per_sm : 0;
-        info->n_col = hoist ? uint32_t(prog.col_values.size()) : 0;
-        info->n_row = hoist ? uint32_t(prog.row_values.size()) : 0;
-        info->dynamic_smem_bytes = scratch ? 2 * kScratchRows * block * uint32_t(sizeof(double)) : 0;   // argument rows + result rows
-        if (scratch && opt.scratch_tables) info->dynamic_smem_bytes += 4096;                            // + glibc's exp and log tables
+        // argument rows + result rows, then glibc's exp and log tables
+        info->dynamic_smem_bytes = use_batches ? 2 * kScratchRows * block * uint32_t(sizeof(double)) + 4096 : 0;
     }
     return modules;
 }

@@ -33,56 +33,26 @@ struct CodegenOptions {
     // frame best is taken: 1 024 x 1 024 pixels are 11.07 rounds of 640 (12 paid) but 6.92 rounds of 1 024.
     uint64_t frame_pixels_hint = 0;
     uint32_t sm_count_hint = 148;
-    // The kernel of an unsegmented program loops over the blocks of its band (grid = resident blocks) instead of
-    // being launched once per block: no block hand-over on the SM between two blocks (MARAY_JIT_PERSISTENT).
-    bool persistent = false;
     // Threads per block of the generated kernel (a multiple of 32; one pixel per thread).
     uint32_t block = 256;
     // __launch_bounds__ second argument: resident blocks per SM the register allocation must allow
     // (0 = leave it to ptxas).  2 x 256 threads caps the kernel at 128 registers = 16 resident warps
     // per SM, the best point of the sweep in profiles/ (ptxas left alone lands anywhere in 128..190).
     uint32_t min_blocks_per_sm = 2;
-    // A block-wide barrier every this many statements (0 = none).  The kernel is hundreds of KB of
-    // straight-line code, far beyond the instruction caches; keeping the warps of a block within
-    // one cache's reach of each other lets them share instruction fetches (DESIGN.md).
-    uint32_t sync_every = 0;
     // Scene constants live in a __constant__ table and are read as c[bank][offset] operands of the
     // FP64 instructions instead of being materialised with two 32-bit moves each.
     bool constants_in_bank = true;
-    // The table holds one entry per constant OPERAND, in statement order, instead of one per distinct constant:
-    // sm_100 has no constant-bank operands for FP64 instructions (every constant is an LDCU into a uniform register
-    // first), and neighbours in the table can share one 128-bit load.
-    bool constants_in_use_order = false;
-    // Evaluate x-only / y-only values once per column / row in prologue kernels and load them in the
-    // per-pixel kernel (the GPU form of the reference's row cache).  OFF by default: measured on
-    // B200 it LOSES (chess_4k 9.95 ms vs 7.77 ms, sdf 0.225 vs 0.184 ms) -- the 417 table loads per
-    // pixel cost more issue slots and exposed latency than the 1 227 mostly one-instruction values
-    // they replace.  Kept as MARAY_JIT_HOIST=1 for scenes with expensive x-only/y-only sub-programs.
-    bool hoist = false;
     // step(sin(u)) with no other reader of the sine evaluates only the sign of the sine (mr_sin_ge0): exact, and on
     // chess.maray a quarter of all instructions (MARAY_JIT_SIGN_OF_SINE=0 for A/B).
     bool sign_of_sine = true;
     // Programs above segment_values: one KERNEL per segment, each its own translation unit, values that cross
     // a cut in a global-memory frame F[slot * FS + pixel].  The units share nothing: NVRTC compiles them
     // concurrently, nothing is linked, no segment pays a call ABI.  false = __noinline__ segment functions in
-    // one unit with a per-thread local-memory frame (round 1's form, kept for A/B: MARAY_JIT_CHAIN=0).
+    // one unit with a per-thread local-memory frame (round 1's form: generate_cuda_source, MARAY_JIT_CHAIN=0).
     bool chain = true;
     // Size of a chain segment.  Smaller than segment_values on purpose: the cut-off decides WHETHER a program is
     // cut (below it one kernel is fastest), this decides how many units compile concurrently once it is.
     uint32_t chain_segment_values = 6144;
-    // Out-of-line sin/exp/ln batches pass arguments and results through per-thread rows of dynamic
-    // shared memory to leaf helpers (device_libm.cuh, "scratch-batched form") instead of through the
-    // call ABI's registers.  false = the register-argument x4/x2 helpers.
-    bool scratch_batches = true;
-    // The batch helpers read glibc's exp and log tables from shared memory (copied behind the scratch rows once per
-    // block) instead of global memory: two instructions fewer per value and a short-scoreboard latency.
-    bool scratch_tables = true;
-    // Independent evaluations per iteration of the batch helpers' loop (2 or 4).  4 since the sine lost its table
-    // loads and selects (measured, deep scene at 20 000 values: 13.4 ms against 13.8 with 2; with round 1's sine 4 did
-    // not pay: the helper has the ~38 registers its caller leaves).
-    uint32_t batch_width = 4;
-    // In a segmented single-unit program every segment function gets its own copy of the batch helpers.
-    bool private_batch_helpers = true;
     // Evaluate values that are exactly 0.0 or 1.0 at every pixel (step, products/min/max of such
     // values, 1 - b) as boolean logic instead of FP64 arithmetic.  Exact: no channel bit changes.
     bool boolean_logic = true;
@@ -94,16 +64,12 @@ struct CodegenInfo {
     uint32_t frame_slots = 0;       // doubles per pixel of the frame that carries values across cuts (0 when not segmented)
     bool transcendentals_inlined = true;
     uint32_t block = 256;           // threads per block the kernel must be launched with
-    uint32_t persistent_blocks_per_sm = 0;   // != 0: the kernel loops over blocks; launch at most SMs x this many
-    uint32_t n_col = 0, n_row = 0;  // doubles per column / per row in the hoisting tables (0 = no prologue)
-    uint32_t dynamic_smem_bytes = 0; // dynamic shared memory the kernel must be launched with (batch scratch)
+    uint32_t dynamic_smem_bytes = 0; // dynamic shared memory the kernel must be launched with (batch scratch + tables)
 };
 
 // Names of the generated kernels (extern "C").
 extern const char* const kJitKernelName;
 constexpr uint32_t kOneBlockPerSmValues = 4096;   // CodegenOptions::auto_shape
-constexpr const char* kJitPreXName = "maray_pre_x";
-constexpr const char* kJitPreYName = "maray_pre_y";
 
 // One translation unit (segment functions, if any, as __noinline__ functions of the same unit).
 std::string generate_cuda_source(const Program& prog, const CodegenOptions& opt, CodegenInfo* info);

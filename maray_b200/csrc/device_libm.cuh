@@ -21,17 +21,9 @@ MR_PLAIN_FN double mr_sin(double x) { return sin(x); }
 MR_PLAIN_FN double mr_exp(double x) { return exp(x); }
 MR_PLAIN_FN double mr_log(double x) { return log(x); }
 MR_PLAIN_FN int mr_sin_ge0(double x) { return sin(x) >= 0.0; }
-struct MrD2 { double a, b; };
-struct MrD4 { double a, b, c, d; };
-#define MR_DEFINE_BATCHED(fn)                                                                                   \
-    MR_PLAIN_FN double mr_##fn##_call(double a) { return mr_##fn(a); }                                          \
-    MR_PLAIN_FN MrD2 mr_##fn##_x2(double a, double b) { MrD2 r; r.a = mr_##fn(a); r.b = mr_##fn(b); return r; }  \
-    MR_PLAIN_FN MrD4 mr_##fn##_x4(double a, double b, double c, double d) {                                     \
-        MrD4 r; r.a = mr_##fn(a); r.b = mr_##fn(b); r.c = mr_##fn(c); r.d = mr_##fn(d); return r;               \
-    }
-MR_DEFINE_BATCHED(sin)
-MR_DEFINE_BATCHED(exp)
-MR_DEFINE_BATCHED(log)
+MR_PLAIN_FN double mr_sin_call(double a) { return mr_sin(a); }
+MR_PLAIN_FN double mr_exp_call(double a) { return mr_exp(a); }
+MR_PLAIN_FN double mr_log_call(double a) { return mr_log(a); }
 #ifdef MR_SCR_STRIDE
 #ifndef MR_DYN_DECL
 #define MR_DYN_DECL extern __shared__ double mr_dyn_f64[];
@@ -71,10 +63,7 @@ static inline int mr_hi32(double d) { uint64_t u; memcpy(&u, &d, 8); return (int
 static inline double mr_hilo(int hi, int lo) {
     uint64_t u = ((uint64_t)(uint32_t)hi << 32) | (uint32_t)lo; double d; memcpy(&d, &u, 8); return d;
 }
-static inline double mr_rcp_approx(double b) { return (double)(1.0f / (float)b); }   // >= 20 good bits, like MUFU.RCP64H
 #define MR_SLOW_SIN_F(x) sin(x)
-#define MR_SLOW_EXP_F(x) exp(x)
-#define MR_SLOW_LOG_F(x) log(x)
 #define MR_LDG2(p, lo, hi) do { (lo) = (p)[0]; (hi) = (p)[1]; } while (0)
 #else
 #define MR_FN __device__ __forceinline__
@@ -83,88 +72,45 @@ static inline double mr_rcp_approx(double b) { return (double)(1.0f / (float)b);
 __device__ __forceinline__ int mr_lo32(double d) { return __double2loint(d); }
 __device__ __forceinline__ int mr_hi32(double d) { return __double2hiint(d); }
 __device__ __forceinline__ double mr_hilo(int hi, int lo) { return __hiloint2double(hi, lo); }
-__device__ __forceinline__ double mr_rcp_approx(double b) {
-    double y;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(b));
-    return y;
-}
-// Out-of-range arguments go to libdevice, out of line so the call sites stay small.
+// Out-of-range arguments of the fast sine go to libdevice, out of line so the call sites stay small.
 static __device__ __noinline__ double mr_slow_sin(double x) { return sin(x); }
-static __device__ __noinline__ double mr_slow_exp(double x) { return exp(x); }
-static __device__ __noinline__ double mr_slow_log(double x) { return log(x); }
 #define MR_SLOW_SIN_F(x) mr_slow_sin(x)
-#define MR_SLOW_EXP_F(x) mr_slow_exp(x)
-#define MR_SLOW_LOG_F(x) mr_slow_log(x)
 #define MR_LDG2(p, lo, hi) do { double2 v2_ = __ldg(reinterpret_cast<const double2*>(p)); (lo) = v2_.x; (hi) = v2_.y; } while (0)
 #endif
 
 #include "device_libm_glibc.cuh"   // glibc's routines: mr_*_inrange_g, mr_*_fast_g, mr_*_slow_g (exp and log ARE these)
 
-// Constants, read as constant-bank operands.
+// Constants, read as constant-bank operands.  The compiler fetches two neighbours that share a 16-byte line with one
+// LDCU.128, so where the entries sit relative to those lines shapes the code: entry 1 is unused and keeps 1/pi and the
+// pi parts in the pairs they were measured in, and an odd entry count keeps the scene's constant table (MRK_BITS, next
+// in the bank) on the same alignment.  Dropping entry 1 doubled chess's per-thread constant loads (LDC.64).
 MR_TABLE double MR_LK[] = {
     /* 0 */ 0x1.8p52,                    // round-to-integer magic (1.5 * 2^52)
-    /* 1 */ 0x1.45f306dc9c883p-1,        // 2/pi
-    /* 2 */ 0x1.921fb54442d18p+0,        // pi/2 high
-    /* 3 */ 0x1.1a62633145c06p-54,       // pi/2 middle (one ulp short, so the tail below is positive:
-    /* 4 */ 0x1.c1cd129024e09p-107,      //   all three products of a +0 quotient are -0 and sin(-0) stays -0)
-    /* 5 */ 0x1.71547652b82fep+0,        // log2(e)
-    /* 6 */ 0x1.62e42fefa39efp-1,        // ln2 high
-    /* 7 */ 0x1.abc9e3b39803fp-56,       // ln2 low
-    // exp: (exp(r) - 1 - r)/r^2 on |r| <= ln2/2, degree 10, highest first
-    /* 8 */ 0x1.1f7919372ca92p-29, 0x1.af4f1961bbff2p-26, 0x1.27e4d7fddc246p-22, 0x1.71de018a4e96dp-19,
-    /* 12 */ 0x1.a01a01a82049dp-16, 0x1.a01a01ac27468p-13, 0x1.6c16c16c15fefp-10, 0x1.1111111110045p-7,
-    /* 16 */ 0x1.5555555555556p-5, 0x1.5555555555557p-3, 0x1.0000000000000p-1,
-    // log: (2 atanh(u/2) - u)/u^3 in w = u^2, degree 6, highest first
-    /* 19 */ 0x1.2b66d75b2a50ap-18, 0x1.39fd38054ec10p-16, 0x1.7462bd51227ffp-14, 0x1.c71c62c8e6f51p-12,
-    /* 23 */ 0x1.2492492e04b98p-9, 0x1.999999999527bp-7, 0x1.5555555555558p-4,
-    // leading coefficients of the sin / cos chains (selected by parity with FSEL)
-    /* 26 */ -0x1.8dc40a95e2836p-41,     // sin S6
-    /* 27 */ -0x1.9000fc0d9bc33p-37,     // cos C6
-    // reduction by pi (sign of the sine): entries 1..4 scaled by powers of two, so the same 160 bits
-    /* 28 */ 0x1.45f306dc9c883p-2,       // 1/pi
-    /* 29 */ 0x1.921fb54442d18p+1,       // pi high
-    /* 30 */ 0x1.1a62633145c06p-53,      // pi middle
-    /* 31 */ 0x1.c1cd129024e09p-106,     // pi low
+    /* 1 */ 0.0,                         // unused: alignment (above)
+    // reduction by pi: 160 bits of pi in three parts, the first product exact (pi middle is one ulp short, so the tail
+    // is positive: all three products of a +0 quotient are -0 and sin(-0) stays -0)
+    /* 2 */ 0x1.45f306dc9c883p-2,        // 1/pi
+    /* 3 */ 0x1.921fb54442d18p+1,        // pi high
+    /* 4 */ 0x1.1a62633145c06p-53,       // pi middle
+    /* 5 */ 0x1.c1cd129024e09p-106,      // pi low
     // sin(r) = r + r*s*S(s), s = r*r, |r| <= pi/2: S of degree 8, lowest first (relative error 2^-58.7; tools/gen_libm_coeffs.py)
-    /* 32 */ -0x1.5555555555555p-3, 0x1.11111111110a9p-7, -0x1.a01a01a010c5cp-13, 0x1.71de3a4f8ab99p-19,
-    /* 36 */ -0x1.ae64528659a2dp-26, 0x1.6122db98108c0p-33, -0x1.add52c09d1f58p-41, 0x1.6dc19ddd0cdfbp-49,
-    /* 40 */ 0x1.4b52654981457p-56,
+    /* 6 */ -0x1.5555555555555p-3, 0x1.11111111110a9p-7, -0x1.a01a01a010c5cp-13, 0x1.71de3a4f8ab99p-19,
+    /* 10 */ -0x1.ae64528659a2dp-26, 0x1.6122db98108c0p-33, -0x1.add52c09d1f58p-41, 0x1.6dc19ddd0cdfbp-49,
+    /* 14 */ 0x1.4b52654981457p-56,
 };
 
-// Remaining coefficients of the two chains, highest first, one 48-byte row per parity (16-byte
-// aligned for 128-bit loads).  Row 0 (even quadrant): sin S5..S0.  Row 1 (odd quadrant): cos C5..C0.
-//   sin(r) = r + r*(s*S(s)),  cos(r) = 1 + s*C(s),  s = r*r, |r| <= pi/4
-#ifdef MR_LIBM_HOST
-static const double MR_SINCOS[2][6] = {
-#else
-static __device__ __align__(16) const double MR_SINCOS[2][6] = {
-#endif
-    {0x1.60e694a9b66dap-33, -0x1.ae63f90709ef2p-26, 0x1.71de3a10d6808p-19, -0x1.a01a019fe8dc5p-13,
-     0x1.111111111101fp-7, -0x1.5555555555555p-3},
-    {0x1.1eea8e2e9e889p-29, -0x1.27e4f8fcf0849p-22, 0x1.a01a019e06f51p-16, -0x1.6c16c16c15f43p-10,
-     0x1.5555555555552p-5, -0x1.0000000000000p-1},
-};
-
-// sin(x).  Fast range |x| < 2^22: Cody-Waite reduction by pi/2 with three FMAs, quadrant from the
-// low bits of the magic sum, one 7-step Horner chain whose coefficients depend on the quadrant's
-// parity.  Everything else (incl. NaN, infinity) goes to libdevice.
+// Fast range of the sine: |x| < 2^22.  Everything else (incl. NaN, infinity) goes to libdevice.
 // The range tests look at the high word only (integer pipe, not the FP64 pipe); NaN and infinity
 // have a high word above every bound, so they always take the libdevice branch.
 MR_FN int mr_sin_inrange_f(double x) { return (unsigned int)(mr_hi32(x) & 0x7fffffff) < 0x41500000u; }   // |x| < 2^22
-#ifdef MR_EXPLOG_POLY   /* A/B only: round 1's polynomial exp and log */
-MR_FN int mr_exp_inrange_f(double x) { return (unsigned int)(mr_hi32(x) & 0x7fffffff) < 0x40862000u; }   // |x| < 708
-MR_FN int mr_log_inrange_f(double x) { return (unsigned int)(mr_hi32(x) - 0x00100000) < 0x7fe00000u; }   // positive normal
-#else
 // exp and log are glibc's algorithms in every mode (device_libm_glibc.cuh): fewer FP64 instructions than the
 // polynomial versions they replaced (12 and 15 against 17 and 30), dependency chains half as long -- which is what
 // bounds the batched helpers -- and the reference's bits.  exp: |x| < 512; tiny arguments need no special case here
 // (for |x| < 2^-54 the main path rounds 1 + x + x^2/2.. to exactly what glibc's early `1.0 + x` returns).
 MR_FN int mr_exp_inrange_f(double x) { return (unsigned int)((mr_hi32(x) >> 20) & 0x7ff) < 0x408u; }
 MR_FN int mr_log_inrange_f(double x) { return mr_log_inrange_g(x); }
-#endif
 
 // Straight-line fast paths: safe (no traps, no loops) for ANY argument, meaningful inside the range.
-#ifndef MR_SIN_PARITY
 // sin(x), fast version: x = k*pi + r, |r| <= pi/2 (three FMAs over 160 bits of pi, the first product exact),
 // sin(x) = (-1)^k (r + r*s*S(s)).  One polynomial for every argument -- no parity-dependent coefficient rows, hence no
 // table loads and no selects --, evaluated by Estrin's scheme: eight FMAs in four dependent steps.  More FP64 instructions
@@ -172,126 +118,29 @@ MR_FN int mr_log_inrange_f(double x) { return mr_log_inrange_g(x); }
 // overall, which is what counts in the batched helpers (latency-bound: DESIGN.md 3.1).  sin(-0) = -0: S*s is made +0 by
 // an explicit +0.0 addend, so the last FMA adds (-0) to (-0).
 MR_FN double mr_sin_fast_f(double x) {
-    const double t = MR_FMA(x, MR_LK[28], MR_LK[0]);
+    const double t = MR_FMA(x, MR_LK[2], MR_LK[0]);
     const double k = t - MR_LK[0];
-    double r = MR_FMA(k, -MR_LK[29], x);
-    r = MR_FMA(k, -MR_LK[30], r);
-    r = MR_FMA(k, -MR_LK[31], r);
+    double r = MR_FMA(k, -MR_LK[3], x);
+    r = MR_FMA(k, -MR_LK[4], r);
+    r = MR_FMA(k, -MR_LK[5], r);
     const double s = r * r;
     // the six high coefficients by Estrin's scheme (three independent FMAs, then two steps), the three low ones by
     // Horner's: the low end decides the rounding error, the high end the length of the chain
-    const double p34 = MR_FMA(MR_LK[36], s, MR_LK[35]);
-    const double p56 = MR_FMA(MR_LK[38], s, MR_LK[37]);
-    const double p78 = MR_FMA(MR_LK[40], s, MR_LK[39]);
+    const double p34 = MR_FMA(MR_LK[10], s, MR_LK[9]);
+    const double p56 = MR_FMA(MR_LK[12], s, MR_LK[11]);
+    const double p78 = MR_FMA(MR_LK[14], s, MR_LK[13]);
     const double s2 = s * s;
     double S = MR_FMA(p56, s2, p34);
     S = MR_FMA(p78, s2 * s2, S);
-    S = MR_FMA(S, s, MR_LK[34]);
-    S = MR_FMA(S, s, MR_LK[33]);
-    S = MR_FMA(S, s, MR_LK[32]);
+    S = MR_FMA(S, s, MR_LK[8]);
+    S = MR_FMA(S, s, MR_LK[7]);
+    S = MR_FMA(S, s, MR_LK[6]);
     const double v = MR_FMA(MR_FMA(S, s, 0.0), r, r);
     return mr_hilo((int)((unsigned int)mr_hi32(v) ^ ((unsigned int)mr_lo32(t) << 31)), mr_lo32(v));   // odd k: negate
 }
-#else   /* A/B only: round 1's sine (reduction by pi/2, one 7-step chain chosen by the quadrant's parity) */
-MR_FN double mr_sin_fast_f(double x) {
-    const double t = MR_FMA(x, MR_LK[1], MR_LK[0]);
-    const double q = t - MR_LK[0];
-    double r = MR_FMA(q, -MR_LK[2], x);
-    r = MR_FMA(q, -MR_LK[3], r);
-    r = MR_FMA(q, -MR_LK[4], r);
-    const int qi = mr_lo32(t);
-    const int odd = qi & 1;
-    const double s = r * r;
-    double k6, k5, k4, k3, k2, k1;
-    const double* row = MR_SINCOS[odd];
-    MR_LDG2(row + 0, k6, k5);
-    MR_LDG2(row + 2, k4, k3);
-    MR_LDG2(row + 4, k2, k1);
-    double p = odd ? MR_LK[27] : MR_LK[26];
-    p = MR_FMA(p, s, k6);
-    p = MR_FMA(p, s, k5);
-    p = MR_FMA(p, s, k4);
-    p = MR_FMA(p, s, k3);
-    p = MR_FMA(p, s, k2);
-    p = MR_FMA(p, s, k1);
-    p = MR_FMA(p, s, odd ? 1.0 : 0.0);          // odd: cos(r) = 1 + s*C(s); even: s*S(s)
-    const double sn = MR_FMA(p, r, r);          // even: sin(r) = r + r*(s*S(s))
-    const double v = odd ? p : sn;
-    return mr_hilo((int)((unsigned int)mr_hi32(v) ^ (((unsigned int)qi & 2u) << 30)), mr_lo32(v));   // quadrants 2,3: negate
-}
 
-#endif  // MR_SIN_PARITY
-
-#ifndef MR_EXPLOG_POLY
 MR_FN double mr_exp_fast_f(double x) { return mr_exp_fast_g(x); }
 MR_FN double mr_log_fast_f(double x) { return mr_log_fast_g(x); }
-#undef MR_SLOW_EXP_F
-#undef MR_SLOW_LOG_F
-#define MR_SLOW_EXP_F(x) mr_exp_slow_g(x)
-#define MR_SLOW_LOG_F(x) mr_log_slow_g(x)
-#else
-// exp(x).  Fast range |x| < 708: n = rint(x*log2(e)), r = x - n*ln2 (two FMAs), degree-12 polynomial,
-// scaling by 2^n through the exponent field.
-MR_FN double mr_exp_fast_f(double x) {
-    const double t = MR_FMA(x, MR_LK[5], MR_LK[0]);
-    const double n = t - MR_LK[0];
-    double r = MR_FMA(n, -MR_LK[6], x);
-    r = MR_FMA(n, -MR_LK[7], r);
-    double p = MR_LK[8];
-    p = MR_FMA(p, r, MR_LK[9]);
-    p = MR_FMA(p, r, MR_LK[10]);
-    p = MR_FMA(p, r, MR_LK[11]);
-    p = MR_FMA(p, r, MR_LK[12]);
-    p = MR_FMA(p, r, MR_LK[13]);
-    p = MR_FMA(p, r, MR_LK[14]);
-    p = MR_FMA(p, r, MR_LK[15]);
-    p = MR_FMA(p, r, MR_LK[16]);
-    p = MR_FMA(p, r, MR_LK[17]);
-    p = MR_FMA(p, r, MR_LK[18]);
-    p = MR_FMA(p, r, 1.0);
-    p = MR_FMA(p, r, 1.0);
-    return mr_hilo((int)((unsigned int)mr_hi32(p) + ((unsigned int)mr_lo32(t) << 20)), mr_lo32(p));
-}
-
-// log(x).  Fast range: positive normal finite x.  x = m * 2^e with m in [sqrt(1/2), sqrt(2));
-// u = 2(m-1)/(m+1) from an approximate reciprocal refined by two Newton steps, with the exact
-// remainder of that division carried as u_lo; log(m) = u + u_lo + u^3*Q(u^2); the sum with e*ln2
-// is compensated.
-MR_FN double mr_log_fast_f(double x) {
-    const int hx = mr_hi32(x);
-    int e = (hx >> 20) - 1023;
-    int mh = (hx & 0x000fffff) | 0x3ff00000;
-    if (mh >= 0x3ff6a09f) { mh -= 0x00100000; e += 1; }
-    const double m = mr_hilo(mh, mr_lo32(x));
-    const double a = m - 1.0;                   // exact
-    const double b = m + 1.0;
-    double y = mr_rcp_approx(b);
-    double er = MR_FMA(-b, y, 1.0);
-    y = MR_FMA(y, er, y);
-    er = MR_FMA(-b, y, 1.0);
-    y = MR_FMA(y, er, y);
-    const double qq = a * y;
-    const double u = qq + qq;
-    const double d = a - u;
-    const double rem = MR_FMA(a, -u, d + d);    // 2a - u*(a+2), exact m+1 = a+2
-    const double u_lo = y * rem;
-    const double w = u * u;
-    double Q = MR_LK[19];
-    Q = MR_FMA(Q, w, MR_LK[20]);
-    Q = MR_FMA(Q, w, MR_LK[21]);
-    Q = MR_FMA(Q, w, MR_LK[22]);
-    Q = MR_FMA(Q, w, MR_LK[23]);
-    Q = MR_FMA(Q, w, MR_LK[24]);
-    Q = MR_FMA(Q, w, MR_LK[25]);
-    const double t3 = MR_FMA(u * w, Q, u_lo);
-    const double ed = (double)e;
-    const double h = MR_FMA(ed, MR_LK[6], u);
-    const double c = MR_FMA(ed, MR_LK[6], -h) + u;
-    const double lo = MR_FMA(ed, MR_LK[7], t3) + c;
-    return h + lo;
-}
-#endif  // MR_EXPLOG_POLY
-
 
 // Which implementation the names below mean.  Default: the fast versions above.  MR_LIBM_GLIBC (MARAY_LIBM=glibc):
 // the exact mode of device_libm_glibc.cuh.  MR_LIBM_BOTH (the interpreter kernel, which is compiled ahead of time and
@@ -299,14 +148,12 @@ MR_FN double mr_log_fast_f(double x) {
 #ifdef MR_LIBM_GLIBC
 #define MR_SEL(name) name##_g
 #define MR_SLOW_SIN(x) mr_sin_slow_g(x)
-#define MR_SLOW_EXP(x) mr_exp_slow_g(x)
-#define MR_SLOW_LOG(x) mr_log_slow_g(x)
 #else
 #define MR_SEL(name) name##_f
 #define MR_SLOW_SIN(x) MR_SLOW_SIN_F(x)
-#define MR_SLOW_EXP(x) MR_SLOW_EXP_F(x)
-#define MR_SLOW_LOG(x) MR_SLOW_LOG_F(x)
 #endif
+#define MR_SLOW_EXP(x) mr_exp_slow_g(x)
+#define MR_SLOW_LOG(x) mr_log_slow_g(x)
 #define MR_DEFINE_SELECTED(fn)                                                          \
     MR_FN int mr_##fn##_inrange(double x) { return MR_SEL(mr_##fn##_inrange)(x); }      \
     MR_FN double mr_##fn##_fast(double x) { return MR_SEL(mr_##fn##_fast)(x); }
@@ -328,9 +175,7 @@ MR_FN double mr_sin(double x) {
     return mr_sin_fast(x);
 #else
     double r = mr_sin_fast(x);
-#ifndef MR_NO_SLOW   /* experiment only: measures what the out-of-range branches cost */
     if (MR_UNLIKELY(!mr_sin_inrange(x))) r = MR_SLOW_SIN(x);
-#endif
     return r;
 #endif
 }
@@ -345,9 +190,7 @@ MR_FN double mr_exp(double x) {
     return mr_exp_fast(x);
 #else
     double r = mr_exp_fast(x);
-#ifndef MR_NO_SLOW   /* experiment only: measures what the out-of-range branches cost */
     if (MR_UNLIKELY(!mr_exp_inrange(x))) r = MR_SLOW_EXP(x);
-#endif
     return r;
 #endif
 }
@@ -361,9 +204,7 @@ MR_FN double mr_log(double x) {
     return mr_log_fast(x);
 #else
     double r = mr_log_fast(x);
-#ifndef MR_NO_SLOW   /* experiment only: measures what the out-of-range branches cost */
     if (MR_UNLIKELY(!mr_log_inrange(x))) r = MR_SLOW_LOG(x);
-#endif
     return r;
 #endif
 }
@@ -373,18 +214,17 @@ MR_FN double mr_log_eo(double x) {
 }
 
 // mr_sin(x) >= 0.0 without the sine: what `step(sin(u))` needs (Maray's `chess`, reference src/lib.rs:969-973).
-// x = k*pi + r with |r| <= pi/2 (the Cody-Waite reduction of mr_sin_fast_f, by pi instead of pi/2: the same 160 bits
-// of pi, first product exact): sin(x) = (-1)^k sin(r), and sin(r) has the sign of r and is +-0 exactly when r is.  The
+// x = k*pi + r with |r| <= pi/2 (the Cody-Waite reduction of mr_sin_fast_f: 160 bits of pi, first product exact): sin(x) = (-1)^k sin(r), and sin(r) has the sign of r and is +-0 exactly when r is.  The
 // reduced argument of a nonzero double is never closer to zero than ~2^-60 while r is good to ~2^-100 absolute here, so
 // the sign of r IS the sign of the true sine -- which every sine with a relative error bound returns, the fast one
 // above, libdevice's and glibc's (exact mode) alike.  Checked against both on the host (tools/glibc_libm_check.c, all
 // ranges and the neighbourhoods of 8 000 multiples of pi/2).  Outside |x| < 2^22: the full routine.
 MR_FN int mr_sin_ge0_fast(double x) {
-    const double t = MR_FMA(x, MR_LK[28], MR_LK[0]);
+    const double t = MR_FMA(x, MR_LK[2], MR_LK[0]);
     const double k = t - MR_LK[0];
-    double r = MR_FMA(k, -MR_LK[29], x);
-    r = MR_FMA(k, -MR_LK[30], r);
-    r = MR_FMA(k, -MR_LK[31], r);
+    double r = MR_FMA(k, -MR_LK[3], x);
+    r = MR_FMA(k, -MR_LK[4], r);
+    r = MR_FMA(k, -MR_LK[5], r);
     // r, or -r for odd k; -0 >= 0 holds, as step(-0.0) = 1 requires
     return mr_hilo((int)((unsigned int)mr_hi32(r) ^ ((unsigned int)mr_lo32(t) << 31)), mr_lo32(r)) >= 0.0;
 }
@@ -395,52 +235,38 @@ static __device__ __noinline__ int mr_sin_ge0_slow(double x) { return mr_sin_eo(
 #endif
 MR_FN int mr_sin_ge0(double x) {
     int ge = mr_sin_ge0_fast(x);                 // safe for any argument; repaired below (the cold block goes out of line)
-#ifndef MR_NO_SLOW   /* experiment only: measures what the out-of-range branches cost */
     if (MR_UNLIKELY(!mr_sin_inrange_f(x))) ge = mr_sin_ge0_slow(x);
-#endif
     return ge;
 }
 
 #ifndef MR_LIBM_HOST
-// Batched forms for the out-of-line path of the NVRTC back end: two or four independent evaluations
-// per call give the FP64 pipe independent dependency chains and amortise the call.  (A variant that
-// ran all fast paths first and repaired out-of-range arguments in one shared branch measured 35 %
-// slower: the results stay live across the possible libdevice calls and get spilled.)
-struct MrD2 { double a, b; };
-struct MrD4 { double a, b, c, d; };
-#define MR_DEFINE_BATCHED(fn)                                                                          \
-    static __device__ __noinline__ double mr_##fn##_call(double a) { return mr_##fn##_eo(a); }         \
-    static __device__ __noinline__ MrD2 mr_##fn##_x2(double a, double b) {                             \
-        MrD2 r; r.a = mr_##fn##_eo(a); r.b = mr_##fn##_eo(b); return r;                                \
-    }                                                                                                  \
-    static __device__ __noinline__ MrD4 mr_##fn##_x4(double a, double b, double c, double d) {         \
-        MrD4 r; r.a = mr_##fn##_eo(a); r.b = mr_##fn##_eo(b); r.c = mr_##fn##_eo(c); r.d = mr_##fn##_eo(d); return r; \
-    }
-MR_DEFINE_BATCHED(sin)
-MR_DEFINE_BATCHED(exp)
-MR_DEFINE_BATCHED(log)
+// One out-of-line evaluation: what the NVRTC back end emits for a transcendental that is not in a batch.
+static __device__ __noinline__ double mr_sin_call(double a) { return mr_sin_eo(a); }
+static __device__ __noinline__ double mr_exp_call(double a) { return mr_exp_eo(a); }
+static __device__ __noinline__ double mr_log_call(double a) { return mr_log_eo(a); }
 
 // Scratch-batched form (the NVRTC back end's default for transcendental-heavy programs).  Arguments
 // and results travel through a per-thread column of dynamic shared memory, MR_S(k) = row k of this
 // thread, instead of the call ABI's fixed registers: one STS + one LDS per value replaces four moves,
-// and the helper is a LEAF with a two-wide loop -- no nested call, so nothing has to survive one, no
-// callee-saved registers are touched and nothing is spilled (the register-argument x4 helpers above
-// spend 4/5 of their instructions on exactly that).  The loop body is a few hundred bytes and stays
-// in the instruction cache, which is what bounds straight-line code of this size (DESIGN.md 3.1).
+// and the helper is a LEAF with a four-wide loop -- no nested call, so nothing has to survive one, no
+// callee-saved registers are touched and nothing is spilled (helpers that took four arguments and
+// returned four results in the call ABI's registers spent 4/5 of their instructions on exactly that).
+// The loop body is a few hundred bytes and stays in the instruction cache, which is what bounds
+// straight-line code of this size (DESIGN.md 3.1).
 // Out-of-range arguments are left in place and reported in the returned mask; the caller hands the
 // mask to mr_*_fix (libdevice), a call that is practically never executed.
 #ifdef MR_SCR_STRIDE
 extern __shared__ double mr_dyn_f64[];
 #define MR_S(k) mr_dyn_f64[(k) * MR_SCR_STRIDE + threadIdx.x]
-#ifndef MR_BATCH_WIDTH
-#define MR_BATCH_WIDTH 2      /* independent evaluations per loop iteration (2 or 4; the scratch has 8 rows) */
-#endif
-#define MR_W MR_BATCH_WIDTH
+// Independent evaluations per loop iteration (the scratch has 8 rows).  4 since the sine lost its table loads and
+// selects (measured, deep scene at 20 000 values: 13.4 ms against 13.8 with 2; with round 1's sine 4 did not pay: the
+// helper has the ~38 registers its caller leaves).
+#define MR_W 4
 #define MR_EACH _Pragma("unroll") for (int i = 0; i < MR_W; i++)
-// MR_SCR_TABLES: glibc's exp and log tables (2 KB each) sit in shared memory behind the 16 scratch rows, copied there
-// once per block by mr_scratch_tables_init().  A lookup is then one LDS.128 at a 32-bit offset instead of a 64-bit
-// address computation (IADD3 + IMAD.X) and an LDG whose latency is the long scoreboard's.
-#ifdef MR_SCR_TABLES
+// glibc's exp and log tables (2 KB each) sit in shared memory behind the 16 scratch rows, copied there once per block
+// by mr_scratch_tables_init().  A lookup is then one LDS.128 at a 32-bit offset instead of a 64-bit address computation
+// (IADD3 + IMAD.X) and an LDG whose latency is the long scoreboard's (measured, deep scene at 20 000 values: 12.87 ms
+// against 13.35 with the tables in global memory).
 #define MR_TAB_EXP (reinterpret_cast<const unsigned long long*>(mr_dyn_f64 + 16 * MR_SCR_STRIDE))
 #define MR_TAB_LOG (mr_dyn_f64 + 16 * MR_SCR_STRIDE + 256)
 #define MR_TAB_LD2U(p, a, b) do { const ulonglong2 v2_ = *reinterpret_cast<const ulonglong2*>(p); (a) = v2_.x; (b) = v2_.y; } while (0)
@@ -452,132 +278,33 @@ __device__ __forceinline__ void mr_scratch_tables_init() {
     }
     __syncthreads();
 }
-#else
-#define MR_TAB_EXP MRG_EXP_TAB
-#define MR_TAB_LOG MRG_LOG_TAB
-#define MR_TAB_LD2U(p, a, b) MRG_LDG2U(p, a, b)
-#define MR_TAB_LD2(p, a, b) MR_LDG2(p, a, b)
-__device__ __forceinline__ void mr_scratch_tables_init() {}
-#endif
 // The fast paths again, MR_W evaluations at a time and written STEP-MAJOR: every step is applied to
 // all lanes before the next one, so the lanes' dependent DFMA chains are interleaved in program order.
 // (Left to itself the compiler emits one whole chain after the other -- measured: 47 % of the helpers'
 // cycles were fixed-latency waits on the previous DFMA with 4 warps per scheduler.)  Same operations in
 // the same order per lane as mr_sin_fast / mr_exp_fast / mr_log_fast: bit-identical results.
-#ifndef MR_SIN_PARITY
 __device__ __forceinline__ void mr_sin_fast_w_f(const double* x, double* out) {
     double t[MR_W], k[MR_W], r[MR_W], s[MR_W], p34[MR_W], p56[MR_W], p78[MR_W], s2[MR_W], S[MR_W];
-    MR_EACH t[i] = MR_FMA(x[i], MR_LK[28], MR_LK[0]);
+    MR_EACH t[i] = MR_FMA(x[i], MR_LK[2], MR_LK[0]);
     MR_EACH k[i] = t[i] - MR_LK[0];
-    MR_EACH r[i] = MR_FMA(k[i], -MR_LK[29], x[i]);
-    MR_EACH r[i] = MR_FMA(k[i], -MR_LK[30], r[i]);
-    MR_EACH r[i] = MR_FMA(k[i], -MR_LK[31], r[i]);
+    MR_EACH r[i] = MR_FMA(k[i], -MR_LK[3], x[i]);
+    MR_EACH r[i] = MR_FMA(k[i], -MR_LK[4], r[i]);
+    MR_EACH r[i] = MR_FMA(k[i], -MR_LK[5], r[i]);
     MR_EACH s[i] = r[i] * r[i];
-    MR_EACH p34[i] = MR_FMA(MR_LK[36], s[i], MR_LK[35]);
-    MR_EACH p56[i] = MR_FMA(MR_LK[38], s[i], MR_LK[37]);
-    MR_EACH p78[i] = MR_FMA(MR_LK[40], s[i], MR_LK[39]);
+    MR_EACH p34[i] = MR_FMA(MR_LK[10], s[i], MR_LK[9]);
+    MR_EACH p56[i] = MR_FMA(MR_LK[12], s[i], MR_LK[11]);
+    MR_EACH p78[i] = MR_FMA(MR_LK[14], s[i], MR_LK[13]);
     MR_EACH s2[i] = s[i] * s[i];
     MR_EACH S[i] = MR_FMA(p56[i], s2[i], p34[i]);
     MR_EACH S[i] = MR_FMA(p78[i], s2[i] * s2[i], S[i]);
-    MR_EACH S[i] = MR_FMA(S[i], s[i], MR_LK[34]);
-    MR_EACH S[i] = MR_FMA(S[i], s[i], MR_LK[33]);
-    MR_EACH S[i] = MR_FMA(S[i], s[i], MR_LK[32]);
+    MR_EACH S[i] = MR_FMA(S[i], s[i], MR_LK[8]);
+    MR_EACH S[i] = MR_FMA(S[i], s[i], MR_LK[7]);
+    MR_EACH S[i] = MR_FMA(S[i], s[i], MR_LK[6]);
     MR_EACH {
         const double v = MR_FMA(MR_FMA(S[i], s[i], 0.0), r[i], r[i]);
         out[i] = mr_hilo((int)((unsigned int)mr_hi32(v) ^ ((unsigned int)mr_lo32(t[i]) << 31)), mr_lo32(v));
     }
 }
-#else
-__device__ __forceinline__ void mr_sin_fast_w_f(const double* x, double* out) {
-    double t[MR_W], q[MR_W], r[MR_W], s[MR_W], p[MR_W], k[MR_W][6], sn[MR_W];
-    int qi[MR_W], odd[MR_W];
-    MR_EACH t[i] = MR_FMA(x[i], MR_LK[1], MR_LK[0]);
-    MR_EACH q[i] = t[i] - MR_LK[0];
-    MR_EACH r[i] = MR_FMA(q[i], -MR_LK[2], x[i]);
-    MR_EACH r[i] = MR_FMA(q[i], -MR_LK[3], r[i]);
-    MR_EACH r[i] = MR_FMA(q[i], -MR_LK[4], r[i]);
-    MR_EACH { qi[i] = mr_lo32(t[i]); odd[i] = qi[i] & 1; }
-    MR_EACH {
-        const double* row = MR_SINCOS[odd[i]];
-        MR_LDG2(row + 0, k[i][0], k[i][1]);
-        MR_LDG2(row + 2, k[i][2], k[i][3]);
-        MR_LDG2(row + 4, k[i][4], k[i][5]);
-    }
-    MR_EACH s[i] = r[i] * r[i];
-    MR_EACH p[i] = odd[i] ? MR_LK[27] : MR_LK[26];
-    MR_EACH p[i] = MR_FMA(p[i], s[i], k[i][0]);
-    MR_EACH p[i] = MR_FMA(p[i], s[i], k[i][1]);
-    MR_EACH p[i] = MR_FMA(p[i], s[i], k[i][2]);
-    MR_EACH p[i] = MR_FMA(p[i], s[i], k[i][3]);
-    MR_EACH p[i] = MR_FMA(p[i], s[i], k[i][4]);
-    MR_EACH p[i] = MR_FMA(p[i], s[i], k[i][5]);
-    MR_EACH p[i] = MR_FMA(p[i], s[i], odd[i] ? 1.0 : 0.0);
-    MR_EACH sn[i] = MR_FMA(p[i], r[i], r[i]);
-    MR_EACH {
-        const double v = odd[i] ? p[i] : sn[i];
-        out[i] = mr_hilo((int)((unsigned int)mr_hi32(v) ^ (((unsigned int)qi[i] & 2u) << 30)), mr_lo32(v));
-    }
-}
-#endif  // MR_SIN_PARITY
-#ifdef MR_EXPLOG_POLY
-__device__ __forceinline__ void mr_exp_fast_w_f(const double* x, double* out) {
-    double t[MR_W], n[MR_W], r[MR_W], p[MR_W];
-    MR_EACH t[i] = MR_FMA(x[i], MR_LK[5], MR_LK[0]);
-    MR_EACH n[i] = t[i] - MR_LK[0];
-    MR_EACH r[i] = MR_FMA(n[i], -MR_LK[6], x[i]);
-    MR_EACH r[i] = MR_FMA(n[i], -MR_LK[7], r[i]);
-    MR_EACH p[i] = MR_LK[8];
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[9]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[10]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[11]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[12]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[13]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[14]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[15]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[16]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[17]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], MR_LK[18]);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], 1.0);
-    MR_EACH p[i] = MR_FMA(p[i], r[i], 1.0);
-    MR_EACH out[i] = mr_hilo((int)((unsigned int)mr_hi32(p[i]) + ((unsigned int)mr_lo32(t[i]) << 20)), mr_lo32(p[i]));
-}
-__device__ __forceinline__ void mr_log_fast_w_f(const double* x, double* out) {
-    double m[MR_W], a[MR_W], b[MR_W], y[MR_W], er[MR_W], u[MR_W], d[MR_W], rem[MR_W], u_lo[MR_W], w[MR_W], Q[MR_W];
-    double t3[MR_W], ed[MR_W], h[MR_W], c[MR_W], lo[MR_W];
-    MR_EACH {
-        const int hx = mr_hi32(x[i]);
-        int e = (hx >> 20) - 1023;
-        int mh = (hx & 0x000fffff) | 0x3ff00000;
-        if (mh >= 0x3ff6a09f) { mh -= 0x00100000; e += 1; }
-        m[i] = mr_hilo(mh, mr_lo32(x[i]));
-        ed[i] = (double)e;
-    }
-    MR_EACH a[i] = m[i] - 1.0;
-    MR_EACH b[i] = m[i] + 1.0;
-    MR_EACH y[i] = mr_rcp_approx(b[i]);
-    MR_EACH er[i] = MR_FMA(-b[i], y[i], 1.0);
-    MR_EACH y[i] = MR_FMA(y[i], er[i], y[i]);
-    MR_EACH er[i] = MR_FMA(-b[i], y[i], 1.0);
-    MR_EACH y[i] = MR_FMA(y[i], er[i], y[i]);
-    MR_EACH { const double qq = a[i] * y[i]; u[i] = qq + qq; }
-    MR_EACH d[i] = a[i] - u[i];
-    MR_EACH rem[i] = MR_FMA(a[i], -u[i], d[i] + d[i]);
-    MR_EACH u_lo[i] = y[i] * rem[i];
-    MR_EACH w[i] = u[i] * u[i];
-    MR_EACH Q[i] = MR_LK[19];
-    MR_EACH Q[i] = MR_FMA(Q[i], w[i], MR_LK[20]);
-    MR_EACH Q[i] = MR_FMA(Q[i], w[i], MR_LK[21]);
-    MR_EACH Q[i] = MR_FMA(Q[i], w[i], MR_LK[22]);
-    MR_EACH Q[i] = MR_FMA(Q[i], w[i], MR_LK[23]);
-    MR_EACH Q[i] = MR_FMA(Q[i], w[i], MR_LK[24]);
-    MR_EACH Q[i] = MR_FMA(Q[i], w[i], MR_LK[25]);
-    MR_EACH t3[i] = MR_FMA(u[i] * w[i], Q[i], u_lo[i]);
-    MR_EACH h[i] = MR_FMA(ed[i], MR_LK[6], u[i]);
-    MR_EACH c[i] = MR_FMA(ed[i], MR_LK[6], -h[i]) + u[i];
-    MR_EACH lo[i] = MR_FMA(ed[i], MR_LK[7], t3[i]) + c[i];
-    MR_EACH out[i] = h[i] + lo[i];
-}
-#else
 // glibc's exp, MR_W evaluations step-major: same operations per lane as mr_exp_fast_g.
 __device__ __forceinline__ void mr_exp_fast_w_f(const double* x, double* out) {
     double kd0[MR_W], kd[MR_W], r[MR_W], tail[MR_W], p23[MR_W], tr[MR_W], r2[MR_W], p45[MR_W], t1[MR_W], scale[MR_W];
@@ -626,7 +353,6 @@ __device__ __forceinline__ void mr_log_fast_w_f(const double* x, double* out) {
     MR_EACH out[i] = MR_FMA(r3[i], a34[i], lo[i]) + hi[i];
     MR_EACH if ((unsigned int)(mr_hi32(x[i]) - 0x3fee0000) < 0x30900u) out[i] = mr_log_fast_g(x[i]);
 }
-#endif  // MR_EXPLOG_POLY
 #ifdef MR_LIBM_GLIBC
 // The exact mode branches inside an evaluation (ranges of sin, the near-1 path of log), so it is not written step-major.
 #define MR_DEFINE_FAST_W(fn) __device__ __forceinline__ void mr_##fn##_fast_w(const double* x, double* out) { MR_EACH out[i] = mr_##fn##_fast_g(x[i]); }

@@ -171,8 +171,7 @@ __device__ __forceinline__ void mr_un(const Files<P>& f, double (&acc)[P], doubl
     case BC_H_OUT + (C) * 4 + 2: { double x[P]; mr_fetch<P, 2>(F, acc, sacc, a, x); F.store(out16 + (C) * slot16, x); } break; \
     case BC_H_OUT + (C) * 4 + 3: { double x[P]; mr_fetch<P, 3>(F, acc, sacc, a, x); F.store(out16 + (C) * slot16, x); } break;
 
-// DISPATCH: 0 = inline-PTX inner loop (jump table), 1 = C++ switch only (A/B, debugging).
-template <int P, int DISPATCH>
+template <int P>
 __global__ void __launch_bounds__(512) maray_interp(const MrTileParams p, const uint64_t* __restrict__ code, unsigned int n_instr,
                                                     const double* __restrict__ consts, unsigned int n_consts, unsigned int n_scal,
                                                     unsigned int n_wide, unsigned int all_wide) {
@@ -238,12 +237,10 @@ __global__ void __launch_bounds__(512) maray_interp(const MrTileParams p, const 
         for (;;) {
             // Inner loop (inline PTX, interp_dispatch.inc): fetch, indexed branch into a body specialised on
             // operation and operand kinds, store, next -- until an instruction it has no body for.
-            if constexpr (DISPATCH == 0) {
-                if constexpr (P == 1) MR_INTERP_LOOP_P1(acc[0], sacc, pc, wbase_s, sbase_s, F.half_stride);
-                else if constexpr (P == 2) MR_INTERP_LOOP_P2(acc[0], acc[1], sacc, pc, wbase_s, sbase_s, F.half_stride);
-                else MR_INTERP_LOOP_P4(acc[0], acc[1], acc[2], acc[3], sacc, pc, wbase_s, sbase_s, F.half_stride);
-            }
-            // One instruction through the C++ switch, which implements EVERY handler (with TREE: all of them).
+            if constexpr (P == 1) MR_INTERP_LOOP_P1(acc[0], sacc, pc, wbase_s, sbase_s, F.half_stride);
+            else if constexpr (P == 2) MR_INTERP_LOOP_P2(acc[0], acc[1], sacc, pc, wbase_s, sbase_s, F.half_stride);
+            else MR_INTERP_LOOP_P4(acc[0], acc[1], acc[2], acc[3], sacc, pc, wbase_s, sbase_s, F.half_stride);
+            // The instruction it stopped at goes through the C++ switch, which implements EVERY handler.
             const uint64_t w = cs[(pc - cs_s) >> 3];
             pc += 8u;
             const unsigned int lo = (unsigned int)w, hi = (unsigned int)(w >> 32);
@@ -370,19 +367,19 @@ size_t interp_smem_bytes(unsigned int block, unsigned int pixels_per_thread, uns
            (size_t)(n_wide + 3u) * pixels_per_thread * block * sizeof(double);   // + 3 channel-output slots
 }
 
-template <int P, int DISPATCH>
+template <int P>
 static cudaError_t launch_interp_as(const MrTileParams& p, const uint64_t* d_code, unsigned int n_instr, const double* d_consts,
                                     unsigned int n_consts, unsigned int n_scal, unsigned int n_wide, bool all_wide,
                                     unsigned int block, unsigned int grid, size_t smem, cudaStream_t stream) {
-    cudaError_t e = cudaFuncSetAttribute(maray_interp<P, DISPATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(maray_interp<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    maray_interp<P, DISPATCH><<<grid, block, smem, stream>>>(p, d_code, n_instr, d_consts, n_consts, n_scal, n_wide, all_wide ? 1u : 0u);
+    maray_interp<P><<<grid, block, smem, stream>>>(p, d_code, n_instr, d_consts, n_consts, n_scal, n_wide, all_wide ? 1u : 0u);
     return cudaGetLastError();
 }
 
 cudaError_t launch_interp(MrTileParams p, const uint64_t* d_code, unsigned int n_instr, const double* d_consts,
                           unsigned int n_consts, unsigned int n_uniform, unsigned int n_wide, bool all_wide, unsigned int block,
-                          unsigned int pixels_per_thread, cudaStream_t stream, int dispatch) {
+                          unsigned int pixels_per_thread, cudaStream_t stream) {
     if (p.rows == 0 || p.x1 <= p.x0) return cudaSuccess;
     const unsigned int n_scal = n_consts + n_uniform;
     const size_t smem = interp_smem_bytes(block, pixels_per_thread, n_wide, n_scal);
@@ -390,9 +387,7 @@ cudaError_t launch_interp(MrTileParams p, const uint64_t* d_code, unsigned int n
     p.nxb = (p.x1 - p.x0 + span - 1) / span;
     if ((uint64_t)p.nxb * p.rows > 0x7fffffffull) return cudaErrorInvalidValue;
     const unsigned int grid = p.nxb * p.rows;
-#define MR_LAUNCH(PP)                                                                                                         \
-    (dispatch == 1 ? launch_interp_as<PP, 1>(p, d_code, n_instr, d_consts, n_consts, n_scal, n_wide, all_wide, block, grid, smem, stream) \
-                   : launch_interp_as<PP, 0>(p, d_code, n_instr, d_consts, n_consts, n_scal, n_wide, all_wide, block, grid, smem, stream))
+#define MR_LAUNCH(PP) launch_interp_as<PP>(p, d_code, n_instr, d_consts, n_consts, n_scal, n_wide, all_wide, block, grid, smem, stream)
     switch (pixels_per_thread) {
     case 1: return MR_LAUNCH(1);
     case 2: return MR_LAUNCH(2);
@@ -433,32 +428,29 @@ cudaError_t launch_fp64_issue_rate(bool fma, double* d_sink, int iters, int bloc
 // ------------------------------------------------------------------------------------------------
 // Completion signal between the processes that render row bands into one frame (api.cu: maray_cuda_band_signal /
 // maray_cuda_band_wait).  A band kernel's stores into the frame of GPU 0 travel over NVLink; the kernel boundary
-// orders them before this one 4-byte store, and the store is a system-scope release, so a reader that has seen the
-// counter reach `value` (system-scope acquire) sees the band.  The wait is bounded: after ~2 s of polling it records
-// a time-out and ends, so a lost peer can never hang the GPU.
-__global__ void band_signal(unsigned int* counter, unsigned int value, int mode) {
+// orders them before this one 4-byte write, and the write is a system-scope release, so a reader that has seen the
+// counter reach `value` (system-scope acquire) sees the band.  Both sides are atomics, performed at the home L2 of the
+// counter (the exporting GPU), like every atomic over NVLink: polled with loads instead (acquire.sys or volatile), the
+// exporting GPU saw a peer's write 1-50 ms late, with the atomic poll in 6-8 us (measured at N = 2,
+// profiles/r02c_band_completion_signal_n2.md).  The wait is bounded: after ~2 s of polling it records a time-out and
+// ends, so a lost peer can never hang the GPU.
+__global__ void band_signal(unsigned int* counter, unsigned int value) {
     __threadfence_system();
-    if (mode & 1) {   // performed at the home L2 of the counter (the exporting GPU), like every atomic over NVLink
-        unsigned int old;
-        asm volatile("atom.exch.release.sys.global.b32 %0, [%1], %2;" : "=r"(old) : "l"(counter), "r"(value) : "memory");
-        (void)old;
-    } else {
-        asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(counter), "r"(value) : "memory");
-    }
+    unsigned int old;
+    asm volatile("atom.exch.release.sys.global.b32 %0, [%1], %2;" : "=r"(old) : "l"(counter), "r"(value) : "memory");
+    (void)old;
     __threadfence_system();
 }
 
 __global__ void band_wait(unsigned int* counters, unsigned int stride, unsigned int n, unsigned int value, unsigned int* timed_out,
-                          long long max_cycles, int mode) {
+                          long long max_cycles) {
     const unsigned int i = threadIdx.x;
     if (i >= n) return;
     unsigned int* c = counters + size_t(i) * stride;
     const long long t0 = clock64();
     for (;;) {
         unsigned int seen;
-        if ((mode >> 1) == 1) asm volatile("atom.add.acquire.sys.global.u32 %0, [%1], 0;" : "=r"(seen) : "l"(c) : "memory");
-        else if ((mode >> 1) == 2) asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(seen) : "l"(c) : "memory");
-        else asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(seen) : "l"(c) : "memory");
+        asm volatile("atom.add.acquire.sys.global.u32 %0, [%1], 0;" : "=r"(seen) : "l"(c) : "memory");
         if (int(seen - value) >= 0) break;               // counters only grow; wrapping compare
         if (clock64() - t0 > max_cycles) { *timed_out = 1u; break; }
         __nanosleep(64);
@@ -466,14 +458,14 @@ __global__ void band_wait(unsigned int* counters, unsigned int stride, unsigned 
     __threadfence_system();
 }
 
-cudaError_t launch_band_signal(unsigned int* counter, unsigned int value, cudaStream_t stream, int mode) {
-    band_signal<<<1, 1, 0, stream>>>(counter, value, mode);
+cudaError_t launch_band_signal(unsigned int* counter, unsigned int value, cudaStream_t stream) {
+    band_signal<<<1, 1, 0, stream>>>(counter, value);
     return cudaGetLastError();
 }
 
 cudaError_t launch_band_wait(unsigned int* counters, unsigned int stride, unsigned int n, unsigned int value, unsigned int* timed_out,
-                             long long max_cycles, cudaStream_t stream, int mode) {
-    band_wait<<<1, ((n + 31) / 32) * 32, 0, stream>>>(counters, stride, n, value, timed_out, max_cycles, mode);
+                             long long max_cycles, cudaStream_t stream) {
+    band_wait<<<1, ((n + 31) / 32) * 32, 0, stream>>>(counters, stride, n, value, timed_out, max_cycles);
     return cudaGetLastError();
 }
 

@@ -30,15 +30,13 @@ size_t interp_smem_bytes(unsigned int block, unsigned int pixels_per_thread, uns
 // d_code / n_instr: the stream made by bytecode_for_launch (a whole number of kBcChunk-word chunks).
 cudaError_t launch_interp(MrTileParams p, const uint64_t* d_code, unsigned int n_instr, const double* d_consts,
                           unsigned int n_consts, unsigned int n_uniform, unsigned int n_wide, bool all_wide, unsigned int block,
-                          unsigned int pixels_per_thread, cudaStream_t stream, int dispatch = 0);
-// dispatch: 0 = the inline-PTX inner loop with its jump table (default); 1 = every handler through the C++
-// switch, which nvcc lowers to a compare-and-branch tree (A/B, debugging: MARAY_INTERP_DISPATCH=tree).
+                          unsigned int pixels_per_thread, cudaStream_t stream);
 
 cudaError_t launch_fp64_issue_rate(bool fma, double* d_sink, int iters, int blocks, cudaStream_t stream);
 
 // Completion counters of a frame shared by band processes (kernels.cu, "band_signal/wait").
-cudaError_t launch_band_signal(unsigned int* counter, unsigned int value, cudaStream_t stream, int mode);
+cudaError_t launch_band_signal(unsigned int* counter, unsigned int value, cudaStream_t stream);
 cudaError_t launch_band_wait(unsigned int* counters, unsigned int stride, unsigned int n, unsigned int value, unsigned int* timed_out,
-                             long long max_cycles, cudaStream_t stream, int mode);
+                             long long max_cycles, cudaStream_t stream);
 
 }  // namespace maray

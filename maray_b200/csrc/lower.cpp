@@ -518,27 +518,6 @@ void lower_job_body(LowerJob* j) {
         P->order.swap(out);
         P->batch.swap(out_batch);
     }
-    // Frontier of the x-only / y-only sub-programs.
-    {
-        std::vector<uint8_t> wanted(P->nodes.size(), 0);
-        for (uint32_t id : P->order) {
-            const Node& n = P->nodes[id];
-            auto use = [&](uint32_t v) {
-                const Node& o = P->nodes[v];
-                if ((o.dep == DEP_X || o.dep == DEP_Y) && o.op != OP_X && o.op != OP_Y && n.dep != o.dep) wanted[v] = 1;
-            };
-            if (op_is_unary(n.op) || op_is_binary(n.op)) use(n.a);
-            if (op_is_binary(n.op)) use(n.b);
-        }
-        for (int c = 0; c < 3; c++) {
-            const Node& o = P->nodes[P->root[c]];
-            if ((o.dep == DEP_X || o.dep == DEP_Y) && o.op != OP_X && o.op != OP_Y) wanted[P->root[c]] = 1;
-        }
-        P->col_values.clear();
-        P->row_values.clear();
-        for (uint32_t id : P->order)
-            if (wanted[id]) (P->nodes[id].dep == DEP_X ? P->col_values : P->row_values).push_back(id);
-    }
     P->stats = st;
     j->ok = true;
 }

@@ -63,10 +63,6 @@ struct Program {
     // are sin/exp/ln values of one kind that are mutually independent and whose operands all precede
     // the first of them -- they may be evaluated together (instruction-level parallelism, one call).
     std::vector<uint32_t> batch;
-    // Hoisting (the counterpart of the reference's row cache, reference src/cache.rs:18-20 + dep_x):
-    // values that depend on x only / y only and are read by a value that depends on both (or are a
-    // channel) -- they can be computed once per column / row instead of once per pixel.
-    std::vector<uint32_t> col_values, row_values;
     uint32_t n_textures = 0;        // textures the program was lowered against
     ProgramStats stats;
 };

@@ -74,20 +74,11 @@ using std::sin; using std::exp; using std::log;
 
 HOST_DRIVER = r"""
 extern "C" void host_run(unsigned char* out, double* f64_out, unsigned long long plane, const MrTexture* tex,
-                         unsigned int p0, unsigned int n, unsigned int W, double* colv, double* rowv) {
+                         unsigned int p0, unsigned int n, unsigned int W) {
     MrParams p;
     p.out = out; p.f64_out = f64_out; p.f64_plane = plane; p.tex = tex; p.p0 = p0; p.n = n; p.W = W;
     p.out_aligned = 0;
-    const unsigned int y_first = p0 / W, rows = (p0 + n - 1) / W - y_first + 1;
-    p.colv = colv; p.rowv = rowv; p.row_base = y_first; p.rows = rows;
     blockDim.x = 256; blockDim.y = blockDim.z = 1;
-#ifdef MR_HOST_HAS_PROLOGUE
-    // the two prologue kernels, one "thread" per column / row
-    blockIdx.x = 0; blockDim.x = 0x7fffffff;
-    for (unsigned int t = 0; t < W; t++) { threadIdx.x = t; maray_pre_x(colv, W, 0u, tex); }
-    for (unsigned int t = 0; t < rows; t++) { threadIdx.x = t; maray_pre_y(rowv, rows, y_first, tex); }
-    blockDim.x = 256;
-#endif
     unsigned int blocks = (n + 255) / 256;
     for (unsigned int b = 0; b < blocks; b++) {
         blockIdx.x = b;
@@ -107,7 +98,7 @@ extern "C" void host_run(unsigned char* out, double* f64_out, unsigned long long
                          unsigned int p0, unsigned int n, unsigned int W, double* F, unsigned long long FS) {
     MrParams p;
     p.out = out; p.f64_out = f64_out; p.f64_plane = plane; p.tex = tex; p.p0 = p0; p.n = n; p.W = W;
-    p.out_aligned = 0; p.colv = nullptr; p.rowv = nullptr; p.row_base = 0; p.rows = 0;
+    p.out_aligned = 0;
     blockDim.x = 256; blockDim.y = blockDim.z = 1;
     unsigned int blocks = (n + 255) / 256;
     for (unsigned int b = 0; b < blocks; b++) {
@@ -138,8 +129,6 @@ def host_jit_run(source: str, w: int, p0: int, n: int, textures=(), perturb_libm
             if perturb_libm:
                 f.write("#define MR_HOST_PERTURB_LIBM 1\n")
             f.write(HOST_SHIM)
-            if "maray_pre_x" in source:
-                f.write("#define MR_HOST_HAS_PROLOGUE 1\n")
             f.write(source.replace('extern "C" __global__', "static"))
             f.write(HOST_DRIVER)
         so = os.path.join(d, "k.so")
@@ -147,7 +136,7 @@ def host_jit_run(source: str, w: int, p0: int, n: int, textures=(), perturb_libm
                                "-w", "-o", so, src])
         lib = ctypes.CDLL(so)
         lib.host_run.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_ulonglong, ctypes.c_void_p,
-                                 ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p]
+                                 ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32]
         _CACHE[key] = lib
     rgb = np.zeros((n, 3), dtype=np.uint8)
     planes = np.zeros((3, n), dtype=np.float64)
@@ -156,11 +145,7 @@ def host_jit_run(source: str, w: int, p0: int, n: int, textures=(), perturb_libm
     for i, a in enumerate(arrs):
         tab[i].data = a.ctypes.data
         tab[i].w, tab[i].h = a.shape[1], a.shape[0]
-    # hoisting tables, generously sized (the host check does not know the table widths)
-    rows = (p0 + n - 1) // w - p0 // w + 1
-    colv = np.zeros(4096 * w, dtype=np.float64)
-    rowv = np.zeros(4096 * rows, dtype=np.float64)
-    lib.host_run(rgb.ctypes.data, planes.ctypes.data, n, ctypes.addressof(tab), p0, n, w, colv.ctypes.data, rowv.ctypes.data)
+    lib.host_run(rgb.ctypes.data, planes.ctypes.data, n, ctypes.addressof(tab), p0, n, w)
     return rgb, planes
 
 

@@ -159,9 +159,6 @@ def test_launch_shape_follows_the_program(monkeypatch, chess_bytes):
     assert block == 640 and "__launch_bounds__(640, 1) maray_jit" in src
     block, src = shape(chess_bytes, MARAY_JIT_BLOCK="256")
     assert block == 256 and "__launch_bounds__(256, 2) maray_jit" in src
-    block, src = shape(scenes.chess_4k(), MARAY_JIT_PERSISTENT="1")
-    assert block == 640 and "for (unsigned int blk = blockIdx.x; blk * blockDim.x < p.n; blk += gridDim.x)" in src
-    assert "mr_store_block_at(" in src
     block, src = shape(scenes.sdf(64, 48, 6, seed=4))
     assert block == 256 and "__launch_bounds__(256, 2) maray_jit" in src
     block, src = shape(scenes.deep(64, 64, n_values=9000, seed=3))          # batched helpers: scratch rows sized for 256 threads

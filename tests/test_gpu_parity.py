@@ -221,7 +221,7 @@ def _heavy_scene_with_out_of_range_arguments(w, h):
     return E.to_bytes([w, h], out)
 
 
-@pytest.mark.parametrize("form", ["scratch", "registers", "chain", "functions"])
+@pytest.mark.parametrize("form", ["scratch", "chain", "functions"])
 def test_batched_transcendentals_and_their_repair_path(monkeypatch, form):
     """The out-of-line sin/exp/ln forms of the NVRTC back end on a program above the batching threshold,
     with arguments that must take the libdevice repair path, and both ways of cutting a large program (a chain
@@ -231,8 +231,6 @@ def test_batched_transcendentals_and_their_repair_path(monkeypatch, form):
     w, h = 96, 64
     scene = _heavy_scene_with_out_of_range_arguments(w, h)
     want_rgb, want = OracleScene(scene).render_window(0, w, 0, h, want_f64=True)
-    if form == "registers":
-        monkeypatch.setenv("MARAY_JIT_SCRATCH", "0")
     monkeypatch.setenv("MARAY_JIT_SEGMENT_VALUES", "3000" if form in ("chain", "functions") else "100000")
     if form == "functions":
         monkeypatch.setenv("MARAY_JIT_CHAIN", "0")
@@ -247,7 +245,7 @@ def test_batched_transcendentals_and_their_repair_path(monkeypatch, form):
     if form == "functions":
         assert st["jit_units"] == 1 and st["jit_segments"] >= 3
     assert np.array_equal(frame, rgb)
-    for k in ("MARAY_JIT_SCRATCH", "MARAY_JIT_CHAIN", "MARAY_JIT_SEGMENT_VALUES", "MARAY_JIT_FRAME_MB"):
+    for k in ("MARAY_JIT_CHAIN", "MARAY_JIT_SEGMENT_VALUES", "MARAY_JIT_FRAME_MB"):
         monkeypatch.delenv(k, raising=False)
     # yardstick: the interpreter kernel, whose handlers inline the scalar routines
     with _renderer(scene, "interp") as r:
@@ -475,34 +473,6 @@ def test_pipelined_host_render(monkeypatch):
             assert np.array_equal(got[y], want_rows[i])
 
 
-def test_hoisted_prologue_form(monkeypatch):
-    """MARAY_JIT_HOIST=1: x-only / y-only values from the prologue kernels' tables.  Same bytes as the
-    default form on whole frames; bands issued on two different streams share the per-GPU tables."""
-    import torch
-    tex = scenes.synthetic_textures(2, 16)
-    x, y = E.x(), E.y()
-    t57 = E.app(E.channel(0, 1), E.nat(5), E.nat(7))
-    const_tex = E.to_bytes([64, 48], [E.add(t57, x), E.mul(E.sin(E.add(E.app(E.channel(1, 2), E.nat(3), E.nat(2)), x)), y),
-                                      E.add(E.mul(t57, y), E.app(E.channel(1, 0), E.nat(15), E.nat(0)))])
-    for scene, w, h, textures in [(scenes.chess_1k(), 1024, 1024, ()), (scenes.sdf(640, 360, 16, seed=2), 640, 360, ()),
-                                  (const_tex, 64, 48, tex)]:
-        with _renderer(scene, "nvrtc", textures) as r:
-            base = r.render(w, h)
-        monkeypatch.setenv("MARAY_JIT_HOIST", "1")
-        with _renderer(scene, "nvrtc", textures) as r:
-            got = r.render(w, h)
-            frame = torch.zeros(h * w * 3, dtype=torch.uint8, device="cuda")
-            s1, s2 = torch.cuda.Stream(), torch.cuda.Stream()
-            cuts = [0, h // 3, h // 2, h]
-            for i in range(3):
-                st = (s1, s2)[i % 2]
-                r.render_band(w, h, cuts[i], cuts[i + 1], frame.data_ptr() + cuts[i] * w * 3, st.cuda_stream)
-            torch.cuda.synchronize()
-        monkeypatch.delenv("MARAY_JIT_HOIST")
-        assert np.array_equal(got, base)
-        assert np.array_equal(frame.cpu().numpy().reshape(h, w, 3), base)
-
-
 @pytest.mark.parametrize("backend", BACKENDS)
 def test_texture_fetch_at_constant_coordinates_on_device(backend):
     """App(channel, const, const): both coordinates literal (the advisor's round-1 finding for the bytecode)."""
@@ -632,17 +602,16 @@ def test_chain_segmentations_render_the_same_frame(monkeypatch):
 
 
 def test_code_generation_knobs_render_the_same_frame(monkeypatch):
-    """The forms the code generator can take for a transcendental-heavy program (helper width, scratch or register
-    arguments, literal or banked constants, libm flavour for exp/log, segment functions instead of a chain) must all
-    render the bytes of the default form: the class of fault the NVRTC 12.8 miscompile belonged to (DESIGN.md 10.7)."""
+    """The forms the code generator can take for a transcendental-heavy program (literal or banked constants, segment
+    functions instead of a chain, other chain cuts, no boolean logic) must all render the bytes of the default form: the
+    class of fault the NVRTC 12.8 miscompile belonged to (DESIGN.md 10.7)."""
     w, h = 384, 256
     scene = scenes.deep(w, h, n_values=12000, seed=2)
     with _renderer(scene, "nvrtc") as r:
         want = r.render(w, h)
-    variants = [{"MARAY_JIT_BATCH_WIDTH": "4"}, {"MARAY_JIT_SCRATCH": "0"}, {"MARAY_JIT_CONST_BANK": "0"},
+    variants = [{"MARAY_JIT_CONST_BANK": "0"},
                 {"MARAY_JIT_CHAIN": "0", "MARAY_JIT_SEGMENT_VALUES": "4096"}, {"MARAY_JIT_CHAIN_SEGMENT_VALUES": "2000", "MARAY_JIT_SEGMENT_VALUES": "4096"},
-                {"MARAY_LIBM_EXPLOG": "poly"}, {"MARAY_JIT_BOOLEAN": "0"}, {"MARAY_JIT_LINEINFO": "0"},
-                {"MARAY_JIT_SCRATCH_TABLES": "0"}, {"MARAY_JIT_CONST_ORDER": "1"}, {"MARAY_JIT_CARVEOUT": "-2"}]
+                {"MARAY_JIT_BOOLEAN": "0"}, {"MARAY_JIT_LINEINFO": "0"}, {"MARAY_JIT_CARVEOUT": "-2"}]
     for env in variants:
         for k, v in env.items():
             monkeypatch.setenv(k, v)
@@ -650,21 +619,17 @@ def test_code_generation_knobs_render_the_same_frame(monkeypatch):
             got = r.render(w, h)
         for k in env:
             monkeypatch.delenv(k)
-        if "MARAY_LIBM_EXPLOG" in env:       # other (1-ULP) exp/log: the bytes may move by one grey level at most
-            assert np.abs(got.astype(int) - want.astype(int)).max() <= 1, env
-        else:
-            assert np.array_equal(got, want), env
+        assert np.array_equal(got, want), env
 
 
-LAUNCH_SHAPE_VARIANTS = [{"MARAY_JIT_BLOCK": "256"}, {"MARAY_JIT_PERSISTENT": "1"}, {"MARAY_JIT_CONST_ORDER": "1"},
-                         {"MARAY_JIT_BLOCK": "640", "MARAY_JIT_MIN_BLOCKS": "1"},
-                         {"MARAY_JIT_BLOCK": "128", "MARAY_JIT_MIN_BLOCKS": "5", "MARAY_JIT_PERSISTENT": "1"}]
+LAUNCH_SHAPE_VARIANTS = [{"MARAY_JIT_BLOCK": "256"}, {"MARAY_JIT_BLOCK": "640", "MARAY_JIT_MIN_BLOCKS": "1"},
+                         {"MARAY_JIT_BLOCK": "128", "MARAY_JIT_MIN_BLOCKS": "5"}]
 
 
 def test_launch_shapes_render_the_same_frame(monkeypatch):
     """A large straight-line program runs as one 640-thread block per SM by default (DESIGN.md 3.1 "launch shape").
     The frame must not depend on that choice: ragged sizes (the last block is partial, rows straddle blocks), the old
-    256 x 2 shape, hand-set shapes, the persistent form and the use-ordered constant table render the same bytes, and
+    256 x 2 shape and hand-set shapes render the same bytes, and
     the default form matches the oracle."""
     scene = scenes.chess_1k()
     w, h = 1001, 77                       # 77 077 pixels: not a multiple of 640, 256, 1024 or 128

@@ -52,18 +52,15 @@ def test_textured_scene_bit_exact():
     _check_scene(scenes.textured(256, 128), 256, [0, 64, 127], tex)
 
 
-def test_texture_fetch_at_constant_coordinates(monkeypatch):
+def test_texture_fetch_at_constant_coordinates():
     """App(channel, const, const) -- both coordinates literal.  The bytecode must not route one of them
-    through a slot (the kernel fetches operands one instruction ahead of the store); with hoisting on, the
-    prologue kernels must define such a value when an x-only / y-only value reads it."""
+    through a slot (the kernel fetches operands one instruction ahead of the store)."""
     tex = scenes.synthetic_textures(2, 16)
     x, y = E.x(), E.y()
     t57 = E.app(E.channel(0, 1), E.nat(5), E.nat(7))
     color = [E.add(t57, x), E.mul(E.sin(E.add(E.app(E.channel(1, 2), E.nat(3), E.nat(2)), x)), y),
              E.add(E.mul(t57, y), E.app(E.channel(1, 0), E.nat(15), E.nat(0)))]
     scene = E.to_bytes([24, 6], color)
-    _check_scene(scene, 24, [0, 5], tex)
-    monkeypatch.setenv("MARAY_JIT_HOIST", "1")
     _check_scene(scene, 24, [0, 5], tex)
 
 
@@ -258,31 +255,11 @@ def test_sign_only_rewrites_keep_every_value(monkeypatch):
     _check_scene(scene, 32, [0, 1, 3])
 
 
-def test_hoisting_option_is_value_preserving(monkeypatch, chess_bytes):
-    """MARAY_JIT_HOIST=1: x-only / y-only frontier values come from the prologue kernels' tables; every
-    channel value must stay bit-identical (same operations on the same operands, evaluated elsewhere)."""
-    monkeypatch.setenv("MARAY_JIT_HOIST", "1")
-    for scene, w, rows in ((scenes.sdf(320, 200, 16, seed=2), 320, [0, 199]), (chess_bytes, 1024, [512])):
-        with CudaRenderer(gpus=0) as r:
-            r.load(scene)
-            r.compile("nvrtc")
-            src = r.source()
-        assert "maray_pre_x" in src and "maray_pre_y" in src and "__ldg(CV" in src and "__ldg(RV" in src
-        for y in rows:
-            want_rgb, want = _oracle_window(scene, [], 0, w, y, y + 1)
-            rgb, planes = host_jit_run(src, w, y * w, w)
-            assert bits_equal(planes, want.reshape(3, w)).all()
-            assert np.array_equal(rgb, want_rgb.reshape(w, 3))
-
-
-@pytest.mark.parametrize("form", ["scratch", "registers", "chain", "functions"])
+@pytest.mark.parametrize("form", ["scratch", "chain", "functions"])
 def test_transcendental_batching_keeps_values(monkeypatch, form):
-    """Programs with >= 2048 sin/exp/ln values get their schedule batched and call out-of-line helpers:
-    through the per-thread shared-memory scratch (default) or through register arguments (x4/x2).  Above the
-    segment size a program is cut: into a CHAIN of kernels, one translation unit each, values crossing a cut
+    """Programs with >= 2048 sin/exp/ln values get their schedule batched and call out-of-line helpers
+    through the per-thread shared-memory scratch.  Above the segment size a program is cut: into a CHAIN of kernels, one translation unit each, values crossing a cut
     in a global frame (default), or into segment functions inside one unit (MARAY_JIT_CHAIN=0)."""
-    if form == "registers":
-        monkeypatch.setenv("MARAY_JIT_SCRATCH", "0")
     monkeypatch.setenv("MARAY_JIT_SEGMENT_VALUES", "3000" if form in ("chain", "functions") else "100000")
     if form in ("chain", "functions"):
         monkeypatch.setenv("MARAY_JIT_CACHE", "off")          # the compile statistics below are those of a real compile
@@ -298,7 +275,7 @@ def test_transcendental_batching_keeps_values(monkeypatch, form):
         code, consts = r.bytecode()
     assert st["n_sin"] + st["n_exp"] + st["n_ln"] >= 2048
     body = src[src.index("mr_seg0") if "mr_seg0" in src else src.index('extern "C" __global__'):]
-    assert ("_x4(" in body) if form == "registers" else ("_batch" in body and "MR_R(" in body)
+    assert "_batch" in body and "MR_R(" in body
     want_rgb, want = _oracle_window(scene, [], 0, 48, 7, 8)
     if form == "chain":
         assert st["jit_segments"] >= 3 and st["jit_units"] == st["jit_segments"] == len(modules) and st["jit_compile_threads"] >= 1

@@ -143,6 +143,21 @@ int maray_cuda_compile(maray_cuda_t* h, int backend, maray_cuda_stats* stats);
 /* Progress settings for maray_cuda_render (default: MARAY_REPORT_NONE). */
 int maray_cuda_set_report(maray_cuda_t* h, int kind, uint32_t every, maray_report_fn fn, void* user);
 
+/* Supersampled anti-aliasing: s x s samples per pixel (1 <= s <= 16, else MARAY_E_INVALID), box-filtered to RGB8.
+ * Every handle starts at s = 1, which is exactly the reference's frame (one sample at the integer coordinate).
+ *   sample offsets   o_k = (double)(2k + 1 - s) * (1.0 / (2.0 * s)), k in [0, s): the centres of an s x s grid over the
+ *                    pixel footprint [xi - 1/2, xi + 1/2), which is centred on the reference's sample point;
+ *   sample (i, j)    of pixel (xi, yi) is the scene evaluated at X = (double)xi + o_i, Y = (double)yi + o_j (one IEEE
+ *                    addition each), each channel converted with the reference's saturating `as u8`;
+ *   pixel            per channel (sum over the s*s u8 samples + s*s/2) / (s*s), integer division: the box filter of the
+ *                    reference's own frame rendered at s x the resolution.
+ * Sample (i, j) is therefore pixel (xi, yi) of the reference's frame of the scene with x -> x + o_i, y -> y + o_j
+ * substituted everywhere.  The frame is rendered as s*s passes of the compiled kernels, so it costs about s*s frames;
+ * each GPU of the handle keeps a 6-byte-per-pixel accumulator, allocated at the first supersampled render.  Takes
+ * effect at the next render (nothing is recompiled), on every render call; maray_cuda_render_window_f64 returns
+ * MARAY_E_INVALID while s > 1.  Valid on a host-only handle. */
+int maray_cuda_set_samples(maray_cuda_t* h, uint32_t s);
+
 /* `gen_to_image(method, rt, color, &mut img, report)` (reference src/lib.rs:1177-1195):
  * renders a w x h image into the caller's HOST buffer `rgb` (w*h*3 bytes, the raw RgbImage layout,
  * so Rust passes img.as_mut_ptr(); a pageable Vec<u8> is the expected case).  One GPU: the frame is rendered

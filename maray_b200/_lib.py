@@ -53,6 +53,7 @@ SYMBOLS = [
     ("maray_cuda_load_maray", ctypes.c_int, [_P, ctypes.c_char_p, ctypes.c_size_t]),
     ("maray_cuda_scene_size", ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_uint32), ctypes.POINTER(ctypes.c_uint32)]),
     ("maray_cuda_set_libm", ctypes.c_int, [_P, ctypes.c_int]),
+    ("maray_cuda_set_samples", ctypes.c_int, [_P, ctypes.c_uint32]),
     ("maray_cuda_compile", ctypes.c_int, [_P, ctypes.c_int, ctypes.POINTER(Stats)]),
     ("maray_cuda_set_report", ctypes.c_int, [_P, ctypes.c_int, ctypes.c_uint32, REPORT_FN, _P]),
     ("maray_cuda_render", ctypes.c_int, [_P, ctypes.c_uint32, ctypes.c_uint32, _P, ctypes.POINTER(Stats)]),

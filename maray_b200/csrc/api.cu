@@ -57,6 +57,8 @@ struct Gpu {
     // band / frame buffer
     uint8_t* d_out = nullptr; size_t out_cap = 0;
     double* d_f64 = nullptr; size_t f64_cap = 0;
+    // supersampling: uint16 x 3 sums per pixel, indexed by the pixel's index in the frame (maray_cuda_set_samples)
+    uint16_t* d_acc = nullptr; size_t acc_cap = 0;
     // textures
     std::vector<uint8_t*> d_tex;
     MrTexture* d_textab = nullptr;
@@ -117,6 +119,7 @@ struct maray_cuda {
     std::vector<uint64_t> bc_device;                   // bc.code with operand fields scaled for the launch shape
     unsigned interp_block = 128, interp_ppt = 2;       // launch shape: threads per block, pixels per thread
     int libm = MARAY_LIBM_FAST;                        // maray_cuda_set_libm / MARAY_LIBM
+    uint32_t samples = 1;                              // maray_cuda_set_samples: s x s samples per pixel
     unsigned jit_block = 256;
     unsigned jit_dyn_smem = 0;                         // dynamic shared memory of the generated kernel
     unsigned jit_maxreg = 0;
@@ -651,8 +654,10 @@ int adopt_finished_job(maray_cuda* h) {
     return jit_install(h, std::move(job->build));
 }
 
-int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint8_t* d_out, double* d_f64,
-                size_t f64_plane, cudaStream_t stream) {
+// One pass of the kernels over pixels p0 .. p0+n-1.  sp: the pass's sampling state (zero: one sample per pixel), its
+// accumulator, if any, already offset to pixel p0.
+int launch_pass(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint8_t* d_out, double* d_f64,
+                size_t f64_plane, cudaStream_t stream, const MrSampling& sp) {
     MrParams p{};
     p.out = d_out; p.f64_out = d_f64; p.f64_plane = f64_plane; p.tex = g.d_textab;
     p.p0 = p0; p.n = n; p.W = w;
@@ -660,7 +665,8 @@ int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
     if (n == 0) return MARAY_OK;
     if (h->use_jit) {
         if (!h->jit_chain) {
-            void* args[] = {&p};
+            MrSampling a = sp;
+            void* args[] = {&p, &a};
             const unsigned grid = (n + h->jit_block - 1) / h->jit_block;
             CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(g.jit_kernels[0]), dim3(grid), dim3(h->jit_block), args, h->jit_dyn_smem, stream));
         } else {
@@ -691,7 +697,9 @@ int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
                 q.out = d_out + 3 * done;
                 q.out_aligned = (reinterpret_cast<uintptr_t>(q.out) % 16 == 0) ? 1u : 0u;
                 if (d_f64) q.f64_out = d_f64 + done;
-                void* args[] = {&q, &g.d_frame, &fs};
+                MrSampling a = sp;
+                if (a.acc) a.acc += 3 * done;
+                void* args[] = {&q, &g.d_frame, &fs, &a};
                 unsigned grid = (q.n + h->jit_block - 1) / h->jit_block;
                 for (cudaKernel_t k : g.jit_kernels)
                     CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(k), dim3(grid), dim3(h->jit_block), args, h->jit_dyn_smem, stream));
@@ -716,12 +724,52 @@ int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
             t.x0 = x; t.x1 = x + cols; t.y0 = y; t.rows = rows; t.nxb = 0;
             t.out_aligned = (reinterpret_cast<uintptr_t>(t.out) % 16 == 0) ? 1u : 0u;
             t.libm_exact = h->libm == MARAY_LIBM_GLIBC ? 1u : 0u;
+            t.ox = sp.ox; t.oy = sp.oy;
+            t.acc = sp.acc ? sp.acc + 3 * done : nullptr;
+            t.pass = sp.pass; t.count = sp.count;
             CU_TRY(h, launch_interp(t, g.d_code, unsigned(h->bc_device.size()), g.d_consts, unsigned(h->bc.consts.size()),
                                     h->bc.n_uniform, h->bc.n_wide, !h->bc.row_uniform, h->interp_block, h->interp_ppt, stream));
             const uint32_t count = cols * rows;
             done += count; pix += count; left -= count;
         }
     }
+    return MARAY_OK;
+}
+
+// Offset of sample k of s along one axis: the centres of an s x s grid over the pixel footprint [xi - 1/2, xi + 1/2).
+double sample_offset(uint32_t k, uint32_t s) { return double(int(2 * k + 1) - int(s)) * (1.0 / (2.0 * double(s))); }
+
+int ensure_acc(maray_cuda* h, Gpu& g, size_t pixels) {
+    if (g.acc_cap >= pixels) return MARAY_OK;
+    CU_TRY(h, cudaSetDevice(g.device));
+    if (g.d_acc) cudaFree(g.d_acc);   // synchronises: no pass that still uses the old buffer is left running
+    g.d_acc = nullptr; g.acc_cap = 0;
+    CU_TRY(h, cudaMalloc(&g.d_acc, pixels * 3 * sizeof(uint16_t)));
+    g.acc_cap = pixels;
+    return MARAY_OK;
+}
+
+// Renders pixels p0 .. p0+n-1 of a w-wide frame into d_out: every render path comes through here.  With s x s samples
+// per pixel (maray_cuda_set_samples) that is s*s passes in order on `stream`, each at one sub-pixel offset; the last
+// resolves the accumulator into RGB8.  The accumulator is indexed by the pixel's index in the frame, so launches on
+// disjoint pixel ranges (row chunks on several streams, bands) never share a word.
+int launch_band(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint8_t* d_out, double* d_f64,
+                size_t f64_plane, cudaStream_t stream) {
+    const uint32_t s = h->samples;
+    if (s <= 1 || n == 0) return launch_pass(h, g, w, p0, n, d_out, d_f64, f64_plane, stream, MrSampling{});
+    int rc = ensure_acc(h, g, size_t(p0) + n);
+    if (rc) return rc;
+    MrSampling sp{};
+    sp.acc = g.d_acc + 3 * size_t(p0);
+    sp.count = s * s;
+    for (uint32_t jy = 0; jy < s; jy++)
+        for (uint32_t ix = 0; ix < s; ix++) {
+            sp.ox = sample_offset(ix, s);
+            sp.oy = sample_offset(jy, s);
+            sp.pass = jy * s + ix;
+            rc = launch_pass(h, g, w, p0, n, d_out, d_f64, f64_plane, stream, sp);
+            if (rc) return rc;
+        }
     return MARAY_OK;
 }
 
@@ -891,6 +939,9 @@ int render_frame(maray_cuda* h, uint32_t w, uint32_t hgt, uint8_t* host_rgb) {
     Gpu& g0 = h->gpus[0];
     rc = ensure_out(h, g0, size_t(w) * hgt * 3);
     if (rc) return rc;
+    for (Gpu& g : h->gpus) {   // the accumulators before any pass is in flight (a larger one replaces the old)
+        if (h->samples > 1 && (rc = ensure_acc(h, g, size_t(w) * hgt)) != MARAY_OK) return rc;
+    }
     for (double& k : h->stats.kernel_ms) k = 0.0;
     h->stats.gather_ms = 0.0; h->stats.d2h_ms = 0.0;
     rc = adopt_finished_job(h);
@@ -1028,6 +1079,7 @@ void maray_cuda_destroy(maray_cuda_t* h) {
         cudaSetDevice(g.device);
         if (g.d_out) cudaFree(g.d_out);
         if (g.d_f64) cudaFree(g.d_f64);
+        if (g.d_acc) cudaFree(g.d_acc);
         if (g.d_sink) cudaFree(g.d_sink);
         if (g.frame_done) cudaEventDestroy(g.frame_done);
         if (g.ev0) cudaEventDestroy(g.ev0);
@@ -1151,6 +1203,13 @@ int maray_cuda_set_libm(maray_cuda_t* h, int libm) {
     return MARAY_OK;
 }
 
+int maray_cuda_set_samples(maray_cuda_t* h, uint32_t s) {
+    if (!h) return MARAY_E_INVALID;
+    if (s < 1 || s > 16) return fail(h, MARAY_E_INVALID, "maray_cuda_set_samples: samples per axis must be 1..16, got " + std::to_string(s));
+    h->samples = s;
+    return MARAY_OK;
+}
+
 int maray_cuda_set_report(maray_cuda_t* h, int kind, uint32_t every, maray_report_fn fn, void* user) {
     if (!h || kind < MARAY_REPORT_NONE || kind > MARAY_REPORT_DURATION_MS) return fail(h, MARAY_E_INVALID, "bad report kind");
     h->report_kind = kind; h->report_every = every; h->report_fn = fn; h->report_user = user;
@@ -1259,6 +1318,8 @@ int maray_cuda_render_window_f64(maray_cuda_t* h, uint32_t w, uint32_t hgt, uint
     int rc = check_renderable(h, w, hgt);
     if (rc) return rc;
     if (x0 > x1 || x1 > w || y0 > y1 || y1 > hgt) return fail(h, MARAY_E_INVALID, "window outside the image");
+    if (h->samples > 1)   // the f64 planes are the values of single samples
+        return fail(h, MARAY_E_INVALID, "maray_cuda_render_window_f64 renders one sample per pixel; call maray_cuda_set_samples(h, 1) first");
     const uint32_t ww = x1 - x0, hh = y1 - y0;
     const size_t npx = size_t(ww) * hh;
     if (npx == 0) return MARAY_OK;

@@ -1,6 +1,8 @@
 // maray_cuda -- command-line front end of the CUDA render path, shaped like the reference's CLI
 // (reference examples/maray.rs:9-47):
-//     maray_cuda -i scene.maray -o out.png [-t tex0.png tex1.png ...] [-c N] [-g GPUS] [-b nvrtc|interp]
+//     maray_cuda -i scene.maray -o out.png [-t tex0.png tex1.png ...] [-c N] [-g GPUS] [-b nvrtc|interp] [-s N]
+// -s/--samples N renders N x N samples per pixel, box-filtered (maray_cuda_set_samples; 1, the default, is the
+// reference's frame).
 // -c/--cpus is accepted for command-line compatibility and ignored, exactly as the reference ignores
 // it at HEAD (reference examples/maray.rs:55: parsed into `_cpus`).  Progress is reported every
 // 500 ms the way `gen` does (reference src/lib.rs:1203-1208, examples/maray.rs:77-79): percentage on
@@ -29,7 +31,7 @@ int usage() {
     std::fprintf(stderr,
                  "Maray (CUDA render path)\n"
                  "usage: maray_cuda -i <file.maray> -o <file.png> [-t <texture.png>...] [-c <cpus, ignored>]\n"
-                 "                  [-g <gpus>] [-b nvrtc|interp]\n");
+                 "                  [-g <gpus>] [-b nvrtc|interp] [-s <samples per axis, 1..16>]\n");
     return 2;
 }
 
@@ -38,7 +40,7 @@ int usage() {
 int main(int argc, char** argv) {
     std::string input, output, backend = "nvrtc";
     std::vector<std::string> textures;
-    int gpus = 1;
+    int gpus = 1, samples = 1;
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         auto value = [&]() -> const char* { return i + 1 < argc ? argv[++i] : nullptr; };
@@ -46,12 +48,13 @@ int main(int argc, char** argv) {
         else if (a == "-o" || a == "--output") { const char* v = value(); if (!v) return usage(); output = v; }
         else if (a == "-c" || a == "--cpus") { if (!value()) return usage(); }
         else if (a == "-g" || a == "--gpus") { const char* v = value(); if (!v) return usage(); gpus = std::atoi(v); }
+        else if (a == "-s" || a == "--samples") { const char* v = value(); if (!v) return usage(); samples = std::atoi(v); }
         else if (a == "-b" || a == "--backend") { const char* v = value(); if (!v) return usage(); backend = v; }
         else if (a == "-t" || a == "--textures") {
             while (i + 1 < argc && argv[i + 1][0] != '-') textures.push_back(argv[++i]);
         } else return usage();
     }
-    if (input.empty() || output.empty() || gpus < 1 || (backend != "nvrtc" && backend != "interp")) return usage();
+    if (input.empty() || output.empty() || gpus < 1 || samples < 1 || samples > 16 || (backend != "nvrtc" && backend != "interp")) return usage();
 
     // open(file)  (reference src/lib.rs:1227-1235)
     std::vector<uint8_t> scene;
@@ -84,6 +87,7 @@ int main(int argc, char** argv) {
     if (maray_cuda_load_maray(h, scene.data(), scene.size()) != MARAY_OK) return die("open");
     uint32_t w = 0, hgt = 0;
     maray_cuda_scene_size(h, &w, &hgt);
+    if (maray_cuda_set_samples(h, uint32_t(samples)) != MARAY_OK) return die("samples");
     maray_cuda_stats st;
     if (maray_cuda_compile(h, backend == "nvrtc" ? MARAY_BACKEND_NVRTC : MARAY_BACKEND_INTERP, &st) != MARAY_OK) return die("compile");
     std::vector<uint8_t> img(size_t(w) * hgt * 3);

@@ -348,12 +348,16 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
     prelude += "\n";
 
     char buf[320];
+    // The sampling state is the last parameter, after the chain kernels' frame arguments (whose offsets stay put), with
+    // a zero default: one sample per pixel at the integer coordinate.
     auto kernel_head = [&](std::string& out, const char* extra_args) {
         if (min_blocks_per_sm)
-            std::snprintf(buf, sizeof buf, "extern \"C\" __global__ void __launch_bounds__(%u, %u) %s(const MrParams p%s) {\n",
+            std::snprintf(buf, sizeof buf,
+                          "extern \"C\" __global__ void __launch_bounds__(%u, %u) %s(const MrParams p%s, const MrSampling sp = MrSampling{}) {\n",
                           block, min_blocks_per_sm, kJitKernelName, extra_args);
         else
-            std::snprintf(buf, sizeof buf, "extern \"C\" __global__ void __launch_bounds__(%u) %s(const MrParams p%s) {\n",
+            std::snprintf(buf, sizeof buf,
+                          "extern \"C\" __global__ void __launch_bounds__(%u) %s(const MrParams p%s, const MrSampling sp = MrSampling{}) {\n",
                           block, kJitKernelName, extra_args);
         out += buf;
         out += "  __shared__ unsigned int stage[3 * " + std::to_string(block) + " / 4];\n  (void)stage;\n";
@@ -362,20 +366,22 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         out += "  const unsigned int pix = p.p0 + (active ? j : 0u);\n";   // idle lanes redo pixel p0
         out += "  const unsigned int yi = pix / p.W;\n";
         out += "  const unsigned int xi = pix - yi * p.W;\n";
-        out += "  const double X = (double)xi;\n  const double Y = (double)yi;\n";   // `x as f64`
+        // `x as f64`, moved by the pass's sub-pixel offset (+0.0 with one sample per pixel: the same bits)
+        out += "  const double X = (double)xi + sp.ox;\n  const double Y = (double)yi + sp.oy;\n";
         out += "  const MrTexture* __restrict__ T = p.tex;\n  (void)T;\n";
         if (use_batches) out += "  mr_scratch_tables_init();\n";
     };
     auto store_call = [&](std::string& out, const std::vector<int32_t>& slot, const std::function<std::string(int32_t)>& frame_ref,
                           const Emitter& e, const std::vector<uint8_t>* in_scope) {
-        out += "  mr_store_block(p, stage, ";
+        std::string args;
         for (int c = 0; c < 3; c++) {
             uint32_t r = prog.root[c];
-            if (slot[r] >= 0 && !(in_scope && (*in_scope)[r])) out += frame_ref(slot[r]);
-            else e.operand(out, r);
-            out += ", ";
+            if (slot[r] >= 0 && !(in_scope && (*in_scope)[r])) args += frame_ref(slot[r]);
+            else e.operand(args, r);
+            args += ", ";
         }
-        out += "active, j);\n}\n";
+        out += "  if (sp.acc != nullptr) mr_store_sampled(p, sp, stage, " + args + "active, j);\n";   // a supersampling pass
+        out += "  else mr_store_block(p, stage, " + args + "active, j);\n}\n";
     };
 
     std::vector<std::string> modules;

@@ -93,16 +93,42 @@ struct MrParams {
     unsigned int row_base, rows;
 };
 
-// Packs one pixel into the block's staging tile and writes the tile with coalesced 16-byte
+// Supersampling (maray_cuda_set_samples): a frame of s x s samples per pixel is rendered as s*s passes of the same
+// kernel, each with one uniform sub-pixel offset; the kernel evaluates the scene at X = xi + ox, Y = yi + oy.  The u8
+// samples are summed in a uint16 x 3 accumulator (pixel p0+j of the launch at acc[3*j .. 3*j+2]) and the last pass
+// writes the box mean (sum + count/2) / count as RGB8.  A separate kernel parameter, not a field of MrParams: host
+// code that builds an MrParams and calls the kernel with it alone still gets the zero value, one sample per pixel.
+struct MrSampling {
+    double ox, oy;             // this pass's sub-pixel offset
+    unsigned short* acc;       // null: one sample per pixel, the epilogue stores RGB8 directly
+    unsigned int pass, count;  // pass in [0, count); count = s*s
+};
+
+// Adds this pass's u8 samples to the accumulator.  Returns true on the last pass, with (r8, g8, b8) resolved to the
+// pixel's RGB8; false otherwise (nothing to store yet).  `pass` and `count` are uniform, so is the result.
+__device__ __forceinline__ bool mr_accumulate(const MrSampling& sp, size_t idx, bool active, unsigned int& r8,
+                                              unsigned int& g8, unsigned int& b8) {
+    unsigned short* a = sp.acc + 3u * idx;
+    if (active && sp.pass != 0u) { r8 += a[0]; g8 += a[1]; b8 += a[2]; }
+    if (sp.pass + 1u < sp.count) {
+        if (active) { a[0] = (unsigned short)r8; a[1] = (unsigned short)g8; a[2] = (unsigned short)b8; }
+        return false;
+    }
+    const unsigned int half = sp.count >> 1;
+    r8 = (r8 + half) / sp.count; g8 = (g8 + half) / sp.count; b8 = (b8 + half) / sp.count;
+    return true;
+}
+
+// Packs one pixel's RGB8 into the block's staging tile and writes the tile with coalesced 16-byte
 // stores (768 B per 256 pixels).  Every thread of the block must call this.
-__device__ __forceinline__ void mr_store_block(const MrParams& p, unsigned int* stage, double r, double g, double b,
-                                               bool active, unsigned int j) {
+__device__ __forceinline__ void mr_store_rgb8(const MrParams& p, unsigned int* stage, unsigned int r8, unsigned int g8,
+                                              unsigned int b8, double r, double g, double b, bool active, unsigned int j) {
     const unsigned int tid = threadIdx.x;
     const unsigned int first = blockIdx.x * blockDim.x;
     unsigned char* sb = reinterpret_cast<unsigned char*>(stage);
-    sb[3u * tid + 0u] = (unsigned char)mr_as_u8(r);
-    sb[3u * tid + 1u] = (unsigned char)mr_as_u8(g);
-    sb[3u * tid + 2u] = (unsigned char)mr_as_u8(b);
+    sb[3u * tid + 0u] = (unsigned char)r8;
+    sb[3u * tid + 1u] = (unsigned char)g8;
+    sb[3u * tid + 2u] = (unsigned char)b8;
     if (p.f64_out != nullptr && active) {
         p.f64_out[j] = r;
         p.f64_out[(size_t)p.f64_plane + j] = g;
@@ -117,6 +143,22 @@ __device__ __forceinline__ void mr_store_block(const MrParams& p, unsigned int* 
     } else {
         for (unsigned int i = tid; i < 3u * valid; i += blockDim.x) dst[i] = sb[i];
     }
+}
+
+// The epilogue of a generated kernel: `as u8` of the three channels, then mr_store_rgb8.  (Its arguments stay as they
+// are: host code compiled against the generated text, like the oracle's JIT stand-in, puts its own store in its place.)
+__device__ __forceinline__ void mr_store_block(const MrParams& p, unsigned int* stage, double r, double g, double b,
+                                               bool active, unsigned int j) {
+    mr_store_rgb8(p, stage, mr_as_u8(r), mr_as_u8(g), mr_as_u8(b), r, g, b, active, j);
+}
+
+// The epilogue of a supersampling pass (sp.acc != null): adds the u8 samples to the accumulator; the last pass stores
+// the resolved pixels.  Every thread of the block must call this; before the last pass the whole block returns.
+__device__ __forceinline__ void mr_store_sampled(const MrParams& p, const MrSampling& sp, unsigned int* stage, double r,
+                                                 double g, double b, bool active, unsigned int j) {
+    unsigned int r8 = mr_as_u8(r), g8 = mr_as_u8(g), b8 = mr_as_u8(b);
+    if (!mr_accumulate(sp, j, active, r8, g8, b8)) return;
+    mr_store_rgb8(p, stage, r8, g8, b8, r, g, b, active, j);
 }
 
 #endif  // MARAY_DEVICE_SEM_CUH

@@ -206,15 +206,16 @@ __global__ void __launch_bounds__(512) maray_interp(const MrTileParams p, const 
 #pragma unroll
         for (int k = 0; k < P; k++) {
             const unsigned int xi = xs + k * B + tid;
-            xv[k] = (double)(xi < p.x1 ? xi : p.x1 - 1u);   // idle lanes redo the row's last pixel; `x as f64`, reference src/render.rs:25
-            yv[k] = (double)yi;
+            // idle lanes redo the row's last pixel; `x as f64` (reference src/render.rs:25) plus the pass's offset
+            xv[k] = (double)(xi < p.x1 ? xi : p.x1 - 1u) + p.ox;
+            yv[k] = (double)yi + p.oy;
             acc[k] = 0.0;
         }
         F.store(0, xv);
         if (all_wide) F.store(slot16, yv);
     }
     for (unsigned int i = tid; i < n_consts; i += B) scal[i] = consts[i];
-    if (!all_wide && tid == 0) scal[n_consts] = (double)yi;
+    if (!all_wide && tid == 0) scal[n_consts] = (double)yi + p.oy;   // Y stays uniform along the row in every pass
 
     // The stream is a whole number of chunks (bytecode_for_launch): all but the last end with YIELD, the last
     // is padded with END.
@@ -328,7 +329,8 @@ __global__ void __launch_bounds__(512) maray_interp(const MrTileParams p, const 
         }
     }
 
-    // `as u8` + RGB pack through the staging tile, then coalesced 16-byte stores.
+    // `as u8` + RGB pack through the staging tile, then coalesced 16-byte stores.  A supersampling pass first adds its
+    // samples to the accumulator; only the last pass stores (the pass index is uniform, so the whole block returns).
     const unsigned int ww = p.x1 - p.x0;
     const size_t row_first = (size_t)row * ww + (xs - p.x0);     // index of this block's first pixel in the output
     {
@@ -336,18 +338,24 @@ __global__ void __launch_bounds__(512) maray_interp(const MrTileParams p, const 
         F.load(out16, o_r);
         F.load(out16 + slot16, o_g);
         F.load(out16 + 2u * slot16, o_b);
+        MrSampling sp;
+        sp.acc = p.acc; sp.pass = p.pass; sp.count = p.count;
+        bool store = true;
 #pragma unroll
         for (int k = 0; k < P; k++) {
             const unsigned int l = k * B + tid;                  // pixel within the block
-            stage[3u * l + 0u] = (unsigned char)mr_as_u8(o_r[k]);
-            stage[3u * l + 1u] = (unsigned char)mr_as_u8(o_g[k]);
-            stage[3u * l + 2u] = (unsigned char)mr_as_u8(o_b[k]);
+            unsigned int r8 = mr_as_u8(o_r[k]), g8 = mr_as_u8(o_g[k]), b8 = mr_as_u8(o_b[k]);
+            if (p.acc != nullptr) store = mr_accumulate(sp, row_first + l, xs + l < p.x1, r8, g8, b8);
+            stage[3u * l + 0u] = (unsigned char)r8;
+            stage[3u * l + 1u] = (unsigned char)g8;
+            stage[3u * l + 2u] = (unsigned char)b8;
             if (p.f64_out != nullptr && xs + l < p.x1) {
                 p.f64_out[row_first + l] = o_r[k];
                 p.f64_out[(size_t)p.f64_plane + row_first + l] = o_g[k];
                 p.f64_out[2u * (size_t)p.f64_plane + row_first + l] = o_b[k];
             }
         }
+        if (!store) return;
     }
     __syncthreads();
     const unsigned int span = B * P;

@@ -20,6 +20,11 @@ struct MrTileParams {
     unsigned int nxb;              // blocks per row (set by launch_interp)
     unsigned int out_aligned;      // out is 16-byte aligned: full, aligned blocks store uint4
     unsigned int libm_exact;       // 1: sin/exp/ln return glibc's bits (device_libm_glibc.cuh, MARAY_LIBM=glibc)
+    // Supersampling pass (device_sem.cuh MrSampling): pixel (x, y) is evaluated at (x + ox, y + oy); with acc set its
+    // u8 samples are summed at acc[3 * i ..], i indexed like `out`, and the last of `count` passes stores the mean.
+    double ox, oy;
+    unsigned short* acc;           // null: one sample per pixel
+    unsigned int pass, count;
 };
 
 namespace maray {

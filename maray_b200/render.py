@@ -2,7 +2,7 @@
 
   reference                                   here
   ------------------------------------------  ---------------------------------------------
-  RenderMethod::{..}   src/lib.rs:1154-1173   RenderMethod.Cuda(gpus, report, backend)  (new arm)
+  RenderMethod::{..}   src/lib.rs:1154-1173   RenderMethod.Cuda(gpus, report, backend, samples)  (new arm)
   Report               src/report.rs:19-27    Report.none() / Report.row(n) / Report.duration(ms)
   Runtime<Textures>    src/lib.rs:72-98       Runtime(Textures(images))  (functions = textures.functions(n))
   gen_to_image         src/lib.rs:1177-1195   gen_to_image(method, rt, color, img, report)
@@ -56,6 +56,8 @@ class RenderMethod:
         # "nvrtc": the JIT sibling of wasm.rs, compiled before the first render; "interp": the bytecode kernel only
         backend: str = "auto"
         device_ids: Optional[Sequence[int]] = None
+        # anti-aliasing: samples x samples per pixel, box-filtered (CudaRenderer.set_samples); 1 is the reference's frame
+        samples: int = 1
 
 
 @dataclass
@@ -146,6 +148,13 @@ class CudaRenderer:
         """"fast" (default), "glibc" (exact mode: the bits of the host libm the reference calls, reference
         src/lib.rs:648-650) or "cuda" (libdevice).  Takes effect at the next compile."""
         self._check(self._L.maray_cuda_set_libm(self._h, {"fast": _lib.LIBM_FAST, "glibc": _lib.LIBM_GLIBC, "cuda": _lib.LIBM_CUDA}[libm]))
+
+    def set_samples(self, s: int) -> None:
+        """Supersampled anti-aliasing: s x s samples per pixel (1 <= s <= 16), box-filtered to RGB8 (maray_cuda_set_samples).
+        Sample (i, j) of pixel (x, y) is the scene at (x + o_i, y + o_j), o_k = (2k + 1 - s) * (1 / (2s)); the pixel is
+        the rounded integer mean of the samples' u8 values.  1, the default, is the reference's frame.  Takes effect at
+        the next render; nothing is recompiled."""
+        self._check(self._L.maray_cuda_set_samples(self._h, int(s)))
 
     def compile(self, backend: str = "nvrtc", libm: Optional[str] = None) -> dict:
         if libm is not None:
@@ -280,6 +289,7 @@ def gen_to_image(method: "RenderMethod.Cuda", rt: Runtime, color, img: np.ndarra
         r.set_textures(rt.ctx.images)
         r.load(color if isinstance(color, (bytes, bytearray)) else ([w, h], list(color)))
         stats = r.compile(method.backend)
+        r.set_samples(method.samples)
         r.set_report(method.report, report)
         stats.update({k: v for k, v in r.render_into(img).items() if k.endswith("_ms")})
         return stats

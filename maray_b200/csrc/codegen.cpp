@@ -232,6 +232,121 @@ std::vector<uint8_t> find_sign_only_sines(const Program& prog, const std::vector
     return mark;
 }
 
+// Guarded regions of the straight-line kernel.  For a boolean AND G = a && b (OP_MUL or OP_MIN of two booleans),
+// `false && anything == false`: when one operand (the guard) is false on every lane of a warp, the other (the body)
+// need not be evaluated at all, provided every value it consists of is read only through that operand edge of G.
+// Such a value is post-dominated by the edge: every path from it to the program's outputs passes through it.  With one
+// pseudo-node per operand edge of each AND, the body of an edge is the edge's subtree of the post-dominator tree of
+// the use graph, so bodies of different edges are nested or disjoint and the regions form a tree.  Every read counts:
+// both operands, the three channel roots, and the NOT form's extra read of b (`1 + -(b)` is emitted as `!b`).
+struct GuardRegion {
+    uint32_t guard;    // evaluated in place, before the region
+    uint32_t body;     // evaluated inside `if (mr_warp_any(guard))`
+};
+struct GuardRegions {
+    std::vector<GuardRegion> regions;
+    std::vector<int32_t> owner;       // value -> innermost region whose body holds it, or -1
+    std::vector<int32_t> rooted_at;   // value -> the region whose AND it is, or -1
+};
+
+GuardRegions find_guard_regions(const Program& prog, const std::vector<uint8_t>& booleans, const std::vector<uint8_t>& sign_only,
+                                const std::function<uint32_t(uint32_t)>& not_operand) {
+    const uint32_t n = uint32_t(prog.nodes.size());
+    auto is_value = [&](uint32_t id) { const Op o = prog.nodes[id].op; return o != OP_CONST && o != OP_X && o != OP_Y; };
+    // candidates: ANDs of two booleans, neither a constant
+    std::vector<int32_t> cand(n, -1);
+    std::vector<uint32_t> cands;
+    for (uint32_t i = 0; i < n; i++) {
+        const Node& nd = prog.nodes[i];
+        if ((nd.op == OP_MUL || nd.op == OP_MIN) && booleans[i] && is_value(nd.a) && is_value(nd.b)) {
+            cand[i] = int32_t(cands.size());
+            cands.push_back(i);
+        }
+    }
+    GuardRegions out;
+    out.owner.assign(n, -1);
+    out.rooted_at.assign(n, -1);
+    if (cands.empty()) return out;
+    // extended nodes: values 0..n-1, EXIT = n, the pseudo-node of edge k of candidate c = n + 1 + 2c + k
+    const uint32_t exit_node = n, n_ext = n + 1 + 2 * uint32_t(cands.size());
+    auto edge_node = [&](uint32_t c, uint32_t k) { return n + 1 + 2 * c + k; };
+    // successors (readers) of every value, in CSR form
+    std::vector<uint32_t> deg(n + 1, 0), succ;
+    auto for_each_read = [&](auto&& fn) {   // fn(operand, successor)
+        for (uint32_t r = 0; r < n; r++) {
+            const Node& nd = prog.nodes[r];
+            if (!is_value(r)) continue;
+            if (cand[r] >= 0) { fn(nd.a, edge_node(uint32_t(cand[r]), 0)); fn(nd.b, edge_node(uint32_t(cand[r]), 1)); continue; }
+            if (op_is_unary(nd.op) || op_is_binary(nd.op)) fn(nd.a, r);
+            if (op_is_binary(nd.op)) fn(nd.b, r);
+            if (uint32_t x = not_operand(r); x != UINT32_MAX) fn(x, r);
+        }
+        for (int c = 0; c < 3; c++) fn(prog.root[c], exit_node);
+    };
+    for_each_read([&](uint32_t v, uint32_t) { deg[v + 1]++; });
+    for (uint32_t i = 0; i < n; i++) deg[i + 1] += deg[i];
+    succ.resize(deg[n]);
+    {
+        std::vector<uint32_t> fill(deg.begin(), deg.end() - 1);
+        for_each_read([&](uint32_t v, uint32_t s) { succ[fill[v]++] = s; });
+    }
+    // immediate post-dominators: readers come after their operands, so one pass from the outputs backwards suffices
+    std::vector<uint32_t> ipdom(n_ext, exit_node), depth(n_ext, 0);
+    auto meet = [&](uint32_t x, uint32_t y) {
+        while (x != y) {
+            if (depth[x] < depth[y]) std::swap(x, y);
+            x = ipdom[x];
+        }
+        return x;
+    };
+    for (uint32_t v = n; v-- > 0;) {
+        // A value nothing reads (none exist: every node is reachable from a root) keeps EXIT; so would its edge
+        // pseudo-nodes if it were an AND, which is harmless -- only values as dead as it could fall under them.
+        if (!is_value(v) || deg[v] == deg[v + 1]) continue;
+        uint32_t p = succ[deg[v]];
+        for (uint32_t e = deg[v] + 1; e < deg[v + 1]; e++) p = meet(p, succ[e]);
+        ipdom[v] = p;
+        depth[v] = depth[p] + 1;
+        if (cand[v] >= 0)
+            for (uint32_t k = 0; k < 2; k++) {
+                ipdom[edge_node(uint32_t(cand[v]), k)] = v;
+                depth[edge_node(uint32_t(cand[v]), k)] = depth[v] + 1;
+            }
+    }
+    // weight of each post-dominator subtree: about what evaluating it costs per pixel
+    auto weight = [&](uint32_t v) -> uint32_t {
+        switch (prog.nodes[v].op) {
+        case OP_NEG: return 0;                                   // folded into its reader's operand
+        case OP_SIN: case OP_EXP: case OP_LN: return !sign_only.empty() && sign_only[v] ? 7 : 16;
+        default: return 1;
+        }
+    };
+    std::vector<uint64_t> sub(n_ext, 0);
+    for (uint32_t v = 0; v < n; v++) {
+        if (!is_value(v)) continue;
+        if (cand[v] >= 0) sub[v] += sub[edge_node(uint32_t(cand[v]), 0)] + sub[edge_node(uint32_t(cand[v]), 1)];
+        sub[v] += weight(v);
+        sub[ipdom[v]] += sub[v];
+    }
+    // regions and their members, from the outputs backwards: a value belongs to the innermost region of its post-dominator
+    std::vector<int32_t> ext_owner(n_ext, -1);
+    for (uint32_t v = n; v-- > 0;) {
+        if (!is_value(v)) continue;
+        out.owner[v] = ext_owner[v] = ext_owner[ipdom[v]];
+        if (cand[v] < 0) continue;
+        const uint32_t c = uint32_t(cand[v]);
+        const uint32_t kb = sub[edge_node(c, 1)] > sub[edge_node(c, 0)] ? 1 : 0;   // the dearer operand is the body
+        ext_owner[edge_node(c, 0)] = ext_owner[edge_node(c, 1)] = ext_owner[v];
+        if (sub[edge_node(c, kb)] >= kGuardBodyMinWeight) {
+            const Node& nd = prog.nodes[v];
+            out.rooted_at[v] = int32_t(out.regions.size());
+            ext_owner[edge_node(c, kb)] = int32_t(out.regions.size());
+            out.regions.push_back({kb ? nd.a : nd.b, kb ? nd.b : nd.a});
+        }
+    }
+    return out;
+}
+
 // Common generator.  Three forms:
 //   * one kernel (programs up to opt.segment_values values);
 //   * larger programs, opt.chain: one KERNEL per segment, each its own translation unit (modules[s]); values
@@ -337,6 +452,9 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         }
     }
     const bool use_batches = !em.inline_trans;
+    // guarded regions: the straight-line form only (one kernel, sin/exp/ln inlined), like the sign-only sines
+    const GuardRegions guards = opt.boolean_logic && !segmented && !use_batches
+                                    ? find_guard_regions(prog, booleans, sign_only, not_operand) : GuardRegions{};
     std::string prelude = "// generated by maray_b200 (NVRTC back end); compiled with --fmad=false\n";
     // one private instance of the batch helpers per segment function of a single-unit program
     const bool private_helpers = use_batches && segmented && !chain;
@@ -535,6 +653,28 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
                 std::snprintf(buf, sizeof buf, "  mr_seg%u(F, X, Y, T);\n", s);
                 src += buf;
             }
+        } else if (!guards.regions.empty()) {
+            // Body values leave their places in the schedule and are emitted, in schedule order, where their AND is.
+            // Valid: a body value's other operands precede it and so precede the AND, and nothing outside the body reads
+            // it.  All 32 lanes reach every vote: idle lanes redo pixel p0, and an inner region sits inside its outer
+            // region's warp-uniform branch.
+            std::vector<std::vector<uint32_t>> members(guards.regions.size() + 1);
+            for (uint32_t id : order) members[size_t(guards.owner[id] + 1)].push_back(id);
+            std::function<void(int32_t)> emit_members = [&](int32_t r) {
+                for (uint32_t id : members[size_t(r + 1)]) {
+                    const int32_t g = guards.rooted_at[id];
+                    if (g < 0) { em.statement(src, id); continue; }
+                    const GuardRegion& gr = guards.regions[size_t(g)];
+                    std::snprintf(buf, sizeof buf, "  bool b%u = false;\n  if (mr_warp_any(", id);
+                    src += buf; em.bool_operand(src, gr.guard); src += ")) {\n";
+                    emit_members(g);
+                    std::snprintf(buf, sizeof buf, "  b%u = ", id);
+                    src += buf; em.bool_operand(src, gr.guard); src += " && "; em.bool_operand(src, gr.body); src += ";\n  }\n";
+                    std::snprintf(buf, sizeof buf, "  const double v%u = b%u ? 1.0 : 0.0;\n", id, id);
+                    src += buf;
+                }
+            };
+            emit_members(-1);
         } else {
             emit_range(src, em, 0, order.size(), lref, "");
         }

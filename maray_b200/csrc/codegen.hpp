@@ -70,6 +70,14 @@ struct CodegenInfo {
 // Names of the generated kernels (extern "C").
 extern const char* const kJitKernelName;
 constexpr uint32_t kOneBlockPerSmValues = 4096;   // CodegenOptions::auto_shape
+// Guarded regions (codegen.cpp find_guard_regions): a boolean AND whose dearer operand is read by nothing else
+// evaluates that operand only when the other one is true on some lane of the warp.  A region is made when the skipped
+// operand weighs at least this much (one per value, 7 per sign-only sine, 16 per inlined sin/exp/ln).  Chess's texture
+// operands weigh 40-51 and get a region each; the ANDs inside them (23-25) and beside them (11) do not pay: measured,
+// chess_4k on one B200, profiles/r04_guard_threshold_sweep.jsonl: 3.517 ms without regions, 2.939 ms with the
+// 128 texture regions, 2.943 / 2.982 / 3.058 ms when the 15 / 128 / 207 smaller ANDs get regions too.  sdf, textured
+// and deep have no AND this heavy.
+constexpr uint32_t kGuardBodyMinWeight = 32;
 
 // One translation unit (segment functions, if any, as __noinline__ functions of the same unit).
 std::string generate_cuda_source(const Program& prog, const CodegenOptions& opt, CodegenInfo* info);

@@ -37,6 +37,18 @@ __device__ __forceinline__ double mr_pick(bool take_b, double a, double b) {
 __device__ __forceinline__ double mr_max(double a, double b) { return mr_pick((b > a) || (a != a), a, b); }
 __device__ __forceinline__ double mr_min(double a, double b) { return mr_pick((b < a) || (a != a), a, b); }
 
+// The vote in front of a guarded region of a generated kernel (codegen.cpp find_guard_regions): is the guard true on
+// some lane of this warp?  Every lane of the warp reaches every vote.  The host builds of the text run one thread at a
+// time: there the guard decides alone, or, with MR_HOST_GUARDS_ALWAYS, every region is evaluated at every pixel -- the
+// two extremes between which the GPU lies, warp by warp.
+#if defined(MR_HOST_GUARDS_ALWAYS)
+static inline bool mr_warp_any(bool) { return true; }
+#elif defined(MR_HOST_TEXT)
+static inline bool mr_warp_any(bool b) { return b; }
+#else
+__device__ __forceinline__ bool mr_warp_any(bool b) { return __any_sync(0xffffffffu, b); }
+#endif
+
 // Recip(a) = 1.0 / a, IEEE round-to-nearest.  reference src/lib.rs:642
 __device__ __forceinline__ double mr_recip(double v) { return __drcp_rn(v); }
 // Sqrt(a), IEEE round-to-nearest.  reference src/lib.rs:643

@@ -42,7 +42,10 @@ def fp64_ops_per_pixel(stats: dict) -> int:
 def executed_counts(cubin: bytes, kernel: str = "maray_jit"):
     """FP64-pipe and total SASS instructions of `kernel` in a cubin, via `cuobjdump -sass` (None if the tool is
     missing).  For a straight-line kernel (one unit, no batched helper loops) this is what one pixel executes, the
-    never-taken out-of-range blocks aside (a handful of integer instructions per sine)."""
+    never-taken out-of-range blocks aside (a handful of integer instructions per sine).  None as well when the kernel
+    has guarded regions (a warp vote, VOTE, in its SASS; codegen.cpp find_guard_regions): a warp runs a region's body
+    only when its guard is true on some lane, so what a pixel executes depends on the frame and no longer on the code
+    alone, and the static count would overstate it."""
     import os
     import re
     import shutil
@@ -64,6 +67,8 @@ def executed_counts(cubin: bytes, kernel: str = "maray_jit"):
         op = m.group(1)
         if op == "NOP":
             continue
+        if op == "VOTE":
+            return None
         total += 1
         fp64 += op in ("DFMA", "DMUL", "DADD", "DSETP")
         if op == "EXIT" and total > 64:      # end of the kernel's own path: out-of-line device functions (libdevice

@@ -83,10 +83,13 @@ typedef struct maray_cuda_stats {
     uint32_t tier_rows_interp;    /* MARAY_BACKEND_AUTO, last render: rows the interpreter rendered before the
                                      generated kernels took over (0 once they are installed)               */
     uint32_t jit_active;          /* 1 when launches go to the generated kernels                           */
-    uint32_t jit_block;           /* generated kernels: threads (= pixels) per block                       */
+    uint32_t jit_block;           /* generated kernels: threads per block                                  */
     uint32_t jit_round_pixels;    /* generated kernels: pixels one round of resident blocks covers on the first GPU
-                                     (SMs x resident blocks x jit_block; 0 without a GPU).  A band or row chunk that is
-                                     a whole number of rounds long pays no tail: hosts that cut a frame can cut there */
+                                     (SMs x resident blocks x jit_block x jit_pixels_per_thread; 0 without a GPU).  A
+                                     band or row chunk that is a whole number of rounds long pays no tail: hosts that
+                                     cut a frame can cut there */
+    uint32_t jit_pixels_per_thread; /* generated kernels: pixels per thread (2 with pixel pairs; a block covers
+                                     jit_block x jit_pixels_per_thread consecutive pixels)                    */
     /* timings, milliseconds */
     double lower_ms;              /* Expr -> SSA                                                     */
     double codegen_ms;            /* SSA -> source / bytecode                                        */

@@ -28,7 +28,8 @@ class Stats(ctypes.Structure):
             "dag_depth", "legacy_layout", "backend", "interp_instructions", "interp_slots",
             "jit_segments", "jit_frame_slots", "jit_registers", "jit_source_bytes", "jit_cubin_bytes",
             "jit_units", "jit_compile_threads", "jit_cache_hit", "interp_uniform_slots", "interp_block",
-            "interp_pixels_per_thread", "tier_rows_interp", "jit_active", "jit_block", "jit_round_pixels")]
+            "interp_pixels_per_thread", "tier_rows_interp", "jit_active", "jit_block", "jit_round_pixels",
+            "jit_pixels_per_thread")]
         + [("lower_ms", ctypes.c_double), ("codegen_ms", ctypes.c_double), ("nvrtc_ms", ctypes.c_double),
            ("load_ms", ctypes.c_double), ("kernel_ms", ctypes.c_double * 8), ("gather_ms", ctypes.c_double),
            ("d2h_ms", ctypes.c_double), ("render_ms", ctypes.c_double)]

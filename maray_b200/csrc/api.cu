@@ -121,6 +121,7 @@ struct maray_cuda {
     int libm = MARAY_LIBM_FAST;                        // maray_cuda_set_libm / MARAY_LIBM
     uint32_t samples = 1;                              // maray_cuda_set_samples: s x s samples per pixel
     unsigned jit_block = 256;
+    unsigned jit_ppt = 1;             // pixels per thread of the generated kernel (CodegenInfo::pixels_per_thread)
     unsigned jit_dyn_smem = 0;                         // dynamic shared memory of the generated kernel
     unsigned jit_maxreg = 0;
     bool jit_chain = false;                            // one kernel per segment, launched in order over a global frame
@@ -514,6 +515,7 @@ int jit_build(const Program& prog, JitBuild* jb, bool cached_only, const std::at
     if (const char* e = std::getenv("MARAY_JIT_SIGN_OF_SINE")) copt.sign_of_sine = std::strtoul(e, nullptr, 10) != 0;
     if (const char* e = std::getenv("MARAY_JIT_BLOCK")) { copt.block = uint32_t(std::strtoul(e, nullptr, 10)); copt.auto_shape = false; }
     if (const char* e = std::getenv("MARAY_JIT_MIN_BLOCKS")) { copt.min_blocks_per_sm = uint32_t(std::strtoul(e, nullptr, 10)); copt.auto_shape = false; }
+    if (const char* e = std::getenv("MARAY_JIT_PAIRS")) copt.pixel_pairs = std::strtoul(e, nullptr, 10) != 0;
     jb->maxreg = 0;
     if (const char* e = std::getenv("MARAY_JIT_MAXREG")) jb->maxreg = unsigned(std::strtoul(e, nullptr, 10));
     // Programs above the segment size compile as a CHAIN of kernels, one translation unit each (codegen.hpp):
@@ -554,6 +556,7 @@ void fill_jit_stats(maray_cuda* h) {
     h->stats.jit_cache_hit = jb.cache_hit;
     h->stats.jit_registers = jb.registers;
     h->stats.jit_block = jb.info.block;
+    h->stats.jit_pixels_per_thread = jb.info.pixels_per_thread;
     h->stats.jit_round_pixels = 0;
     h->stats.jit_cubin_bytes = 0;
     for (const std::vector<char>& c : jb.cubins) h->stats.jit_cubin_bytes += uint32_t(c.size());
@@ -563,6 +566,7 @@ void fill_jit_stats(maray_cuda* h) {
 int jit_install(maray_cuda* h, JitBuild&& jb) {
     h->jit = std::move(jb);
     h->jit_block = h->jit.info.block;
+    h->jit_ppt = h->jit.info.pixels_per_thread;
     h->jit_dyn_smem = h->jit.info.dynamic_smem_bytes;
     h->jit_chain = h->jit.info.chain;
     h->jit_frame_slots = h->jit.info.frame_slots;
@@ -588,7 +592,7 @@ int jit_install(maray_cuda* h, JitBuild&& jb) {
                 const size_t smem_per_block = h->jit_dyn_smem + fa.sharedSizeBytes + 1024;
                 unsigned blocks = std::min(std::min(65536u / ((regs + 7) / 8 * 8 * blk), 2048u / blk), 32u);
                 blocks = std::max(1u, std::min<unsigned>(blocks, unsigned(233472 / smem_per_block)));      // resident blocks per SM
-                if (&g == &h->gpus[0] && &cubin == &h->jit.cubins[0]) h->stats.jit_round_pixels = uint32_t(g.sms) * blocks * blk;
+                if (&g == &h->gpus[0] && &cubin == &h->jit.cubins[0]) h->stats.jit_round_pixels = uint32_t(g.sms) * blocks * blk * h->jit_ppt;
                 int pct = -1;
                 if (const char* e = std::getenv("MARAY_JIT_CARVEOUT")) pct = int(std::strtol(e, nullptr, 10));   // percent; -1 = computed, -2 = driver's choice
                 if (pct == -1) {
@@ -667,7 +671,8 @@ int launch_pass(maray_cuda* h, Gpu& g, uint32_t w, uint32_t p0, uint32_t n, uint
         if (!h->jit_chain) {
             MrSampling a = sp;
             void* args[] = {&p, &a};
-            const unsigned grid = (n + h->jit_block - 1) / h->jit_block;
+            const unsigned span = h->jit_block * h->jit_ppt;   // pixels per block
+            const unsigned grid = unsigned((size_t(n) + span - 1) / span);
             CU_TRY(h, cudaLaunchKernel(reinterpret_cast<const void*>(g.jit_kernels[0]), dim3(grid), dim3(h->jit_block), args, h->jit_dyn_smem, stream));
         } else {
             // Chain form: the segment kernels run in order over a chunk of pixels whose frame (values that cross

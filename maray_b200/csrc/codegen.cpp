@@ -46,13 +46,16 @@ struct Emitter {
     // Sines that are only ever asked for their sign (see find_sign_only_sines): never materialised.
     const std::vector<uint8_t>* sign_only = nullptr;
     bool is_sign_only(uint32_t id) const { return sign_only && (*sign_only)[id]; }
+    // Appended to the name of every per-pixel value (vN, bN, X, Y): "" for a thread's first pixel, "_b" for the second
+    // pixel of a pixel pair.  Constants and the constant bank are shared.
+    const char* sfx = "";
 
     bool is_bool(uint32_t id) const { return boolean && (*boolean)[id]; }
     void bool_operand(std::string& s, uint32_t id) const {
         const Node& n = P.nodes[id];
         if (n.op == OP_CONST) { s += (n.k != 0.0) ? "true" : "false"; return; }
-        char buf[16];
-        std::snprintf(buf, sizeof buf, "b%u", id);
+        char buf[24];
+        std::snprintf(buf, sizeof buf, "b%u%s", id, sfx);
         s += buf;
     }
     // `const bool bN = vN != 0.0;` after a boolean value arrived as a double (frame import)
@@ -73,10 +76,10 @@ struct Emitter {
             } else append_const(s, n.k);
             return;
         }
-        if (n.op == OP_X) { s += "X"; return; }
-        if (n.op == OP_Y) { s += "Y"; return; }
-        char buf[16];
-        std::snprintf(buf, sizeof buf, "v%u", id);
+        if (n.op == OP_X) { s += "X"; s += sfx; return; }
+        if (n.op == OP_Y) { s += "Y"; s += sfx; return; }
+        char buf[24];
+        std::snprintf(buf, sizeof buf, "v%u%s", id, sfx);
         s += buf;
     }
 
@@ -113,7 +116,7 @@ struct Emitter {
         if (is_bool(id)) {
             // 0/1-valued: compares and bit logic instead of FP64 multiplies, min/max and selects.  The
             // double shadow is what every non-boolean consumer reads; unused shadows are dead code.
-            std::snprintf(buf, sizeof buf, "  const bool b%u = ", id);
+            std::snprintf(buf, sizeof buf, "  const bool b%u%s = ", id, sfx);
             s += buf;
             switch (n.op) {
             case OP_STEP:
@@ -133,11 +136,11 @@ struct Emitter {
             case OP_MAX: s += "("; bool_operand(s, n.a); s += " || "; bool_operand(s, n.b); s += ")"; break;
             default: s += "false"; break;
             }
-            std::snprintf(buf, sizeof buf, ";\n  const double v%u = b%u ? 1.0 : 0.0;\n", id, id);
+            std::snprintf(buf, sizeof buf, ";\n  const double v%u%s = b%u%s ? 1.0 : 0.0;\n", id, sfx, id, sfx);
             s += buf;
             return;
         }
-        std::snprintf(buf, sizeof buf, "  const double v%u = ", id);
+        std::snprintf(buf, sizeof buf, "  const double v%u%s = ", id, sfx);
         s += buf;
         auto un = [&](const char* pre, const char* post) { s += pre; operand(s, n.a); s += post; };
         auto bin = [&](const char* pre, const char* mid, const char* post) {
@@ -455,6 +458,14 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
     // guarded regions: the straight-line form only (one kernel, sin/exp/ln inlined), like the sign-only sines
     const GuardRegions guards = opt.boolean_logic && !segmented && !use_batches
                                     ? find_guard_regions(prog, booleans, sign_only, not_operand) : GuardRegions{};
+    // Pixel pairs: a kernel with guarded regions evaluates two pixels per thread, every statement once for each, so each
+    // dependent chain of compares has an independent twin beside it and one vote and branch cover two pixels.
+    const bool pairs = opt.pixel_pairs && !guards.regions.empty();
+    const uint32_t ppt = pairs ? 2 : 1;
+    Emitter em_b = em;
+    em_b.sfx = "_b";
+    std::vector<const Emitter*> pixels{&em};
+    if (pairs) pixels.push_back(&em_b);
     std::string prelude = "// generated by maray_b200 (NVRTC back end); compiled with --fmad=false\n";
     // one private instance of the batch helpers per segment function of a single-unit program
     const bool private_helpers = use_batches && segmented && !chain;
@@ -478,14 +489,28 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
                           "extern \"C\" __global__ void __launch_bounds__(%u) %s(const MrParams p%s, const MrSampling sp = MrSampling{}) {\n",
                           block, kJitKernelName, extra_args);
         out += buf;
-        out += "  __shared__ unsigned int stage[3 * " + std::to_string(block) + " / 4];\n  (void)stage;\n";
-        out += "  const unsigned int j = blockIdx.x * blockDim.x + threadIdx.x;\n";
-        out += "  const bool active = j < p.n;\n";
-        out += "  const unsigned int pix = p.p0 + (active ? j : 0u);\n";   // idle lanes redo pixel p0
-        out += "  const unsigned int yi = pix / p.W;\n";
-        out += "  const unsigned int xi = pix - yi * p.W;\n";
-        // `x as f64`, moved by the pass's sub-pixel offset (+0.0 with one sample per pixel: the same bits)
-        out += "  const double X = (double)xi + sp.ox;\n  const double Y = (double)yi + sp.oy;\n";
+        out += "  __shared__ unsigned int stage[3 * " + std::to_string(block * ppt) + " / 4];\n  (void)stage;\n";
+        if (pairs) {
+            // the block covers 2 * blockDim.x consecutive pixels; this thread's two are one half apart (both coalesced)
+            out += "  const unsigned int j = blockIdx.x * 2u * blockDim.x + threadIdx.x;\n";
+            out += "  const unsigned int j_b = j + blockDim.x;\n";
+        } else {
+            out += "  const unsigned int j = blockIdx.x * blockDim.x + threadIdx.x;\n";
+        }
+        for (const Emitter* e : pixels) {
+            const char* s = e->sfx;
+            std::snprintf(buf, sizeof buf, "  const bool active%s = j%s < p.n;\n", s, s);
+            out += buf;
+            std::snprintf(buf, sizeof buf, "  const unsigned int pix%s = p.p0 + (active%s ? j%s : 0u);\n", s, s, s);   // idle lanes redo pixel p0
+            out += buf;
+            std::snprintf(buf, sizeof buf, "  const unsigned int yi%s = pix%s / p.W;\n  const unsigned int xi%s = pix%s - yi%s * p.W;\n",
+                          s, s, s, s, s);
+            out += buf;
+            // `x as f64`, moved by the pass's sub-pixel offset (+0.0 with one sample per pixel: the same bits)
+            std::snprintf(buf, sizeof buf, "  const double X%s = (double)xi%s + sp.ox;\n  const double Y%s = (double)yi%s + sp.oy;\n",
+                          s, s, s, s);
+            out += buf;
+        }
         out += "  const MrTexture* __restrict__ T = p.tex;\n  (void)T;\n";
         if (use_batches) out += "  mr_scratch_tables_init();\n";
     };
@@ -497,6 +522,14 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             if (slot[r] >= 0 && !(in_scope && (*in_scope)[r])) args += frame_ref(slot[r]);
             else e.operand(args, r);
             args += ", ";
+        }
+        if (pairs) {
+            args += "active, j, ";
+            for (int c = 0; c < 3; c++) { em_b.operand(args, prog.root[c]); args += ", "; }
+            args += "active_b, j_b);\n";
+            out += "  if (sp.acc != nullptr) mr_store_sampled_pair(p, sp, stage, " + args;
+            out += "  else mr_store_block_pair(p, stage, " + args + "}\n";
+            return;
         }
         out += "  if (sp.acc != nullptr) mr_store_sampled(p, sp, stage, " + args + "active, j);\n";   // a supersampling pass
         out += "  else mr_store_block(p, stage, " + args + "active, j);\n}\n";
@@ -657,21 +690,39 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             // Body values leave their places in the schedule and are emitted, in schedule order, where their AND is.
             // Valid: a body value's other operands precede it and so precede the AND, and nothing outside the body reads
             // it.  All 32 lanes reach every vote: idle lanes redo pixel p0, and an inner region sits inside its outer
-            // region's warp-uniform branch.
+            // region's warp-uniform branch.  With pixel pairs every statement is emitted for both pixels, one after the
+            // other, and one vote on `guard || guard_b` covers the two: a body evaluated for a pixel whose own guard is
+            // false is discarded by that pixel's `guard && body`, as on a lane whose guard is false.
             std::vector<std::vector<uint32_t>> members(guards.regions.size() + 1);
             for (uint32_t id : order) members[size_t(guards.owner[id] + 1)].push_back(id);
             std::function<void(int32_t)> emit_members = [&](int32_t r) {
                 for (uint32_t id : members[size_t(r + 1)]) {
                     const int32_t g = guards.rooted_at[id];
-                    if (g < 0) { em.statement(src, id); continue; }
+                    if (g < 0) {
+                        for (const Emitter* e : pixels) e->statement(src, id);
+                        continue;
+                    }
                     const GuardRegion& gr = guards.regions[size_t(g)];
-                    std::snprintf(buf, sizeof buf, "  bool b%u = false;\n  if (mr_warp_any(", id);
-                    src += buf; em.bool_operand(src, gr.guard); src += ")) {\n";
+                    for (const Emitter* e : pixels) {
+                        std::snprintf(buf, sizeof buf, "  bool b%u%s = false;\n", id, e->sfx);
+                        src += buf;
+                    }
+                    src += "  if (mr_warp_any(";
+                    for (const Emitter* e : pixels) {
+                        if (e != pixels[0]) src += " || ";
+                        e->bool_operand(src, gr.guard);
+                    }
+                    src += ")) {\n";
                     emit_members(g);
-                    std::snprintf(buf, sizeof buf, "  b%u = ", id);
-                    src += buf; em.bool_operand(src, gr.guard); src += " && "; em.bool_operand(src, gr.body); src += ";\n  }\n";
-                    std::snprintf(buf, sizeof buf, "  const double v%u = b%u ? 1.0 : 0.0;\n", id, id);
-                    src += buf;
+                    for (const Emitter* e : pixels) {
+                        std::snprintf(buf, sizeof buf, "  b%u%s = ", id, e->sfx);
+                        src += buf; e->bool_operand(src, gr.guard); src += " && "; e->bool_operand(src, gr.body); src += ";\n";
+                    }
+                    src += "  }\n";
+                    for (const Emitter* e : pixels) {
+                        std::snprintf(buf, sizeof buf, "  const double v%u%s = b%u%s ? 1.0 : 0.0;\n", id, e->sfx, id, e->sfx);
+                        src += buf;
+                    }
                 }
             };
             emit_members(-1);
@@ -688,6 +739,7 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         info->frame_slots = segmented ? frame_slots : 0;
         info->transcendentals_inlined = em.inline_trans;
         info->block = block;
+        info->pixels_per_thread = ppt;
         // argument rows + result rows, then glibc's exp and log tables
         info->dynamic_smem_bytes = use_batches ? 2 * kScratchRows * block * uint32_t(sizeof(double)) + 4096 : 0;
     }

@@ -56,6 +56,11 @@ struct CodegenOptions {
     // Evaluate values that are exactly 0.0 or 1.0 at every pixel (step, products/min/max of such
     // values, 1 - b) as boolean logic instead of FP64 arithmetic.  Exact: no channel bit changes.
     bool boolean_logic = true;
+    // Pixel pairs: a straight-line kernel with guarded regions evaluates two pixels per thread, statement by statement
+    // interleaved (thread t of a block of B: pixels t and B + t of the block's 2B), so the dependent compares of one
+    // pixel have independent work beside them and one warp vote serves two pixels.  Other kernels keep one pixel per
+    // thread (MARAY_JIT_PAIRS=0 for A/B).
+    bool pixel_pairs = true;
 };
 
 struct CodegenInfo {
@@ -64,6 +69,7 @@ struct CodegenInfo {
     uint32_t frame_slots = 0;       // doubles per pixel of the frame that carries values across cuts (0 when not segmented)
     bool transcendentals_inlined = true;
     uint32_t block = 256;           // threads per block the kernel must be launched with
+    uint32_t pixels_per_thread = 1; // 2 with pixel pairs: a block covers block * pixels_per_thread pixels
     uint32_t dynamic_smem_bytes = 0; // dynamic shared memory the kernel must be launched with (batch scratch + tables)
 };
 

@@ -173,4 +173,62 @@ __device__ __forceinline__ void mr_store_sampled(const MrParams& p, const MrSamp
     mr_store_rgb8(p, stage, r8, g8, b8, r, g, b, active, j);
 }
 
+// Pixel pairs (codegen.cpp): a block of B threads covers the 2B launch pixels from blockIdx.x * 2B, and thread t
+// evaluates pixels j = that + t and j_b = j + B.  The two-pixel forms of mr_store_rgb8 / mr_store_block /
+// mr_store_sampled; the staging tile holds 3 x 2B bytes.  A block may start at or past p.n (host drivers that size
+// the grid for one pixel per thread): it stores nothing.
+__device__ __forceinline__ void mr_store_rgb8_pair(const MrParams& p, unsigned int* stage, unsigned int r8, unsigned int g8,
+                                                   unsigned int b8, double r, double g, double b, bool active, unsigned int j,
+                                                   unsigned int r8_b, unsigned int g8_b, unsigned int b8_b, double r_b,
+                                                   double g_b, double b_b, bool active_b, unsigned int j_b) {
+    const unsigned int tid = threadIdx.x, tid_b = tid + blockDim.x;
+    const unsigned int span = 2u * blockDim.x, first = blockIdx.x * span;
+    unsigned char* sb = reinterpret_cast<unsigned char*>(stage);
+    sb[3u * tid + 0u] = (unsigned char)r8;
+    sb[3u * tid + 1u] = (unsigned char)g8;
+    sb[3u * tid + 2u] = (unsigned char)b8;
+    sb[3u * tid_b + 0u] = (unsigned char)r8_b;
+    sb[3u * tid_b + 1u] = (unsigned char)g8_b;
+    sb[3u * tid_b + 2u] = (unsigned char)b8_b;
+    if (p.f64_out != nullptr) {
+        if (active) {
+            p.f64_out[j] = r;
+            p.f64_out[(size_t)p.f64_plane + j] = g;
+            p.f64_out[2u * (size_t)p.f64_plane + j] = b;
+        }
+        if (active_b) {
+            p.f64_out[j_b] = r_b;
+            p.f64_out[(size_t)p.f64_plane + j_b] = g_b;
+            p.f64_out[2u * (size_t)p.f64_plane + j_b] = b_b;
+        }
+    }
+    __syncthreads();
+    const unsigned int valid = first >= p.n ? 0u : ((p.n - first < span) ? (p.n - first) : span);
+    unsigned char* dst = p.out + 3u * (size_t)first;
+    if (p.out_aligned && valid == span && (span & 15u) == 0u) {
+        const unsigned int vecs = 3u * span / 16u;   // fewer than the block's threads
+        if (tid < vecs) reinterpret_cast<uint4*>(dst)[tid] = reinterpret_cast<const uint4*>(stage)[tid];
+    } else {
+        for (unsigned int i = tid; i < 3u * valid; i += blockDim.x) dst[i] = sb[i];
+    }
+}
+
+__device__ __forceinline__ void mr_store_block_pair(const MrParams& p, unsigned int* stage, double r, double g, double b,
+                                                    bool active, unsigned int j, double r_b, double g_b, double b_b,
+                                                    bool active_b, unsigned int j_b) {
+    mr_store_rgb8_pair(p, stage, mr_as_u8(r), mr_as_u8(g), mr_as_u8(b), r, g, b, active, j,
+                       mr_as_u8(r_b), mr_as_u8(g_b), mr_as_u8(b_b), r_b, g_b, b_b, active_b, j_b);
+}
+
+// The accumulator stays indexed by the launch pixel (sp.acc + 3 * j), so launches over disjoint pixels never share a word.
+__device__ __forceinline__ void mr_store_sampled_pair(const MrParams& p, const MrSampling& sp, unsigned int* stage, double r,
+                                                      double g, double b, bool active, unsigned int j, double r_b,
+                                                      double g_b, double b_b, bool active_b, unsigned int j_b) {
+    unsigned int r8 = mr_as_u8(r), g8 = mr_as_u8(g), b8 = mr_as_u8(b);
+    unsigned int r8_b = mr_as_u8(r_b), g8_b = mr_as_u8(g_b), b8_b = mr_as_u8(b_b);
+    mr_accumulate(sp, j, active, r8, g8, b8);
+    if (!mr_accumulate(sp, j_b, active_b, r8_b, g8_b, b8_b)) return;   // the same uniform answer for both
+    mr_store_rgb8_pair(p, stage, r8, g8, b8, r, g, b, active, j, r8_b, g8_b, b8_b, r_b, g_b, b_b, active_b, j_b);
+}
+
 #endif  // MARAY_DEVICE_SEM_CUH

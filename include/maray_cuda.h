@@ -33,10 +33,10 @@ enum {
     MARAY_E_INVALID = -1,      /* bad argument / call order                                   */
     MARAY_E_PARSE = -2,        /* not a .maray file (either layout)                           */
     MARAY_E_SCENE = -3,        /* scene rejected: unbound variable, cyclic Let, App id out of the
-                                  texture runtime's table (the reference yields NaN / panics)   */
+                                  runtime's function table (the reference yields NaN / panics)  */
     MARAY_E_COMPILE = -4,      /* NVRTC / code generation failure                             */
     MARAY_E_CUDA = -5,         /* CUDA runtime failure or no usable device                    */
-    MARAY_E_UNSUPPORTED = -6   /* e.g. a Runtime other than the default texture runtime       */
+    MARAY_E_UNSUPPORTED = -6   /* e.g. the interpreter asked to run a custom runtime's App     */
 };
 
 /* Back ends (siblings of the reference's WAT code generator, reference src/wasm.rs). */
@@ -118,6 +118,32 @@ const char* maray_cuda_last_error(const maray_cuda_t* h);
  * row-major R,G,B (image::RgbImage).  Copied to every GPU of the handle.  Must precede compile. */
 int maray_cuda_set_textures(maray_cuda_t* h, uint32_t n, const uint8_t* const* rgb8,
                             const uint32_t* w, const uint32_t* hgt);
+
+/* A Runtime<T> other than the default texture runtime (reference src/lib.rs:72-98).  `cuda_source` defines
+ *     __device__ double maray_app(const unsigned char* ctx, unsigned long long ctx_bytes,
+ *                                 unsigned int id, double a, double b);
+ * and the scene's App(id, a, b) evaluates to maray_app(ctx, ctx_bytes, id, a, b) for id < n_functions (the reference's
+ * functions[id](&ctx, id, a, b), src/lib.rs:664-668).  Replaces the texture runtime, and set_textures replaces it: one
+ * runtime per handle, the last call of set_textures / set_functions wins.  NULL returns the handle to the default
+ * texture runtime with no textures.  Takes effect at the next compile.
+ *   - App id >= n_functions is MARAY_E_SCENE at compile time (the reference's index panic, as for textures).
+ *   - maray_app must be a pure function of its arguments and the context bytes: the code generator may evaluate it
+ *     once for equal arguments, skip it inside a guarded region whose guard is false across a warp, evaluate it twice
+ *     per thread (pixel pairs), and evaluate it for idle lanes that redo a launch's first pixel.  It must not write
+ *     memory, use shared memory, barriers or warp intrinsics.
+ *   - The source is compiled after the library's device prelude with the same NVRTC options (sm_100a, --fmad=false):
+ *     it may call mr_sin, mr_exp, mr_log (in the handle's libm mode, exact mode included), mr_tex and
+ *     mr_as_u32_nonneg.  A compile error in it is MARAY_E_COMPILE; last_error carries the NVRTC log.
+ *   - Only the NVRTC back end can call it.  MARAY_BACKEND_INTERP returns MARAY_E_UNSUPPORTED for a scene that calls
+ *     App under a custom runtime; MARAY_BACKEND_AUTO uses cached cubins at once and otherwise compiles with NVRTC
+ *     before it returns, so on a cold cache the first frame waits for NVRTC.
+ *   - A fault inside maray_app (e.g. a read past ctx_bytes) is a bug of the caller's code: it is the one case in which
+ *     this library's "never a device fault" does not hold. */
+int maray_cuda_set_functions(maray_cuda_t* h, const char* cuda_source, uint32_t n_functions);
+/* The context bytes of the custom runtime (`rt.ctx`), copied to every GPU of the handle.  Valid before or after
+ * compile.  Takes effect at the next render and recompiles nothing.  Waits for the handle's in-flight work on its GPUs
+ * (including bands rendered on a caller's stream) before it replaces the buffer. */
+int maray_cuda_set_context(maray_cuda_t* h, const void* ctx, size_t bytes);
 
 /* `maray::open` on an in-memory file (reference src/lib.rs:1227-1235): bincode
  * ([u32;2],[Expr;3]), current or legacy variant numbering. */

@@ -6,5 +6,5 @@ its host-side mirror of the reference's render API (`render.py`) plus scene-auth
 and a GPU.
 """
 from . import expr  # noqa: F401
-from .render import (CudaRenderer, MarayCudaError, RenderMethod, Report, Runtime, Textures, gen,  # noqa: F401
+from .render import (CudaFunctions, CudaRenderer, MarayCudaError, RenderMethod, Report, Runtime, Textures, gen,  # noqa: F401
                      gen_to_image)

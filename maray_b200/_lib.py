@@ -51,6 +51,8 @@ SYMBOLS = [
     ("maray_cuda_last_error", ctypes.c_char_p, [_P]),
     ("maray_cuda_set_textures", ctypes.c_int, [_P, ctypes.c_uint32, ctypes.POINTER(_P), ctypes.POINTER(ctypes.c_uint32),
                                                ctypes.POINTER(ctypes.c_uint32)]),
+    ("maray_cuda_set_functions", ctypes.c_int, [_P, ctypes.c_char_p, ctypes.c_uint32]),
+    ("maray_cuda_set_context", ctypes.c_int, [_P, _P, ctypes.c_size_t]),
     ("maray_cuda_load_maray", ctypes.c_int, [_P, ctypes.c_char_p, ctypes.c_size_t]),
     ("maray_cuda_scene_size", ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_uint32), ctypes.POINTER(ctypes.c_uint32)]),
     ("maray_cuda_set_libm", ctypes.c_int, [_P, ctypes.c_int]),

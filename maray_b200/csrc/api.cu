@@ -62,6 +62,8 @@ struct Gpu {
     // textures
     std::vector<uint8_t*> d_tex;
     MrTexture* d_textab = nullptr;
+    // custom runtime: the context bytes (maray_cuda_set_context); every loaded unit that calls maray_app points at them
+    uint8_t* d_app_ctx = nullptr;
     // back ends
     std::vector<cudaLibrary_t> libs;                   // one per translation unit (chain form: one per segment)
     std::vector<cudaKernel_t> jit_kernels;             // the kernel of each unit, in launch order
@@ -84,6 +86,7 @@ struct JitBuild {
     CodegenInfo info;
     unsigned maxreg = 0;
     int libm = MARAY_LIBM_FAST;               // which sin/exp/ln the units are compiled against (maray_cuda_set_libm)
+    std::string app_source;                   // custom runtime: the user's maray_app (maray_cuda_set_functions), or ""
     uint64_t frame_pixels = 0;                // the scene's declared size (a hint for the launch shape), 0 = unknown
     uint32_t sms = 148;                       // SMs of the first GPU (148 without one)
     double codegen_ms = 0.0, nvrtc_ms = 0.0;
@@ -107,6 +110,11 @@ struct maray_cuda {
     bool have_scene = false;
     std::vector<HostTexture> textures;
     bool textures_uploaded = false;
+    // custom runtime (maray_cuda_set_functions): replaces the texture runtime while custom_rt is set
+    bool custom_rt = false;
+    std::string app_source;
+    uint32_t app_functions = 0;
+    std::vector<uint8_t> app_ctx;       // maray_cuda_set_context
     Program prog;
     bool compiled = false;
     int backend = -1;                   // as asked for: MARAY_BACKEND_*
@@ -208,6 +216,48 @@ int upload_textures(maray_cuda* h) {
     }
     h->textures_uploaded = true;
     return MARAY_OK;
+}
+
+// Points the custom-runtime constants of every unit loaded on `g` that calls maray_app at g's context buffer.
+int bind_app_context(maray_cuda* h, Gpu& g) {
+    const unsigned long long bytes = h->app_ctx.size();
+    for (cudaLibrary_t lib : g.libs) {
+        void* sym = nullptr;
+        size_t sym_bytes = 0;
+        if (cudaLibraryGetGlobal(&sym, &sym_bytes, lib, "mr_app_ctx") != cudaSuccess) { cudaGetLastError(); continue; }   // calls no maray_app
+        CU_TRY(h, cudaMemcpy(sym, &g.d_app_ctx, sizeof(g.d_app_ctx), cudaMemcpyHostToDevice));
+        CU_TRY(h, cudaLibraryGetGlobal(&sym, &sym_bytes, lib, "mr_app_ctx_bytes"));
+        CU_TRY(h, cudaMemcpy(sym, &bytes, sizeof bytes, cudaMemcpyHostToDevice));
+    }
+    return MARAY_OK;
+}
+
+// Copies the context bytes to every GPU and re-points the loaded units at them.  A band may still be running on a
+// caller's stream (maray_cuda_render_band), reading the old buffer and the constants: the device is synchronised before
+// either changes.
+int upload_app_context(maray_cuda* h) {
+    for (Gpu& g : h->gpus) {
+        CU_TRY(h, cudaSetDevice(g.device));
+        uint8_t* fresh = nullptr;
+        CU_TRY(h, cudaMalloc(&fresh, std::max<size_t>(h->app_ctx.size(), 16)));
+        if (!h->app_ctx.empty()) CU_TRY(h, cudaMemcpy(fresh, h->app_ctx.data(), h->app_ctx.size(), cudaMemcpyHostToDevice));
+        CU_TRY(h, cudaDeviceSynchronize());
+        uint8_t* old = g.d_app_ctx;
+        g.d_app_ctx = fresh;
+        int rc = bind_app_context(h, g);
+        if (old) cudaFree(old);
+        if (rc) return rc;
+    }
+    if (!h->gpus.empty()) cudaSetDevice(h->gpus[0].device);
+    return MARAY_OK;
+}
+
+void release_app_context(maray_cuda* h) {
+    for (Gpu& g : h->gpus) {
+        cudaSetDevice(g.device);
+        if (g.d_app_ctx) { cudaFree(g.d_app_ctx); g.d_app_ctx = nullptr; }
+    }
+    h->app_ctx.clear();
 }
 
 // Completion counters of a frame shared between band processes: one 32-bit counter per rank, in the same allocation
@@ -507,6 +557,7 @@ int jit_build(const Program& prog, JitBuild* jb, bool cached_only, const std::at
     // are 5.7 MB of code and 53 s of NVRTC here instead of 1.7 MB / 11 s).
     if (jb->libm == MARAY_LIBM_GLIBC) copt.inline_transcendentals_below = 0;
     copt.frame_pixels_hint = jb->frame_pixels;
+    copt.app_source = jb->app_source;
     copt.sm_count_hint = jb->sms ? jb->sms : 148;
     if (const char* e = std::getenv("MARAY_JIT_SEGMENT_VALUES")) copt.segment_values = uint32_t(std::strtoul(e, nullptr, 10));
     if (const char* e = std::getenv("MARAY_JIT_INLINE_TRANS_BELOW")) copt.inline_transcendentals_below = uint32_t(std::strtoul(e, nullptr, 10));
@@ -606,6 +657,8 @@ int jit_install(maray_cuda* h, JitBuild&& jb) {
                     cudaGetLastError();
             } else cudaGetLastError();
         }
+        int rc = bind_app_context(h, g);
+        if (rc) return rc;
     }
     if (!h->gpus.empty()) cudaSetDevice(h->gpus[0].device);
     h->stats.load_ms += now_ms() - t3;
@@ -617,6 +670,9 @@ int jit_install(maray_cuda* h, JitBuild&& jb) {
 int interp_build_and_install(maray_cuda* h) {
     double t1 = now_ms();
     std::string err;
+    if (h->prog.stats.op_count[OP_APP])
+        return fail(h, MARAY_E_UNSUPPORTED, "the interpreter back end cannot call a custom runtime's maray_app: it is a prebuilt "
+                                            "kernel (DESIGN.md 3.7); compile with MARAY_BACKEND_NVRTC or MARAY_BACKEND_AUTO");
     // Row-uniform form by default; the all-wide form when the scalar file would crowd out the slot file
     // (or MARAY_INTERP_UNIFORM=0, for A/B).
     bool uniform = true;
@@ -1086,6 +1142,7 @@ void maray_cuda_destroy(maray_cuda_t* h) {
         if (g.d_f64) cudaFree(g.d_f64);
         if (g.d_acc) cudaFree(g.d_acc);
         if (g.d_sink) cudaFree(g.d_sink);
+        if (g.d_app_ctx) cudaFree(g.d_app_ctx);
         if (g.frame_done) cudaEventDestroy(g.frame_done);
         if (g.ev0) cudaEventDestroy(g.ev0);
         if (g.ev1) cudaEventDestroy(g.ev1);
@@ -1102,6 +1159,10 @@ void maray_cuda_destroy(maray_cuda_t* h) {
 int maray_cuda_set_textures(maray_cuda_t* h, uint32_t n, const uint8_t* const* rgb8, const uint32_t* w, const uint32_t* hgt) {
     if (!h || (n && (!rgb8 || !w || !hgt))) return fail(h, MARAY_E_INVALID, "maray_cuda_set_textures: bad arguments");
     release_textures(h);
+    if (h->custom_rt) release_app_context(h);   // one runtime per handle: the texture runtime replaces a custom one
+    h->custom_rt = false;
+    h->app_source.clear();
+    h->app_functions = 0;
     h->textures.clear();
     h->textures.resize(n);
     for (uint32_t i = 0; i < n; i++) {
@@ -1113,6 +1174,25 @@ int maray_cuda_set_textures(maray_cuda_t* h, uint32_t n, const uint8_t* const* r
     }
     h->compiled = false;   // width/height constants are folded into the program
     return MARAY_OK;
+}
+
+int maray_cuda_set_functions(maray_cuda_t* h, const char* cuda_source, uint32_t n_functions) {
+    if (!h) return MARAY_E_INVALID;
+    if (!cuda_source) return maray_cuda_set_textures(h, 0, nullptr, nullptr, nullptr);
+    release_textures(h);
+    h->textures.clear();
+    h->custom_rt = true;
+    h->app_source = cuda_source;
+    h->app_functions = n_functions;
+    h->compiled = false;   // the units must be generated again
+    return MARAY_OK;
+}
+
+int maray_cuda_set_context(maray_cuda_t* h, const void* ctx, size_t bytes) {
+    if (!h || (bytes && !ctx)) return fail(h, MARAY_E_INVALID, "maray_cuda_set_context: bad arguments");
+    const uint8_t* p = static_cast<const uint8_t*>(ctx);
+    h->app_ctx.assign(p, p + bytes);
+    return upload_app_context(h);
 }
 
 int maray_cuda_load_maray(maray_cuda_t* h, const uint8_t* bytes, size_t len) {
@@ -1144,17 +1224,20 @@ int maray_cuda_compile(maray_cuda_t* h, int backend, maray_cuda_stats* stats) {
     h->backend = backend;
 
     double t0 = now_ms();
-    std::vector<TextureDim> dims;
-    for (const HostTexture& t : h->textures) dims.push_back(TextureDim{t.w, t.h});
+    RuntimeDesc rt;
+    for (const HostTexture& t : h->textures) rt.textures.push_back(TextureDim{t.w, t.h});
+    rt.custom = h->custom_rt;
+    rt.n_functions = h->app_functions;
     std::string err;
     Program prog;
-    if (!lower_scene(h->scene, dims, &prog, &err)) return fail(h, MARAY_E_SCENE, err);
+    if (!lower_scene(h->scene, rt, &prog, &err)) return fail(h, MARAY_E_SCENE, err);
     h->prog = std::move(prog);
     h->stats.lower_ms = now_ms() - t0;
     fill_program_stats(h);
     if (!h->gpus.empty()) {
         int rc = upload_textures(h);
         if (rc) return rc;
+        if (h->custom_rt && !h->gpus[0].d_app_ctx && (rc = upload_app_context(h)) != MARAY_OK) return rc;
     }
 
     int rc = MARAY_OK;
@@ -1162,7 +1245,7 @@ int maray_cuda_compile(maray_cuda_t* h, int backend, maray_cuda_stats* stats) {
         rc = interp_build_and_install(h);
     } else if (backend == MARAY_BACKEND_NVRTC) {
         JitBuild jb;
-        jb.libm = h->libm; jb.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; jb.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
+        jb.libm = h->libm; jb.app_source = h->app_source; jb.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; jb.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
         rc = jit_build(h->prog, &jb, /*cached_only=*/false, nullptr);
         if (rc) { h->jit = std::move(jb); fill_jit_stats(h); return fail(h, rc, h->jit.error); }   // the generated text stays inspectable
         rc = jit_install(h, std::move(jb));
@@ -1171,7 +1254,7 @@ int maray_cuda_compile(maray_cuda_t* h, int backend, maray_cuda_stats* stats) {
         // ready in milliseconds -- renders while NVRTC works on another thread; renders switch to the generated
         // kernels, between row chunks, as soon as they are built.  Both back ends produce the same bytes.
         JitBuild jb;
-        jb.libm = h->libm; jb.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; jb.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
+        jb.libm = h->libm; jb.app_source = h->app_source; jb.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; jb.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
         rc = jit_build(h->prog, &jb, /*cached_only=*/true, nullptr);
         if (rc == MARAY_OK) {
             rc = jit_install(h, std::move(jb));
@@ -1180,7 +1263,7 @@ int maray_cuda_compile(maray_cuda_t* h, int backend, maray_cuda_stats* stats) {
             if (rc == MARAY_E_UNSUPPORTED) {
                 // the slot file does not fit: compile now, there is nothing to render with meanwhile
                 JitBuild now;
-                now.libm = h->libm; now.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; now.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
+                now.libm = h->libm; now.app_source = h->app_source; now.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; now.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
                 rc = jit_build(h->prog, &now, false, nullptr);
                 if (rc) return fail(h, rc, now.error);
                 rc = jit_install(h, std::move(now));
@@ -1188,7 +1271,7 @@ int maray_cuda_compile(maray_cuda_t* h, int backend, maray_cuda_stats* stats) {
                 h->job.reset(new JitJob());
                 JitJob* job = h->job.get();
                 job->prog = h->prog;
-                job->build.libm = h->libm; job->build.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; job->build.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
+                job->build.libm = h->libm; job->build.app_source = h->app_source; job->build.frame_pixels = uint64_t(h->scene.size[0]) * h->scene.size[1]; job->build.sms = h->gpus.empty() ? 148u : uint32_t(h->gpus[0].sms);
                 job->th = std::thread([job] {
                     job->rc = jit_build(job->prog, &job->build, false, &job->cancel);
                     job->state = job->rc == MARAY_OK ? 1 : 2;

@@ -257,6 +257,10 @@ std::vector<uint64_t> bytecode_for_launch(const Bytecode& bc, uint32_t slot16, s
 bool compile_bytecode(const Program& prog, Bytecode* out, std::string* err, bool row_uniform) {
     out->code.clear();
     out->consts.clear();
+    if (prog.stats.op_count[OP_APP]) {   // the interpreter is a prebuilt kernel: it cannot call a custom runtime's code
+        if (err) *err = "the interpreter back end cannot call a custom runtime's maray_app (use the NVRTC back end)";
+        return false;
+    }
     BcGen g(prog, *out, row_uniform);
     g.run();
     if (!g.err.empty()) { if (err) *err = g.err; return false; }

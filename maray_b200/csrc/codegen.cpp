@@ -165,6 +165,10 @@ struct Emitter {
             bin(buf, ", ", ")");
             break;
         }
+        case OP_APP:
+            std::snprintf(buf, sizeof buf, "maray_app(mr_app_ctx, mr_app_ctx_bytes, %uu, ", n.imm);
+            bin(buf, ", ", ")");
+            break;
         default: s += "0.0"; break;
         }
         s += ";\n";
@@ -321,6 +325,7 @@ GuardRegions find_guard_regions(const Program& prog, const std::vector<uint8_t>&
         switch (prog.nodes[v].op) {
         case OP_NEG: return 0;                                   // folded into its reader's operand
         case OP_SIN: case OP_EXP: case OP_LN: return !sign_only.empty() && sign_only[v] ? 7 : 16;
+        case OP_APP: return kAppWeight;
         default: return 1;
         }
     };
@@ -475,6 +480,21 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
     }
     prelude += kDeviceSemText;
     prelude += "\n";
+    // A custom runtime's functions, in the units that call them: the user's source after the prelude (so it sees mr_sin,
+    // mr_exp, mr_log, mr_tex and the libm mode), and the context buffer in two constants that the host writes per GPU
+    // after each load (maray_cuda_set_context) -- the kernel parameters, and so F's offset in them, stay as they are.
+    std::string app_text;
+    if (prog.stats.op_count[OP_APP]) {
+        app_text = "// custom runtime (maray_cuda_set_functions / maray_cuda_set_context)\n"
+                   "__constant__ const unsigned char* mr_app_ctx;\n"
+                   "__constant__ unsigned long long mr_app_ctx_bytes;\n";
+        app_text += opt.app_source;
+        app_text += "\n";
+    }
+    auto calls_app = [&](size_t lo, size_t hi) {
+        for (size_t i = lo; i < hi; i++) if (prog.nodes[order[i]].op == OP_APP) return true;
+        return false;
+    };
 
     char buf[320];
     // The sampling state is the last parameter, after the chain kernels' frame arguments (whose offsets stay put), with
@@ -631,6 +651,7 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
             std::string unit;
             unit.reserve((seg_hi(s) - seg_lo(s)) * 56 + prelude.size() + 4096);
             unit += prelude;
+            if (calls_app(seg_lo(s), seg_hi(s))) unit += app_text;
             unit += bank_text(bk);
             std::snprintf(buf, sizeof buf, "// segment %u of %u\n", s, n_seg);
             unit += buf;
@@ -655,6 +676,7 @@ std::vector<std::string> generate(const Program& prog, const CodegenOptions& opt
         std::string src;
         src.reserve(order.size() * 40 + 8192);
         src += prelude;
+        src += app_text;
         src += bank_text(whole_bank);
         auto lref = [](int32_t f) { return "F[" + std::to_string(f) + "]"; };
         if (segmented) {

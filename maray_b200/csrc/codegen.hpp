@@ -61,6 +61,8 @@ struct CodegenOptions {
     // pixel have independent work beside them and one warp vote serves two pixels.  Other kernels keep one pixel per
     // thread (MARAY_JIT_PAIRS=0 for A/B).
     bool pixel_pairs = true;
+    // A custom runtime (maray_cuda_set_functions): CUDA source defining maray_app, put into every unit that calls it.
+    std::string app_source;
 };
 
 struct CodegenInfo {
@@ -84,6 +86,9 @@ constexpr uint32_t kOneBlockPerSmValues = 4096;   // CodegenOptions::auto_shape
 // 128 texture regions, 2.943 / 2.982 / 3.058 ms when the 15 / 128 / 207 smaller ANDs get regions too.  sdf, textured
 // and deep have no AND this heavy.
 constexpr uint32_t kGuardBodyMinWeight = 32;
+// Weight of a custom runtime's maray_app call in a guarded region's body: that of an inlined sin/exp/ln.  Unmeasured --
+// nothing is known about what a user's function costs (DESIGN.md 3.7).
+constexpr uint32_t kAppWeight = 16;
 
 // One translation unit (segment functions, if any, as __noinline__ functions of the same unit).
 std::string generate_cuda_source(const Program& prog, const CodegenOptions& opt, CodegenInfo* info);

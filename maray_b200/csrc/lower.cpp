@@ -13,7 +13,7 @@ namespace maray {
 
 const char* op_name(Op o) {
     static const char* names[OP_COUNT] = {"const", "x", "y", "neg", "abs", "recip", "sqrt", "step", "sin", "exp",
-                                          "ln", "add", "mul", "max", "min", "tex"};
+                                          "ln", "add", "mul", "max", "min", "tex", "app"};
     return o < OP_COUNT ? names[o] : "?";
 }
 
@@ -48,7 +48,7 @@ uint64_t bits_of(double v) { uint64_t b; std::memcpy(&b, &v, 8); return b; }
 
 class Lowering {
 public:
-    Lowering(const std::vector<TextureDim>& tex) : tex_(tex) {}
+    Lowering(const RuntimeDesc& rt) : rt_(rt), tex_(rt.textures) {}
 
     std::vector<Node> nodes;
     std::string err;
@@ -111,8 +111,18 @@ public:
         return intern(op, a, b, 0);
     }
 
-    // App(id, a, b) with the default texture runtime (reference src/textures.rs:14-65).
+    // App(id, a, b) with the default texture runtime (reference src/textures.rs:14-65), or a call of the custom
+    // runtime's maray_app.  The latter is never folded, not even with constant arguments: there is no host twin of the
+    // user's function, and the reference calls it at run time.
     uint32_t app(uint32_t id, uint32_t a, uint32_t b) {
+        if (rt_.custom) {
+            if (id >= rt_.n_functions) {
+                err = "App id " + std::to_string(id) + " is outside the custom runtime's function table (" +
+                      std::to_string(rt_.n_functions) + " functions)";
+                return NONE;
+            }
+            return intern(OP_APP, a, b, id);
+        }
         uint32_t img = id / 5, k = id % 5;
         if (img >= tex_.size()) {
             err = "App id " + std::to_string(id) + " is outside the texture runtime's function table (" +
@@ -211,13 +221,14 @@ private:
         return NONE;
     }
 
+    const RuntimeDesc& rt_;
     const std::vector<TextureDim>& tex_;
     std::unordered_map<Key, uint32_t, KeyHash> table_;
 };
 
 struct LowerJob {
     const Scene* scene;
-    const std::vector<TextureDim>* tex;
+    const RuntimeDesc* rt;
     Program* out;
     std::string* err;
     bool ok;
@@ -244,7 +255,7 @@ void lower_job(void* arg) {
 }
 
 void lower_job_body(LowerJob* j) {
-    Lowering L(*j->tex);
+    Lowering L(*j->rt);
     uint32_t roots[3];
     for (int c = 0; c < 3; c++) {
         roots[c] = L.lower(j->scene->color[c], nullptr);
@@ -302,7 +313,7 @@ void lower_job_body(LowerJob* j) {
     Program* P = j->out;
     P->nodes.swap(out_nodes);
     for (int c = 0; c < 3; c++) P->root[c] = remap[roots[c]];
-    P->n_textures = uint32_t(j->tex->size());
+    P->n_textures = uint32_t(j->rt->textures.size());
     P->order.clear();
     // Two candidate schedules: (a) the depth-first order above, (b) the order in which the scene
     // itself introduces values (Let definitions in file order, then the bodies).  Depth-first keeps
@@ -524,9 +535,9 @@ void lower_job_body(LowerJob* j) {
 
 }  // namespace
 
-bool lower_scene(const Scene& scene, const std::vector<TextureDim>& textures, Program* out, std::string* err) {
+bool lower_scene(const Scene& scene, const RuntimeDesc& rt, Program* out, std::string* err) {
     std::string local;
-    LowerJob j{&scene, &textures, out, err ? err : &local, false};
+    LowerJob j{&scene, &rt, out, err ? err : &local, false};
     if (!run_with_big_stack(lower_job, &j)) {
         if (err) *err = "cannot start the lowering thread (1 GiB stack unavailable)";
         return false;

@@ -21,11 +21,12 @@ enum Op : uint8_t {
     OP_NEG, OP_ABS, OP_RECIP, OP_SQRT, OP_STEP, OP_SIN, OP_EXP, OP_LN,
     OP_ADD, OP_MUL, OP_MAX, OP_MIN,
     OP_TEX,          // a = x coordinate, b = y coordinate, imm = texture*4 + channel
+    OP_APP,          // custom runtime: maray_app(ctx, ctx_bytes, imm, a, b), imm = the App id (never folded)
     OP_COUNT
 };
 
 inline bool op_is_unary(Op o) { return o >= OP_NEG && o <= OP_LN; }
-inline bool op_is_binary(Op o) { return o >= OP_ADD && o <= OP_TEX; }
+inline bool op_is_binary(Op o) { return o >= OP_ADD && o <= OP_APP; }
 const char* op_name(Op o);
 
 enum Dep : uint8_t { DEP_CONST = 0, DEP_X = 1, DEP_Y = 2, DEP_XY = 3 };
@@ -34,11 +35,20 @@ struct Node {
     Op op;
     uint8_t dep;       // Dep bits
     uint32_t a, b;     // operand value ids (unused: 0)
-    uint32_t imm;      // OP_TEX only
+    uint32_t imm;      // OP_TEX, OP_APP only
     double k;          // OP_CONST only
 };
 
 struct TextureDim { uint32_t w, h; };
+
+// What `App(id, a, b)` calls (reference src/lib.rs:72-98, 664-668): the default texture runtime (textures::functions,
+// five functions per texture, width and height folded on the host), or a custom runtime of n_functions functions that
+// the host supplies as CUDA source (maray_cuda_set_functions): every App is an OP_APP value, evaluated at run time.
+struct RuntimeDesc {
+    std::vector<TextureDim> textures;
+    bool custom = false;
+    uint32_t n_functions = 0;
+};
 
 // Programs with at least this many sin/exp/ln values evaluate them out of line (the NVRTC back end
 // calls batched helper functions instead of inlining every body) and get their schedule batched.
@@ -72,8 +82,9 @@ struct Program {
 // matter, like the reference interpreter's by-name lookup, reference src/cache.rs:30-38).
 // Errors (returned as false + message) instead of the reference's silent NaN / panic:
 //   unbound variable (reference src/cache.rs:40 yields NaN), cyclic definitions,
-//   App id >= 5 * textures.size() (reference src/lib.rs:665 panics on the index).
-bool lower_scene(const Scene& scene, const std::vector<TextureDim>& textures, Program* out, std::string* err);
+//   App id >= the runtime's function count: 5 * textures.size(), or n_functions of a custom runtime
+//   (reference src/lib.rs:665 panics on the index).
+bool lower_scene(const Scene& scene, const RuntimeDesc& rt, Program* out, std::string* err);
 
 // ---- operation semantics shared by host constant folding (reference src/lib.rs:632-669) --------
 // f64::max / f64::min: NaN-ignoring; on an equal-compare tie (incl. +0/-0) the first operand wins

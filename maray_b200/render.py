@@ -5,6 +5,7 @@
   RenderMethod::{..}   src/lib.rs:1154-1173   RenderMethod.Cuda(gpus, report, backend, samples)  (new arm)
   Report               src/report.rs:19-27    Report.none() / Report.row(n) / Report.duration(ms)
   Runtime<Textures>    src/lib.rs:72-98       Runtime(Textures(images))  (functions = textures.functions(n))
+  Runtime<T>           src/lib.rs:72-98       Runtime.from_parts(ctx_bytes, CudaFunctions(source, n))
   gen_to_image         src/lib.rs:1177-1195   gen_to_image(method, rt, color, img, report)
   gen                  src/lib.rs:1199-1213   gen(method, rt, color, file, size)
   open / save          src/lib.rs:1216-1235   open_ / save  (maray_b200.expr)
@@ -66,18 +67,33 @@ class Textures:
     images: List[np.ndarray] = field(default_factory=list)
 
 
+@dataclass(frozen=True)
+class CudaFunctions:
+    """The device twin of a `Runtime<T>`'s `functions` (reference src/lib.rs:72-98): CUDA source defining
+    `__device__ double maray_app(const unsigned char* ctx, unsigned long long ctx_bytes, unsigned int id, double a,
+    double b)`, and n = functions.len().  App(id, a, b) evaluates to maray_app(ctx, ctx_bytes, id, a, b) for id < n
+    (include/maray_cuda.h, maray_cuda_set_functions, states what the function may and may not do)."""
+    source: str
+    n: int
+
+
 @dataclass
 class Runtime:
-    """reference src/lib.rs:72-98.  Only the default texture runtime (`textures::functions(n)`,
-    reference src/textures.rs:54-65) can run on the device; `functions` is therefore implied."""
-    ctx: Textures = field(default_factory=Textures)
+    """reference src/lib.rs:72-98.  The default texture runtime (`textures::functions(n)`, reference
+    src/textures.rs:54-65), whose `functions` are implied, or a custom runtime: `functions` a CudaFunctions and `ctx`
+    its context bytes."""
+    ctx: Union[Textures, bytes, np.ndarray] = field(default_factory=Textures)
+    functions: Optional[CudaFunctions] = None
 
     @staticmethod
     def new() -> "Runtime": return Runtime(Textures([]))
     @staticmethod
-    def from_parts(ctx: Textures, functions=None) -> "Runtime":
+    def from_parts(ctx, functions=None) -> "Runtime":
+        if isinstance(functions, CudaFunctions):
+            return Runtime(ctx, functions)
         if functions is not None and len(functions) != 5 * len(ctx.images):
-            raise MarayCudaError(_lib.E_UNSUPPORTED, "only the default texture runtime (5 functions per image) is supported")
+            raise MarayCudaError(_lib.E_UNSUPPORTED, "only the default texture runtime (5 functions per image) or "
+                                                     "CudaFunctions can run on the device")
         return Runtime(ctx)
 
 
@@ -131,6 +147,22 @@ class CudaRenderer:
         ws = (ctypes.c_uint32 * max(n, 1))(*[a.shape[1] for a in arrs])
         hs = (ctypes.c_uint32 * max(n, 1))(*[a.shape[0] for a in arrs])
         self._check(self._L.maray_cuda_set_textures(self._h, n, ptrs, ws, hs))
+
+    def set_functions(self, source: Optional[str], n: int = 0) -> None:
+        """A custom runtime (maray_cuda_set_functions): `source` defines maray_app, App ids below n call it.  None
+        returns to the default texture runtime with no textures.  Takes effect at the next compile."""
+        self._check(self._L.maray_cuda_set_functions(self._h, None if source is None else source.encode(), int(n)))
+
+    def set_context(self, buf) -> None:
+        """The custom runtime's context bytes (maray_cuda_set_context): bytes-like or a C-contiguous numpy array.
+        Takes effect at the next render; nothing is recompiled."""
+        if isinstance(buf, np.ndarray):
+            if not buf.flags.c_contiguous:
+                raise ValueError("the context array must be C-contiguous")
+            data = buf.view(np.uint8).reshape(-1)
+        else:
+            data = np.frombuffer(bytes(buf), dtype=np.uint8)
+        self._check(self._L.maray_cuda_set_context(self._h, data.ctypes.data if data.size else None, data.size))
 
     def load(self, scene: Union[bytes, tuple]) -> tuple:
         """scene: `.maray` bytes, or (size, color) as returned by maray_b200.expr.open_."""
@@ -286,7 +318,11 @@ def gen_to_image(method: "RenderMethod.Cuda", rt: Runtime, color, img: np.ndarra
         raise MarayCudaError(_lib.E_UNSUPPORTED, "only RenderMethod.Cuda is available (no CPU fallback)")
     h, w = img.shape[0], img.shape[1]
     with CudaRenderer(method.gpus, method.device_ids) as r:
-        r.set_textures(rt.ctx.images)
+        if rt.functions is not None:
+            r.set_functions(rt.functions.source, rt.functions.n)
+            r.set_context(rt.ctx)
+        else:
+            r.set_textures(rt.ctx.images)
         r.load(color if isinstance(color, (bytes, bytearray)) else ([w, h], list(color)))
         stats = r.compile(method.backend)
         r.set_samples(method.samples)

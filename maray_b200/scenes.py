@@ -14,7 +14,8 @@ here evaluates an expression.
 from __future__ import annotations
 
 import os
-from typing import List, Tuple
+import struct
+from typing import List, Sequence, Tuple
 
 import numpy as np
 
@@ -304,6 +305,33 @@ def example_test7_rs() -> bytes:
     """examples/test7.rs: `nat(255) * x() / nat(128)` on every channel, 128x128."""
     e = E.nat(255) * E.x() / E.nat(128)
     return E.to_bytes([128, 128], [e, e, e])
+
+
+# The default texture runtime (reference src/textures.rs:27-50) restated as a custom runtime (maray_cuda_set_functions):
+# the context packs the images as a u32 count, then (w u32, h u32, byte offset u64) per image, then the RGB8 data.
+TEXTURE_RUNTIME_SOURCE = r"""
+__device__ double maray_app(const unsigned char* ctx, unsigned long long ctx_bytes, unsigned int id, double a, double b) {
+    const unsigned int img = id / 5u, k = id % 5u;
+    const unsigned char* e = ctx + 8u + 16u * img;
+    const unsigned int w = *reinterpret_cast<const unsigned int*>(e);
+    const unsigned int h = *reinterpret_cast<const unsigned int*>(e + 4);
+    if (k == 3u) return (double)w;                           // fun_image_width
+    if (k == 4u) return (double)h;                           // fun_image_height
+    const unsigned long long off = *reinterpret_cast<const unsigned long long*>(e + 8);
+    return mr_tex(ctx + off, w, h, k, a, b);                 // fun_color_channel
+}
+"""
+
+
+def pack_textures(images: Sequence[np.ndarray]) -> bytes:
+    """The context of TEXTURE_RUNTIME_SOURCE for these (h, w, 3) uint8 images; 5 functions per image."""
+    head = struct.pack("<II", len(images), 0)
+    off = 8 + 16 * len(images)
+    data = b""
+    for im in images:
+        head += struct.pack("<IIQ", im.shape[1], im.shape[0], off + len(data))
+        data += np.ascontiguousarray(im, dtype=np.uint8).tobytes()
+    return head + data
 
 
 def by_name(name: str) -> Tuple[bytes, List[np.ndarray], Tuple[int, int]]:

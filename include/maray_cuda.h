@@ -194,6 +194,28 @@ int maray_cuda_set_samples(maray_cuda_t* h, uint32_t s);
  * into contiguous bands, every GPU renders its band and copies it into `rgb` over its own PCIe link. */
 int maray_cuda_render(maray_cuda_t* h, uint32_t w, uint32_t hgt, uint8_t* rgb, maray_cuda_stats* stats);
 
+/* What maray_cuda_render_png's encoder did. */
+typedef struct maray_cuda_png_stats {
+    uint64_t scanline_bytes;   /* hgt * (3*w + 1): the PNG's uncompressed image data                  */
+    uint64_t png_bytes;        /* the whole file                                                      */
+    uint32_t segments;         /* deflate segments encoded in parallel                                */
+    uint32_t stored_segments;  /* segments emitted as stored blocks because Huffman coding did not pay */
+    double   encode_ms;        /* device time from the filter kernel to the assembled file, first GPU  */
+    double   d2h_ms;           /* copy of the file to the host                                        */
+} maray_cuda_png_stats;
+
+/* `gen(method, rt, color, file, size)` without the file (reference src/lib.rs:1199-1213): renders a w x hgt frame and
+ * encodes it as a PNG (8-bit RGB, not interlaced) on the handle's first GPU.  With `rgb` not NULL the call renders
+ * exactly as maray_cuda_render does (the frame lands in `rgb`, progress reports fire); with `rgb` NULL it renders as
+ * maray_cuda_render_device does.  *png receives a pointer to the file's *len bytes in a pinned host buffer owned by
+ * the handle, valid until the next maray_cuda_render_png or destroy.  The file's bytes are a function of the frame
+ * alone (not of the GPU, the back end or the number of GPUs); decoded, it is the frame.  `stats` and `png_stats` may
+ * be NULL.  Errors as maray_cuda_render; w or hgt above 2^31-1 is MARAY_E_INVALID (PNG fields are 31-bit); a failed
+ * scratch allocation is MARAY_E_CUDA.  The encoder's scratch (about 7 bytes per scanline byte) stays allocated on the
+ * first GPU until destroy. */
+int maray_cuda_render_png(maray_cuda_t* h, uint32_t w, uint32_t hgt, uint8_t* rgb, const uint8_t** png, size_t* len,
+                          maray_cuda_stats* stats, maray_cuda_png_stats* png_stats);
+
 /* Same, but the finished frame stays in device memory on the handle's first GPU (bands of the other GPUs
  * are gathered there by peer copy over NVLink -- the only exchange step of the path):
  * *d_rgb receives a device pointer (owned by the handle, valid until the next render/destroy). */

@@ -43,6 +43,14 @@ class Stats(ctypes.Structure):
         return d
 
 
+class PngStats(ctypes.Structure):
+    _fields_ = [("scanline_bytes", ctypes.c_uint64), ("png_bytes", ctypes.c_uint64), ("segments", ctypes.c_uint32),
+                ("stored_segments", ctypes.c_uint32), ("encode_ms", ctypes.c_double), ("d2h_ms", ctypes.c_double)]
+
+    def as_dict(self) -> dict:
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 # every symbol include/maray_cuda.h declares: (name, restype, argtypes)
 _P = ctypes.c_void_p
 SYMBOLS = [
@@ -60,6 +68,8 @@ SYMBOLS = [
     ("maray_cuda_compile", ctypes.c_int, [_P, ctypes.c_int, ctypes.POINTER(Stats)]),
     ("maray_cuda_set_report", ctypes.c_int, [_P, ctypes.c_int, ctypes.c_uint32, REPORT_FN, _P]),
     ("maray_cuda_render", ctypes.c_int, [_P, ctypes.c_uint32, ctypes.c_uint32, _P, ctypes.POINTER(Stats)]),
+    ("maray_cuda_render_png", ctypes.c_int, [_P, ctypes.c_uint32, ctypes.c_uint32, _P, ctypes.POINTER(_P),
+                                             ctypes.POINTER(ctypes.c_size_t), ctypes.POINTER(Stats), ctypes.POINTER(PngStats)]),
     ("maray_cuda_render_device", ctypes.c_int, [_P, ctypes.c_uint32, ctypes.c_uint32, ctypes.POINTER(_P),
                                                 ctypes.POINTER(Stats)]),
     ("maray_cuda_render_band", ctypes.c_int, [_P, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, _P, _P]),

@@ -29,6 +29,7 @@
 #include "device_sem.cuh"
 #include "expr.hpp"
 #include "kernels.hpp"
+#include "png_gpu.hpp"
 #include "program.hpp"
 
 using namespace maray;
@@ -139,6 +140,7 @@ struct maray_cuda {
     uint32_t report_every = 0;
     maray_report_fn report_fn = nullptr;
     void* report_user = nullptr;
+    PngScratch png;                                    // maray_cuda_render_png, on the first GPU
 };
 
 namespace {
@@ -993,7 +995,9 @@ int render_frame_bands_to_host(maray_cuda* h, uint32_t w, uint32_t hgt, uint8_t*
     return MARAY_OK;
 }
 
-int render_frame(maray_cuda* h, uint32_t w, uint32_t hgt, uint8_t* host_rgb) {
+// keep_frame: the whole frame must also end up in GPU 0's frame buffer (maray_cuda_render_png), so several GPUs
+// gather there instead of copying their bands to the host each.
+int render_frame(maray_cuda* h, uint32_t w, uint32_t hgt, uint8_t* host_rgb, bool keep_frame = false) {
     int rc = check_renderable(h, w, hgt);
     if (rc) return rc;
     double t0 = now_ms();
@@ -1028,7 +1032,8 @@ int render_frame(maray_cuda* h, uint32_t w, uint32_t hgt, uint8_t* host_rgb) {
         (h->report_kind == MARAY_REPORT_NONE || !h->report_fn) && size_t(w) * hgt * 3 >= (size_t(4) << 20)) {
         rc = render_frame_pipelined(h, w, hgt, host_rgb);
         if (rc) return rc;
-    } else if (host_rgb && h->gpus.size() > 1 && hgt >= h->gpus.size() && (h->report_kind == MARAY_REPORT_NONE || !h->report_fn)) {
+    } else if (host_rgb && !keep_frame && h->gpus.size() > 1 && hgt >= h->gpus.size() &&
+               (h->report_kind == MARAY_REPORT_NONE || !h->report_fn)) {
         rc = render_frame_bands_to_host(h, w, hgt, host_rgb);
         if (rc) return rc;
     } else if (h->report_kind == MARAY_REPORT_NONE || !h->report_fn || !host_rgb) {
@@ -1141,6 +1146,7 @@ void maray_cuda_destroy(maray_cuda_t* h) {
         if (g.d_out) cudaFree(g.d_out);
         if (g.d_f64) cudaFree(g.d_f64);
         if (g.d_acc) cudaFree(g.d_acc);
+        if (&g == &h->gpus[0]) png_release(h->png);
         if (g.d_sink) cudaFree(g.d_sink);
         if (g.d_app_ctx) cudaFree(g.d_app_ctx);
         if (g.frame_done) cudaEventDestroy(g.frame_done);
@@ -1319,6 +1325,33 @@ int maray_cuda_render_device(maray_cuda_t* h, uint32_t w, uint32_t hgt, void** d
     if (rc) return rc;
     *d_rgb = h->gpus[0].d_out;
     if (stats) *stats = h->stats;
+    return MARAY_OK;
+}
+
+int maray_cuda_render_png(maray_cuda_t* h, uint32_t w, uint32_t hgt, uint8_t* rgb, const uint8_t** png, size_t* len,
+                          maray_cuda_stats* stats, maray_cuda_png_stats* png_stats) {
+    if (!h) return MARAY_E_INVALID;
+    if (!png || !len) return fail(h, MARAY_E_INVALID, "maray_cuda_render_png: null output pointer");
+    if (w > 0x7fffffffu || hgt > 0x7fffffffu) return fail(h, MARAY_E_INVALID, "maray_cuda_render_png: PNG sizes are at most 2^31-1");
+    int rc = render_frame(h, w, hgt, rgb, /*keep_frame=*/true);
+    if (rc) return rc;
+    Gpu& g = h->gpus[0];
+    CU_TRY(h, cudaSetDevice(g.device));
+    PngResult res;
+    std::string err;
+    if (png_encode_device(h->png, g.d_out, w, hgt, g.stream, &res, &err) != cudaSuccess)
+        return fail(h, MARAY_E_CUDA, "maray_cuda_render_png: " + err);
+    *png = res.file;
+    *len = size_t(res.file_bytes);
+    if (stats) *stats = h->stats;
+    if (png_stats) {
+        png_stats->scanline_bytes = res.scanline_bytes;
+        png_stats->png_bytes = res.file_bytes;
+        png_stats->segments = res.segments;
+        png_stats->stored_segments = res.stored_segments;
+        png_stats->encode_ms = res.encode_ms;
+        png_stats->d2h_ms = res.d2h_ms;
+    }
     return MARAY_OK;
 }
 

@@ -27,6 +27,16 @@ void on_progress(void* user, uint8_t* rgb, uint32_t w, uint32_t h, double progre
     maray::write_png_rgb8(c->out, w, h, rgb, &err);
 }
 
+// Through a temporary file and a rename, as write_png_rgb8 does: a reader never sees a half-written file.
+bool write_file(const std::string& path, const uint8_t* data, size_t len) {
+    std::string tmp = path + ".tmp";
+    FILE* f = std::fopen(tmp.c_str(), "wb");
+    if (!f) return false;
+    bool ok = std::fwrite(data, 1, len, f) == len;
+    ok = (std::fclose(f) == 0) && ok;
+    return ok && std::rename(tmp.c_str(), path.c_str()) == 0;
+}
+
 int usage() {
     std::fprintf(stderr,
                  "Maray (CUDA render path)\n"
@@ -93,11 +103,15 @@ int main(int argc, char** argv) {
     std::vector<uint8_t> img(size_t(w) * hgt * 3);
     ProgressCtx ctx{output};
     maray_cuda_set_report(h, MARAY_REPORT_DURATION_MS, 500, on_progress, &ctx);
-    if (maray_cuda_render(h, w, hgt, img.data(), &st) != MARAY_OK) return die("render");
-    std::string err;
-    if (!maray::write_png_rgb8(output, w, hgt, img.data(), &err)) { std::fprintf(stderr, "error: %s\n", err.c_str()); maray_cuda_destroy(h); return 1; }
-    std::fprintf(stderr, "%ux%u, %llu values, lower %.1f ms, compile %.1f ms, render %.2f ms (kernel %.2f ms on GPU 0)\n", w, hgt,
-                 (unsigned long long)st.dag_nodes, st.lower_ms, st.codegen_ms + st.nvrtc_ms + st.load_ms, st.render_ms, st.kernel_ms[0]);
+    // the final file is encoded on the GPU (maray_cuda_render_png); the partial images above are re-saved on the host
+    const uint8_t* png = nullptr;
+    size_t png_len = 0;
+    maray_cuda_png_stats ps;
+    if (maray_cuda_render_png(h, w, hgt, img.data(), &png, &png_len, &st, &ps) != MARAY_OK) return die("render");
+    if (!write_file(output, png, png_len)) { std::fprintf(stderr, "error: write to %s failed\n", output.c_str()); maray_cuda_destroy(h); return 1; }
+    std::fprintf(stderr, "%ux%u, %llu values, lower %.1f ms, compile %.1f ms, render %.2f ms (kernel %.2f ms on GPU 0), "
+                 "PNG %zu bytes encoded in %.2f ms\n", w, hgt, (unsigned long long)st.dag_nodes, st.lower_ms,
+                 st.codegen_ms + st.nvrtc_ms + st.load_ms, st.render_ms, st.kernel_ms[0], png_len, ps.encode_ms);
     maray_cuda_destroy(h);
     return 0;
 }

@@ -264,6 +264,22 @@ class CudaRenderer:
         self.render_into(img)
         return img
 
+    def render_png(self, w: Optional[int] = None, h: Optional[int] = None, img: Optional[np.ndarray] = None):
+        """Renders a frame and encodes it as a PNG on the first GPU (maray_cuda_render_png).  Returns (file bytes,
+        stats, png_stats).  With `img` (a writable C-contiguous uint8 (h, w, 3) array) the frame also lands there and
+        progress reports fire as in render_into; without it the frame stays on the device."""
+        if img is not None:
+            if img.dtype != np.uint8 or img.ndim != 3 or img.shape[2] != 3 or not img.flags.c_contiguous or not img.flags.writeable:
+                raise ValueError("img must be a writable C-contiguous uint8 array shaped (h, w, 3)")
+            h, w = img.shape[0], img.shape[1]
+        w = self.size[0] if w is None else w
+        h = self.size[1] if h is None else h
+        p, n = ctypes.c_void_p(), ctypes.c_size_t()
+        st, ps = _lib.Stats(), _lib.PngStats()
+        self._check(self._L.maray_cuda_render_png(self._h, w, h, None if img is None else img.ctypes.data, ctypes.byref(p),
+                                                  ctypes.byref(n), ctypes.byref(st), ctypes.byref(ps)))
+        return ctypes.string_at(p.value, n.value), st.as_dict(), ps.as_dict()
+
     def render_device(self, w: int, h: int) -> int:
         """Renders and leaves the frame on the first GPU; returns the device pointer."""
         p = ctypes.c_void_p()
@@ -318,30 +334,47 @@ def gen_to_image(method: "RenderMethod.Cuda", rt: Runtime, color, img: np.ndarra
         raise MarayCudaError(_lib.E_UNSUPPORTED, "only RenderMethod.Cuda is available (no CPU fallback)")
     h, w = img.shape[0], img.shape[1]
     with CudaRenderer(method.gpus, method.device_ids) as r:
-        if rt.functions is not None:
-            r.set_functions(rt.functions.source, rt.functions.n)
-            r.set_context(rt.ctx)
-        else:
-            r.set_textures(rt.ctx.images)
-        r.load(color if isinstance(color, (bytes, bytearray)) else ([w, h], list(color)))
-        stats = r.compile(method.backend)
-        r.set_samples(method.samples)
-        r.set_report(method.report, report)
+        stats = _setup(r, method, rt, color, w, h, report)
         stats.update({k: v for k, v in r.render_into(img).items() if k.endswith("_ms")})
         return stats
 
 
+def _setup(r: CudaRenderer, method: "RenderMethod.Cuda", rt: Runtime, color, w: int, h: int, report) -> dict:
+    """Runtime, scene, back end, samples and progress of a gen_to_image / gen call; returns the compile stats."""
+    if rt.functions is not None:
+        r.set_functions(rt.functions.source, rt.functions.n)
+        r.set_context(rt.ctx)
+    else:
+        r.set_textures(rt.ctx.images)
+    r.load(color if isinstance(color, (bytes, bytearray)) else ([w, h], list(color)))
+    stats = r.compile(method.backend)
+    r.set_samples(method.samples)
+    r.set_report(method.report, report)
+    return stats
+
+
 def gen(method: "RenderMethod.Cuda", rt: Runtime, color, file: str, size: Sequence[int]) -> dict:
-    """reference src/lib.rs:1199-1213: render and save a PNG (progress ticks re-save the partial image)."""
+    """reference src/lib.rs:1199-1213: render and save a PNG.  Progress ticks re-save the partial image on the host;
+    the final file is encoded on the GPU (CudaRenderer.render_png)."""
+    import os
+    import sys
+
     from PIL import Image
 
     img = np.zeros((size[1], size[0], 3), dtype=np.uint8)
 
     def progress(partial: np.ndarray, p: float) -> None:
-        import sys
         print(f"{100.0 * p:.2f} %", file=sys.stderr, flush=True)
         Image.fromarray(partial).save(file)
 
-    stats = gen_to_image(method, rt, color, img, progress)
-    Image.fromarray(img).save(file)
+    if not isinstance(method, RenderMethod.Cuda):
+        raise MarayCudaError(_lib.E_UNSUPPORTED, "only RenderMethod.Cuda is available (no CPU fallback)")
+    with CudaRenderer(method.gpus, method.device_ids) as r:
+        _setup(r, method, rt, color, size[0], size[1], progress)
+        png, stats, png_stats = r.render_png(img=img)
+    tmp = file + ".tmp"
+    with open(tmp, "wb") as f:
+        f.write(png)
+    os.replace(tmp, file)
+    stats.update({"png_" + k: v for k, v in png_stats.items()})
     return stats
